@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RK4 grid-point.steps/s of the pseudospectral barotropic step on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--grid G] [--impl xfb|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--grid G] [--impl xfb|reference] [--dump-outputs DIR]
 
 One "step" is one RK4 step (4 tendency evaluations = 20 2-D FFTs in the reference).
   N = 1 : the elliptic vortex (reference generator makefield-elliptic-vortex.cpp) at 8192^2 -- the headline grid of
@@ -235,6 +235,24 @@ def reference_arm(args):
 # GPU arm
 # --------------------------------------------------------------------------------------------------
 
+DUMP_BYTES = 60 * 10 ** 6         # field data; with the .npy headers the files stay under 64 MB
+DUMP_FIELDS = ("vort", "psi", "u", "v")
+
+
+def dump_outputs(b, n: int, members: int, out_dir: str) -> None:
+    """--dump-outputs: the fields a caller reads back after the timed steps (xfb_get_field: vort, psi, u, v of every
+    member) as <out_dir>/<field>[_m<member>].npy, float32.  Within DUMP_BYTES in all: where a full field does not fit,
+    the same rows are kept in every file, chosen by a fixed seed, so two builds can be compared file by file."""
+    import xlab_fftbarotropic_b200 as xfb
+    rows_fit = max(1, DUMP_BYTES // (len(DUMP_FIELDS) * members * 4 * n))
+    rows = np.arange(n) if rows_fit >= n else np.sort(np.random.default_rng(0).choice(n, rows_fit, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for m in range(members):
+        for name in DUMP_FIELDS:
+            f = b.get_field(getattr(xfb.capi, name.upper()), member=m)
+            np.save(os.path.join(out_dir, name + (f"_m{m}" if m else "") + ".npy"), np.ascontiguousarray(f[rows]))
+
+
 def gpu_arm(args):
     import torch
     import fields
@@ -305,6 +323,8 @@ def gpu_arm(args):
     # `value` is the product's default path (graph replay); the bracketed pass only feeds the per-kernel roofline
     ms_bracketed = ms
     ms = ms_graph
+    if args.dump_outputs and rank == 0:
+        dump_outputs(b, n, args.members, args.dump_outputs)
     if dist is not None:
         t = torch.tensor([ms, ms_bracketed], device=f"cuda:{local_rank}")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -510,7 +530,12 @@ def main():
     ap.add_argument("--chunks", type=int, default=8, help="slab arm: chunks of the compute/exchange overlap")
     ap.add_argument("--no-slab-check", action="store_true", help="slab arm: skip the in-run check against the single-GPU path and T1")
     ap.add_argument("--no-ensemble-record", action="store_true", help="slab arm: skip the ensemble sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="single-GPU arm: after the timed steps, write the fields they "
+                                                          "computed to DIR/<field>.npy (float32, at most 64 MB in all), "
+                                                          "e.g. bench_outputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     # ONE JSON line on stdout: libraries write there too (NCCL prints "NCCL version ..." when NCCL_DEBUG is set), so the
     # process-level stdout goes to stderr while the bench runs and the JSON line is written to the real stdout at the end
     sys.stdout.flush()
@@ -521,6 +546,8 @@ def main():
     slab = args.slab or ((world > 1 or args.gpus > 1) and not args.ensemble)
     if args.grid is None:
         args.grid = 16384 if slab else 8192
+    if args.dump_outputs and (slab or args.impl == "reference"):
+        ap.error("--dump-outputs is supported by the single-GPU product arm only")
     if args.impl == "reference":
         reference_arm(args)
     elif slab:

@@ -17,7 +17,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import rel_l2
+from conftest import check_golden, rel_l2
 import fields
 
 pytestmark = pytest.mark.gpu
@@ -37,22 +37,6 @@ def orc():
     return oracle
 
 
-def _reduce(f, stride, nblk=16):
-    n = f.shape[0]
-    b = n // nblk
-    f64 = f.astype(np.float64).reshape(nblk, b, nblk, b)
-    return np.ascontiguousarray(f[::stride, ::stride]), np.stack([f64.sum(axis=(1, 3)), (f64 * f64).sum(axis=(1, 3))])
-
-
-def _check_golden(got, gold, name, stride, tol):
-    sub, blk = _reduce(got, stride)
-    assert rel_l2(sub, gold[f"{name}_sub"]) < tol, (name, rel_l2(sub, gold[f"{name}_sub"]))
-    # the full field enters through the block sums of squares (64 x 64 or 256 x 256 points each)
-    assert rel_l2(blk[1], gold[f"{name}_blk"][1]) < 2 * tol, (name, "block sums of squares")
-    scale = np.sqrt(gold[f"{name}_blk"][1].sum() * got.size)          # |sum| <= sqrt(N * sum of squares)
-    assert np.abs(blk[0] - gold[f"{name}_blk"][0]).max() < tol * scale, (name, "block sums")
-
-
 # ---- configs[1]: Kuo et al. 2004 binary vortex at 1024^2, reference dt = 3 s -------------------------------------------
 def test_kuo1024_one_step_vs_reference_binary_and_oracle(xfb, orc):
     gold = np.load(os.path.join(GOLDEN, "ref_kuo1024.npz"))
@@ -66,7 +50,7 @@ def test_kuo1024_one_step_vs_reference_binary_and_oracle(xfb, orc):
     o.step(1, 3.0)
     for name, which in (("vort", xfb.capi.VORT), ("psi", xfb.capi.PSI), ("u", xfb.capi.U), ("v", xfb.capi.V)):
         got = b.get_field(which)
-        _check_golden(got, gold, f"{name}_1", 4, 1e-5)                    # unmodified reference main.cpp
+        check_golden(got, gold, f"{name}_1", 4, 1e-5)                    # unmodified reference main.cpp
         assert rel_l2(got, o.get_field(which)) < 1e-5, name               # restatement, full field
     assert rel_l2(b.get_spectrum(), o.get_spectrum()) < 1e-5
     b.close()
@@ -78,7 +62,7 @@ def test_kuo1024_thousand_steps_vs_reference_binary(xfb):
     b = xfb.Backend(n)
     b.set_vorticity(gold["init"])
     b.step(1000, 3.0)
-    _check_golden(b.get_field(xfb.capi.VORT), gold, "vort_1000", 4, 1e-3)
+    check_golden(b.get_field(xfb.capi.VORT), gold, "vort_1000", 4, 1e-3)
     b.close()
 
 
@@ -96,7 +80,7 @@ def test_elliptic4096_one_step_vs_reference_binary_and_oracle(xfb, orc):
     assert rel_l2(b.get_spectrum(), o.get_spectrum()) < 1e-5
     for name, which in (("vort", xfb.capi.VORT), ("u", xfb.capi.U)):
         got = b.get_field(which)
-        _check_golden(got, gold, f"{name}_1", 16, 1e-5)
+        check_golden(got, gold, f"{name}_1", 16, 1e-5)
         assert rel_l2(got, o.get_field(which)) < 1e-5, name
     for which in (xfb.capi.PSI, xfb.capi.V):
         assert rel_l2(b.get_field(which), o.get_field(which)) < 1e-5, which

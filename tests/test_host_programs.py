@@ -1,5 +1,6 @@
 """Host C++ programs: generators byte-identical to the reference (CPU), main.out / invert_pres.out against
-the unmodified reference binaries on the same input (GPU)."""
+the reference main.cpp's record files on the same input (GPU): stored in tests/golden/ref_records.npz
+(tests/golden/make_golden_records.py), and every full field against the CPU restatement run live."""
 import hashlib
 import json
 import os
@@ -9,11 +10,36 @@ import tempfile
 import numpy as np
 import pytest
 
-from conftest import rel_l2
+from conftest import check_golden, rel_l2
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "xlab_fftbarotropic_b200", "bin")
 GOLD = os.path.join(ROOT, "tests", "golden")
+KINDS = ("vort", "psi", "u", "v")
+
+
+def _reference_records(v0, n, dt, steps, rec):
+    """{(kind, step): field} of the reference main.cpp's record files, from the CPU restatement (which writes them bit
+    for bit, tests/test_oracle.py)"""
+    from oracle import oracle as orc
+    o = orc.Oracle(n)
+    o.set_vorticity(v0)
+    out = {}
+    for s in range(steps):
+        if s % rec == 0:
+            for kind in KINDS:
+                out[(kind, s)] = o.get_field(getattr(orc, kind.upper()))
+        o.step(1, dt)
+    return out
+
+
+def _check_records(d, tag, ref, stride, tol=1e-5):
+    """main.out's record files in `d` against ref_records.npz[<tag>_<kind>_<step>] and the full restatement fields"""
+    gold = np.load(os.path.join(GOLD, "ref_records.npz"))
+    for (kind, s), exp in sorted(ref.items()):
+        got = np.fromfile(os.path.join(d, f"output/{kind}_step_{s}.bin"), dtype="<f4").reshape(exp.shape)
+        check_golden(got, gold, f"{tag}_{kind}_{s}", stride, tol)         # the reference binary's record file
+        assert rel_l2(got, exp) < tol, (kind, s)                          # the restatement, full field
 
 
 def test_generators_byte_identical_to_reference():
@@ -130,11 +156,10 @@ def test_script_recipe_forcing():
 
 @pytest.mark.gpu
 def test_main_out_matches_reference_binary():
-    from oracle import oracle as orc
     n, steps, rec = 256, 5, 2
     g = np.load(os.path.join(GOLD, "ref_n256.npz"))
     v0 = g["elliptic_init"]
-    ref = orc.run_reference_main(v0, n, 3.0, steps, rec)
+    ref = _reference_records(v0, n, 3.0, steps, rec)
     with tempfile.TemporaryDirectory() as d:
         os.makedirs(os.path.join(d, "input"))
         os.makedirs(os.path.join(d, "output"))
@@ -146,18 +171,14 @@ def test_main_out_matches_reference_binary():
         log = [ln.strip() for ln in open(os.path.join(d, "log"))]
         want = [f"output/{k}_step_{s}.bin" for s in (0, 2, 4) for k in ("vort_src_input", "vort", "psi", "u", "v")]
         assert log == want                                   # same files, same order as the reference's log
-        for s in (0, 2, 4):
-            for k in ("vort", "psi", "u", "v"):
-                got = np.fromfile(os.path.join(d, f"output/{k}_step_{s}.bin"), dtype="<f4").reshape(n, n)
-                assert rel_l2(got, ref[(k, s)]) < 1e-5, (k, s)
+        _check_records(d, "n256", ref, 8)
 
 
 @pytest.mark.gpu
 def test_example_sh_default_grid_768():
     """test/01-runtest/example.sh with the reference's compile-time defaults: makefield-elliptic-vortex.out writes
     input/initial_vorticity.bin at NPTS = 768 (src/configuration.hpp:18), main.out runs it with no size flag;
-    compared file by file with the UNMODIFIED reference binary built at 768 (shortened to 6 steps, record every 3)."""
-    from oracle import oracle as orc
+    compared file by file with the reference's record files at 768 (shortened to 6 steps, record every 3)."""
     n, steps, rec = 768, 6, 3
     with tempfile.TemporaryDirectory() as d:
         os.makedirs(os.path.join(d, "input"))
@@ -166,13 +187,10 @@ def test_example_sh_default_grid_768():
         v0 = np.fromfile(os.path.join(d, "input", "initial_vorticity.bin"), dtype="<f4")
         assert v0.size == n * n
         v0 = v0.reshape(n, n)
-        ref = orc.run_reference_main(v0, n, 3.0, steps, rec)
+        ref = _reference_records(v0, n, 3.0, steps, rec)
         r = subprocess.run([os.path.join(BIN, "main.out"), "-t", str(steps), "-r", str(rec)], cwd=d, capture_output=True, text=True)
         assert r.returncode == 0, r.stderr
-        for s in (0, 3):
-            for k in ("vort", "psi", "u", "v"):
-                got = np.fromfile(os.path.join(d, f"output/{k}_step_{s}.bin"), dtype="<f4").reshape(n, n)
-                assert rel_l2(got, ref[(k, s)]) < 1e-5, (k, s)
+        _check_records(d, "n768", ref, 24)
 
 
 @pytest.mark.gpu
