@@ -104,4 +104,10 @@ def kuo2004(n):
     return data.astype(np.float32)
 
 
+def wave_source(n):
+    """a smooth forcing term for the source path of the stepper: 2e-8 sin(2 pi 3 x) cos(2 pi 5 y), x, y in [0, 1)"""
+    x = np.arange(n, dtype=np.float32) / n
+    return (2e-8 * np.sin(2 * np.pi * 3 * x)[:, None] * np.cos(2 * np.pi * 5 * x)[None, :]).astype(np.float32)
+
+
 GENERATORS = {"elliptic": elliptic, "const": const_vortex, "gaussian": gaussian, "kuo2004": kuo2004}

@@ -1,6 +1,6 @@
 """GPU parity AT THE SIZES bench.py MEASURES (BASELINE.json configs[1..4], the 8192^2 headline and the 16384^2 slab grid).
 
-The kernels that produce the benchmark numbers at 4096 / 8192 / 16384 (tensor-memory parks, TMA box ring, first-generation
+The kernels that produce the benchmark numbers at 4096 / 8192 / 16384 (tensor-memory parks, TMA box ring, two-level
 16384 lines) are different template instances from the ones the <= 2048 tests exercise, so the reference loop
 /root/reference/src/main.cpp:146-317 is checked here on nonlinear fields at those sizes:
 

@@ -1,15 +1,15 @@
 """GPU checks at BASELINE.json's full sizes (4096^2, 8192^2) that complement the oracle comparisons of
-tests/test_headline_parity.py: size-independent properties of the reference algorithm, and agreement of the kernel
-generations with one another.
+tests/test_headline_parity.py: size-independent properties of the reference algorithm, and forced steps of the default
+kernels against their variants and the oracle.
 
   * KAT-3 linear decay (SURVEY.md section 4): a single mode has zero Jacobian, so one RK4 step multiplies a mode
     inside the dealiasing circle by 1 + z + z^2/2 + z^3/6 + z^4/24, z = -nu |k|^2 dt, and leaves a mode outside
     the circle untouched (the mask is applied to the tendency only, main.cpp:296-312).
   * KAT-5 invariants: mode (0,0) is constant, enstrophy does not grow.
-  * the second-generation kernels (rowpair / colt, TMA-staged, persistent) must reproduce the first-generation
-    ones (XFB_ROW_SINGLE=1 XFB_COL_GEN1=1, the kernels 16384-point lines run on) and both park variants of K-ROW
-    (XFB_ROW_TMEM=0/1) to float32 rounding: the knobs are read once per process, so each variant runs in its own
-    interpreter.
+  * two forced RK4 steps at 1024^2 ... 16384^2: the default kernels must reproduce both park variants of K-ROW
+    (XFB_ROW_TMEM=0/1, <= 8192) and, at 4096, the two-level K-COL of the 16384 grid (XFB_COL_2L=1) against colt_kernel
+    to float32 rounding -- the knobs are read once per process, so each variant runs in its own interpreter -- and
+    the oracle to north_star's one-step tolerance, 1e-5.
 """
 import os
 import subprocess
@@ -106,8 +106,7 @@ import fields, xlab_fftbarotropic_b200 as xfb
 n = {n}
 b = xfb.Backend(n)
 b.set_vorticity(fields.elliptic(n))
-x = np.arange(n, dtype=np.float32) / n
-b.set_source((2e-8 * np.sin(2 * np.pi * 3 * x)[:, None] * np.cos(2 * np.pi * 5 * x)[None, :]).astype(np.float32))   # the forcing path too
+b.set_source(fields.wave_source(n))   # the forcing path too
 b.step(2, {dt})
 np.save({out!r}, b.get_spectrum())
 """
@@ -122,19 +121,29 @@ def _run_variant(n, dt, env, out):
 
 
 @pytest.mark.parametrize("n,dt", [(1024, 3.0), (4096, 1.0), (8192, 0.5), (16384, 0.25)])
-def test_kernel_generations_agree(n, dt, tmp_path):
+def test_forced_steps_kernel_variants_and_oracle(n, dt, tmp_path):
     ref = _run_variant(n, dt, {}, str(tmp_path / "default.npy"))
     assert np.isfinite(ref.view(np.float32)).all()
-    # K-ROW with tensor-memory parks is the default at 8192 only: force it on and off everywhere
-    variants = [{"XFB_ROW_SINGLE": "1", "XFB_COL_GEN1": "1"}, {"XFB_ROW_TMEM": "1"}, {"XFB_ROW_TMEM": "0"}]
+    variants = []
+    if n <= 8192:
+        # K-ROW with tensor-memory parks is the default at >= 4096 only: force it on and off everywhere
+        variants = [{"XFB_ROW_TMEM": "1"}, {"XFB_ROW_TMEM": "0"}]
     if n == 4096:
         variants.append({"XFB_COL_2L": "1"})          # the two-level K-COL of the 16384 grid, forced onto 4096-point columns
-    if n == 16384:
-        # the two-level kernels of 16384-point lines (defaults) against the first-generation ones, one at a time and both
-        variants = [{"XFB_COL_GEN1": "1"}, {"XFB_ROW_2L": "0"}, {"XFB_COL_GEN1": "1", "XFB_ROW_2L": "0"}]
     for env in variants:
         got = _run_variant(n, dt, env, str(tmp_path / "variant.npy"))
         assert rel_l2(got, ref) < 2e-6, (env, rel_l2(got, ref))
+    if n == 16384:
+        import psutil
+        if psutil.virtual_memory().available < 48 * 2 ** 30:
+            pytest.skip("the 16384^2 oracle needs ~30 GiB of host memory")
+    from oracle import oracle as orc
+    orc.set_threads(0)        # the shim FFT's line loops on all host cores; results do not depend on the thread count
+    o = orc.Oracle(n)
+    o.set_vorticity(fields.elliptic(n))
+    o.set_source(fields.wave_source(n))
+    o.step(2, dt)
+    assert rel_l2(ref, o.get_spectrum()) < 1e-5
 
 
 def test_one_step_against_oracle_2048():

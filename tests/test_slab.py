@@ -186,42 +186,6 @@ def test_loopback_team_matches_single_gpu(n, p, c):
     team.close()
 
 
-_FUSED_COL = r"""
-import sys, numpy as np
-sys.path.insert(0, {root!r}); sys.path.insert(0, {root!r} + "/tests")
-import fields, xlab_fftbarotropic_b200 as xfb
-n, p, c = {n}, {p}, {c}
-v0 = fields.kuo2004(n)
-team = xfb.LoopbackTeam(n, p, c)
-team.set_vorticity(v0)
-team.step(3, 3.0)
-np.savez({out!r}, vort=team.get_field(xfb.capi.VORT), u=team.get_field(xfb.capi.U), psi=team.get_field(xfb.capi.PSI))
-"""
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("n,p,c", [(512, 2, 2), (1024, 8, 1)])
-def test_loopback_fused_column_to_row_exchange(n, p, c, tmp_path):
-    """The fused column -> row exchange (K-COL storing every product row straight into its owner's receive array) is
-    served by the first-generation column kernel -- the one 16384-point columns run on.  Forcing that kernel
-    (XFB_COL_GEN1=1) exercises the fused stores (opt-in, XFB_SLAB_FUSED_COL=1) on small grids: the result must be
-    bit-identical to the same kernels exchanging through local arrays and copies."""
-    import subprocess
-    import sys
-    import os
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = {}
-    for tag, env in (("fused", {"XFB_COL_GEN1": "1", "XFB_SLAB_FUSED_COL": "1"}), ("copies", {"XFB_COL_GEN1": "1", "XFB_SLAB_FUSED_COL": "0"})):
-        out = str(tmp_path / f"{tag}.npz")
-        e = dict(os.environ)
-        e.update(env)
-        subprocess.run([sys.executable, "-c", _FUSED_COL.format(root=root, n=n, p=p, c=c, out=out)], check=True, env=e, timeout=600)
-        res[tag] = np.load(out)
-    for k in ("vort", "u", "psi"):
-        assert np.isfinite(res["fused"][k]).all()
-        assert np.array_equal(res["fused"][k], res["copies"][k]), k
-
-
 @pytest.mark.gpu
 def test_loopback_diagnostics_and_keff_histograms():
     """slab handles: both strain diagnostics from one set of second derivatives, and the effective-diffusivity histograms

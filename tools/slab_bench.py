@@ -97,7 +97,7 @@ def run(args):
 
     sb = xfb.SlabBackend(n, rank, world, new_id(), nchunks=args.chunks, device=local_rank)
     transport = sb.transport
-    fused_rows, fused_cols = bool(sb.fused & 1), bool(sb.fused & 2)
+    fused_rows = bool(sb.fused)
     stream = torch.cuda.ExternalStream(sb.stream, device=local_rank)
 
     # ---- 1 + 2: check against the single-GPU path on THIS grid, and T1 -----------------------------------------------
@@ -248,13 +248,10 @@ def run(args):
         nv_total = 20.0 * 4.0 * G / world * (world - 1) / world if world > 1 else 0.0
         # what the communication stream itself carries: the row->column array of each stage is stored into peer memory
         # by K-ROW (fused), so only the four column->row arrays per stage remain there
-        nv_comm = nv_total * ((16.0 if not fused_cols else 0.0) + (0.0 if fused_rows else 4.0)) / 20.0
+        nv_comm = nv_total * (16.0 + (0.0 if fused_rows else 4.0)) / 20.0
         a2a_step = a2a_ms / args.steps
         if world > 1:
-            if fused_rows and fused_cols:
-                limiter = (f"per-rank kernels incl. their NVLink stores (K-ROW spans {row_ms / args.steps:.2f} ms + K-COL spans "
-                           f"{col_ms / args.steps:.2f} ms per step); the communication stream carries only the phase barriers")
-            elif a2a_step > 0.75 * per_step:
+            if a2a_step > 0.75 * per_step:
                 limiter = (f"NVLink exchange: the communication stream is busy {a2a_step:.2f} of {per_step:.2f} ms per step "
                            f"({nv_comm / 1e9:.2f} GB per GPU and direction)")
             else:

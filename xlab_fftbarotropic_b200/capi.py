@@ -317,16 +317,13 @@ class SlabBackend(Backend):
     @property
     def transport(self):
         t = {0: "none", 1: "nccl send/recv", 2: "p2p copy engines (CUDA IPC)", 3: "p2p SM push kernel (CUDA IPC)"}[int(self._L.xfb_slab_transport(self._h))]
-        fused = int(self._L.xfb_slab_fused(self._h))
-        if fused == 3:
-            t = "both transposes fused into the kernels: K-ROW and K-COL store into peer memory over NVLink (CUDA IPC), row->column fused, column->row fused"
-        elif fused & 1:
+        if self.fused:
             t += " for column->row, row->column fused into K-ROW (stores into peer memory)"
         return t
 
     @property
     def fused(self):
-        """bit 0: row->column transpose fused into K-ROW, bit 1: column->row transpose fused into K-COL"""
+        """1: row->column transpose fused into K-ROW, else 0"""
         return int(self._L.xfb_slab_fused(self._h))
 
     def a2a_read(self):

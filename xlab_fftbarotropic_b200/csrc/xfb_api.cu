@@ -658,8 +658,7 @@ extern "C" int xfb_set_tracer(xfb_handle h, int member, const float *tracer, flo
 {
     if (check_member(h, member)) return XFB_E_ARG;
     if (!tracer) return fail(XFB_E_ARG, "null tracer");
-    static const bool gen1_col = getenv("XFB_COL_GEN1") && atoi(getenv("XFB_COL_GEN1")) != 0;
-    if (!fused_diag_ok(h) && !h->generic && h->nranks == 1 && !(h->nx == 16384 && col_two_level(h->nx) && !gen1_col))
+    if (!fused_diag_ok(h) && !h->generic && h->nranks == 1 && h->nx != 16384)
         return fail(XFB_E_SIZE, "the passive tracer needs the fused kernels (power-of-two grids), a generic mixed-radix grid, or a slab-decomposed handle");
     CK(cudaSetDevice(h->device));
     const size_t sb = sizeof(cpx) * h->hpad * h->batch;
@@ -966,10 +965,8 @@ extern "C" int xfb_wait_field(xfb_handle h, int ticket)
 // multipliers.  Replaces 6-9 pointwise passes, 3 column and 3 row transforms of the record path.
 static bool fused_diag_ok(xfb_handle h)
 {
-    // the A/B knobs that select the first-generation kernels also select the unfused record path
-    static const bool off = (getenv("XFB_DIAG_UNFUSED") && atoi(getenv("XFB_DIAG_UNFUSED")) != 0) ||
-                            (getenv("XFB_COL_GEN1") && atoi(getenv("XFB_COL_GEN1")) != 0) ||
-                            (getenv("XFB_ROW_SINGLE") && atoi(getenv("XFB_ROW_SINGLE")) != 0);
+    // XFB_DIAG_UNFUSED=1: every grid takes the unfused record path that 16384 and generic grids take (A/B knob)
+    static const bool off = getenv("XFB_DIAG_UNFUSED") && atoi(getenv("XFB_DIAG_UNFUSED")) != 0;
     return !off && !h->generic && h->nranks == 1 && h->nx <= 8192 && h->ny <= 8192;
 }
 

@@ -15,7 +15,7 @@ static int env_int(const char *name, int dflt)
 
 // Tile width of the K-COL-private state arrays (z0 / zk / acc are tile-major, one column group per block) = the
 // number of columns the stepper transforms together: ColTCfg<NX>::FW (1 at 8192: a staged two-column tile is
-// transformed one column at a time); 16384 runs the first-generation kernel with one column per CTA.
+// transformed one column at a time); 16384 runs the two-level kernel with one column per CTA.
 int col_tile_width(int nx)
 {
     switch (nx) {
@@ -27,11 +27,12 @@ int col_tile_width(int nx)
     }
 }
 
+// the stepper's K-COL on the two-level kernel: always at 16384; XFB_COL_2L=1 also puts 4096-point columns on it (a test
+// knob that checks the 16384 kernel against colt_kernel)
 bool col_two_level(int nx)
 {
-    static const bool gen1 = env_int("XFB_COL_GEN1", 0) != 0;
-    static const int two_level = env_int("XFB_COL_2L", -1);
-    return !gen1 && ((nx == 16384 && two_level != 0) || (nx == 4096 && two_level > 0));
+    static const bool at_4096 = env_int("XFB_COL_2L", 0) == 1;
+    return nx == 16384 || (nx == 4096 && at_4096);
 }
 
 // ---- tensor maps for the TMA tiles of colt_kernel ------------------------------------------------------------
@@ -96,7 +97,7 @@ static int launch_colt_t(const ColParams &p, int batch, cudaStream_t st)
     return (int)cudaGetLastError();
 }
 
-// two-level K-COL (xfb_col2l.cuh): columns of 16384 points (and 4096 under XFB_COL_2L=1, an A/B and test knob)
+// two-level K-COL (xfb_col2l.cuh): columns of 16384 points (and 4096 under XFB_COL_2L=1, a test knob)
 template <int NX, int MODE>
 static int launch_col2l_t(const ColParams &p, int batch, cudaStream_t st)
 {
@@ -133,78 +134,57 @@ static int launch_colt_n(int mode, const ColParams &p, int batch, cudaStream_t s
     return mode == COL_STEP ? launch_colt_t<NX, COL_STEP>(p, batch, st) : launch_colt_t<NX, COL_PRO>(p, batch, st);
 }
 
-template <int NX, int W, int MODE, bool PEER = false>
+template <int NX, int W, int MODE>
 static int launch_col_t(const ColParams &p, int batch, cudaStream_t st)
 {
     typedef ColCfg<NX, W> C;
     static PerDeviceInt cfg;
     int err = 0;
-    if (cfg.get([&](int *e) { return resident_ctas(col_kernel<NX, W, MODE, PEER>, C::THREADS, C::SMEM, 0, e); }, &err) <= 0) return err;
+    if (cfg.get([&](int *e) { return resident_ctas(col_kernel<NX, W, MODE>, C::THREADS, C::SMEM, 0, e); }, &err) <= 0) return err;
     dim3 grid(p.pitch / W, batch);
-    col_kernel<NX, W, MODE, PEER><<<grid, C::THREADS, C::SMEM, st>>>(p);
+    col_kernel<NX, W, MODE><<<grid, C::THREADS, C::SMEM, st>>>(p);
     return (int)cudaGetLastError();
 }
-
-// fused column -> row exchange (ColParams::peer_rows > 0): instantiated for the slab grid of BASELINE.json (16384) and for
-// the two small sizes tests/test_slab.py forces onto this kernel
-template <int NX>
-constexpr bool col_peer_size() { return NX == 16384 || NX == 512 || NX == 1024; }
 
 template <int NX, int W>
 static int launch_col_n(int mode, const ColParams &p, int batch, cudaStream_t st)
 {
-    if (p.peer_rows > 0) {
-        if constexpr (col_peer_size<NX>()) {
-            switch (mode) {
-            case COL_INV: return launch_col_t<NX, W, COL_INV, true>(p, batch, st);
-            case COL_STEP: return launch_col_t<NX, W, COL_STEP, true>(p, batch, st);
-            case COL_PRO: return launch_col_t<NX, W, COL_PRO, true>(p, batch, st);
-            }
-        }
-        return (int)cudaErrorNotSupported;
-    }
-    switch (mode) {
-    case COL_FWD: return launch_col_t<NX, W, COL_FWD>(p, batch, st);
-    case COL_INV: return launch_col_t<NX, W, COL_INV>(p, batch, st);
-    case COL_STEP: return launch_col_t<NX, W, COL_STEP>(p, batch, st);
-    case COL_PRO: return launch_col_t<NX, W, COL_PRO>(p, batch, st);
-    }
-    return (int)cudaErrorInvalidValue;
+    return mode == COL_FWD ? launch_col_t<NX, W, COL_FWD>(p, batch, st) : launch_col_t<NX, W, COL_INV>(p, batch, st);
 }
 
 int launch_col(int nx, int mode, const ColParams &p, int batch, cudaStream_t st)
 {
-    // the stepper's modes run on the TMA-staged persistent kernel (XFB_COL_GEN1=1: first-generation kernel, A/B knob)
-    static const bool gen1 = env_int("XFB_COL_GEN1", 0) != 0;
-    // XFB_COL_2L: 1 = two-level K-COL on 16384- and 4096-point columns, 0 = first-generation kernel at 16384 (A/B knob)
-    if ((mode == COL_STEP || mode == COL_PRO) && p.peer_rows == 0 && col_two_level(nx)) {
+    // the operator tier's plain transforms
+    if (mode == COL_FWD || mode == COL_INV) {
+        switch (nx) {
+        case 256: return launch_col_n<256, 4>(mode, p, batch, st);
+        case 512: return launch_col_n<512, 4>(mode, p, batch, st);
+        case 1024: return launch_col_n<1024, 4>(mode, p, batch, st);
+        case 2048: return launch_col_n<2048, 4>(mode, p, batch, st);
+        case 4096: return launch_col_n<4096, 2>(mode, p, batch, st);
+        case 8192: return launch_col_n<8192, 1>(mode, p, batch, st);
+        case 16384: return launch_col_n<16384, 1>(mode, p, batch, st);
+        }
+        return (int)cudaErrorInvalidValue;
+    }
+    // the stepper's modes: two-level kernel on 16384-point columns, TMA-staged persistent kernel on shorter ones
+    if ((mode == COL_STEP || mode == COL_PRO) && col_two_level(nx)) {
         if (nx == 16384)
             return mode == COL_STEP ? launch_col2l_t<16384, COL_STEP>(p, batch, st) : launch_col2l_t<16384, COL_PRO>(p, batch, st);
         return mode == COL_STEP ? launch_col2l_t<4096, COL_STEP>(p, batch, st) : launch_col2l_t<4096, COL_PRO>(p, batch, st);
     }
-    if ((mode == COL_TSTEP || mode == COL_TPRO) && nx == 16384 && col_two_level(nx))     // passive tracer on the 16384 grid
-        return mode == COL_TSTEP ? launch_col2l_t<16384, COL_TSTEP>(p, batch, st) : launch_col2l_t<16384, COL_TPRO>(p, batch, st);
-    const bool colt_only = (mode == COL_DIAG || mode == COL_FWDT || mode == COL_TSTEP || mode == COL_TPRO);
-    if (colt_only && (gen1 || nx > 8192)) return (int)cudaErrorNotSupported;
-    if ((mode == COL_STEP || mode == COL_PRO || colt_only) && !gen1) {
-        switch (nx) {
-        case 256: return launch_colt_n<256>(mode, p, batch, st);
-        case 512: return launch_colt_n<512>(mode, p, batch, st);
-        case 1024: return launch_colt_n<1024>(mode, p, batch, st);
-        case 2048: return launch_colt_n<2048>(mode, p, batch, st);
-        case 4096: return launch_colt_n<4096>(mode, p, batch, st);
-        case 8192: return launch_colt_n<8192>(mode, p, batch, st);
-        default: break;
-        }
+    if (nx == 16384) {      // passive tracer on the 16384 grid; the diagnostics modes have no 16384 kernel
+        if (mode == COL_TSTEP || mode == COL_TPRO)
+            return mode == COL_TSTEP ? launch_col2l_t<16384, COL_TSTEP>(p, batch, st) : launch_col2l_t<16384, COL_TPRO>(p, batch, st);
+        return (int)cudaErrorNotSupported;
     }
     switch (nx) {
-    case 256: return launch_col_n<256, 4>(mode, p, batch, st);
-    case 512: return launch_col_n<512, 4>(mode, p, batch, st);
-    case 1024: return launch_col_n<1024, 4>(mode, p, batch, st);
-    case 2048: return launch_col_n<2048, 4>(mode, p, batch, st);
-    case 4096: return launch_col_n<4096, 2>(mode, p, batch, st);
-    case 8192: return launch_col_n<8192, 1>(mode, p, batch, st);
-    case 16384: return launch_col_n<16384, 1>(mode, p, batch, st);
+    case 256: return launch_colt_n<256>(mode, p, batch, st);
+    case 512: return launch_colt_n<512>(mode, p, batch, st);
+    case 1024: return launch_colt_n<1024>(mode, p, batch, st);
+    case 2048: return launch_colt_n<2048>(mode, p, batch, st);
+    case 4096: return launch_colt_n<4096>(mode, p, batch, st);
+    case 8192: return launch_colt_n<8192>(mode, p, batch, st);
     }
     return (int)cudaErrorInvalidValue;
 }

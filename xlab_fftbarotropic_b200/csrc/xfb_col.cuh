@@ -1,7 +1,10 @@
 // xfb_col.cuh -- K-COL: transforms along x (the strided direction) on tiles of W adjacent
 // spectral columns, with every pointwise spectral operator of the reference fused around them.
+// This header holds the parameter block and the column transform shared by every K-COL kernel, and col_kernel, the
+// plain forward and inverse column transforms of the operator tier (COL_FWD / COL_INV).
 //
-// One launch of COL_STEP replaces, for its column tile (file:line in /root/reference/src):
+// One launch of COL_STEP (colt_kernel, xfb_colt.cuh; col2l_kernel, xfb_col2l.cuh) replaces, for its column tile
+// (file:line in /root/reference/src):
 //   first-dimension half of the r2c of the tendency                  main.cpp:237
 //   fop.laplacian + `dvortdt_c += lvort_c * NU`                      main.cpp:148,240-243 ; fftwfop.cpp:105-110
 //   fop.dealiase -> rk_k                                             main.cpp:296-306     ; fftwfop.cpp:119-124
@@ -51,21 +54,11 @@ struct ColParams {
     float dt_stage;       // dt/2, dt/2, dt for stages 1..3
     int stage;            // 1..4 ; COL_DIAG: product set (0 strain, 1 tracer, 2 + field id: one record field)
     int nfields;          // COL_DIAG: number of products (3 or 1)
-    // slab-decomposed runs, fused column -> row exchange (peer_rows > 0): the x-inverse-transformed products are not written
-    // to the local t_out arrays for a push kernel to move afterwards; every row is stored straight into the receive
-    // array of the rank that owns it (CUDA-IPC peer mapping over NVLink, or this rank's own).  Rank R owns the rows
-    // [R * peer_rows, (R + 1) * peer_rows); peer_out[R * 4 + f] points at the block of receive array f of rank R that
-    // holds THIS rank's column chunks, peer_chunk_off selects the chunk of this launch; inside the block the rows are in
-    // the pair layout with pitch `pitch` (= columns per chunk).
     // slab-decomposed runs, two-level kernel (xfb_col2l.cuh): the 16-byte pieces [self_piece0, self_piece0 + self_pieces) of a
     // column -- the row pairs this rank owns itself -- go straight into this rank's own receive arrays (self_out[f] points
     // at the block of this launch's chunk), so the exchange has no self-copy to do; self_pieces == 0: everything to t_out
     int self_piece0, self_pieces;
     cpx *self_out[4];
-    int peer_rows;        // 0: local output
-    int peer_rows_shift;  // log2(peer_rows)
-    long long peer_chunk_off;
-    cpx *peer_out[16 * 4];
 };
 
 template <int NX, int W>
@@ -84,21 +77,6 @@ struct ColCfg {
 __device__ __forceinline__ size_t pair_base(const int t, const int j, const int pitch)
 {
     return ((size_t)(t >> 1) * (size_t)pitch + (size_t)j) * 2 + (size_t)(t & 1);
-}
-
-// address of output element (row i = t + k * G, tile column jc) of product f: local pair-layout array, or the owning
-// rank's receive array.  G divides peer_rows (checked on the host), so the owner of row t + k * G is that of row k * G:
-// uniform over the CTA, one parameter-space lookup.
-// PEER is a template parameter: the local path must compile to one base address + constant offsets (a run-time test of
-// p.peer_rows in the store loops cost the single-GPU 16384^2 step 20 %: 36.8 -> 44.9 ms).
-template <int NX, bool PEER>
-__device__ __forceinline__ cpx *col_out_addr(const ColParams &p, const int f, cpx *local_base, const int t, const int jc, const int k)
-{
-    constexpr int G = NX / 16;
-    if (!PEER) return local_base + pair_base(t, jc, p.pitch) + (size_t)(k * G) * p.pitch;
-    const int R = (k * G) >> p.peer_rows_shift;
-    const int rl = (t + k * G) & (p.peer_rows - 1);
-    return p.peer_out[R * 4 + f] + p.peer_chunk_off + (((size_t)(rl >> 1) * (size_t)p.pitch + (size_t)jc) * 2 + (size_t)(rl & 1));
 }
 
 
@@ -177,13 +155,16 @@ __device__ __forceinline__ void col_fft(cpx (&v)[NIT][16], cpx *sm, const int (&
     col_fft<NX, W, NIT, ColFftNoHook>(v, sm, t, c, tw, drain_tma, nohook);
 }
 
-template <int NX, int W, int MODE, bool PEER = false>
+template <int NX, int W, int MODE>
 __global__ void __launch_bounds__(ColCfg<NX, W>::THREADS, ColCfg<NX, W>::MINB)
 col_kernel(const ColParams p)
 {
+    static_assert(MODE == COL_FWD || MODE == COL_INV, "col_kernel has the plain transforms only");
     typedef ColCfg<NX, W> C;
     constexpr int G = C::G, NIT = C::NIT;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
+    // the same symbol as col2l_kernel's staging buffer, which TMA needs 128-byte aligned: declarations that disagree
+    // within one translation unit leave the alignment to the order in which the kernels are instantiated
+    extern __shared__ __align__(128) unsigned char smem_raw[];
     cpx *sm = reinterpret_cast<cpx *>(smem_raw);
 
     const int j0 = blockIdx.x * W;
@@ -202,98 +183,21 @@ col_kernel(const ColParams p)
     }
 
     cpx v[NIT][16];
-    // with one butterfly per thread the new stage state stays in registers for the four products
-    constexpr bool KEEP = (NIT == 1) && (MODE == COL_STEP);
-    cpx zkeep[KEEP ? 16 : 1];
-
-    // ------------------------------------------------------------------ forward + epilogue
-    if (MODE == COL_FWD || MODE == COL_STEP) {
+    if (MODE == COL_FWD) {
 #pragma unroll
         for (int it = 0; it < NIT; ++it) {
             const cpx *src = p.jint + moff + pair_base(t[it], j0 + c[it], p.pitch);
 #pragma unroll
             for (int k = 0; k < 16; ++k) v[it][k] = __ldg(src + (size_t)(k * G) * p.pitch);
         }
-        if (MODE == COL_STEP) {
-            // the epilogue operands of this tile: start them towards L2 now, they are needed after the
-            // forward transform (three passes from here)
-            for (int r = threadIdx.x; r < NX; r += C::THREADS) {
-                const size_t e = soff + (size_t)r * srow;
-                prefetch_l2(p.z0 + e);
-                if (p.stage != 1) {
-                    prefetch_l2(p.zk + e);
-                    prefetch_l2(p.acc + e);
-                }
-            }
-        }
         col_fft<NX, W, NIT>(v, sm, t, c, tw);
 #pragma unroll
         for (int it = 0; it < NIT; ++it) {
-            const int j = p.j_base + j0 + c[it];
-            const float kyv = __ldg(p.ky + j);
-            const float ky2 = kyv * kyv;
             const size_t e0 = soff + (size_t)t[it] * srow + c[it];
-            if (MODE == COL_FWD) {
 #pragma unroll
-                for (int k = 0; k < 16; ++k) p.z0[e0 + (size_t)(k * G) * srow] = v[it][k];
-            } else {
-#pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    // operands of eight elements in flight at once
-                    cpx z0v[8], zkv[8], av[8];
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) z0v[q] = p.z0[e0 + (size_t)((8 * h + q) * G) * srow];
-                    if (p.stage != 1) {
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) {
-                            zkv[q] = p.zk[e0 + (size_t)((8 * h + q) * G) * srow];
-                            av[q] = p.acc[e0 + (size_t)((8 * h + q) * G) * srow];
-                        }
-                    } else {
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) { zkv[q] = z0v[q]; av[q] = mk(0.f, 0.f); }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const int k = 8 * h + q;
-                        const int i = t[it] + k * G;
-                        const size_t e = e0 + (size_t)(k * G) * srow;
-                        const cpx X = v[it][k];
-                        // fused path: kx = (signed index) * TWOPI/Lx and -(kx^2 + ky^2) in float32 (<= 2 ulp
-                        // from the reference tables; the operator tier keeps the exact expressions)
-                        const float kxv = (float)signed_row<NX>(t[it], k) * p.kxscale;
-                        const float lap = -fmaf(kxv, kxv, ky2);
-                        // dvortdt_c += (vort_c * laplacian_coe) * NU
-                        const float tx = __fadd_rn(X.x, __fmul_rn(__fmul_rn(zkv[q].x, lap), p.nu));
-                        const float ty = __fadd_rn(X.y, __fmul_rn(__fmul_rn(zkv[q].y, lap), p.nu));
-                        // dealiasing mask: (i^2 + j^2 >= kd) ? 0 : 1 with i reflected above NX/2
-                        const int ii = (i <= NX / 2) ? i : NX - i;
-                        const float m = (ii * ii + j * j >= p.mask_kd_i) ? 0.0f : 1.0f;
-                        const float rx = __fmul_rn(tx, m), ry = __fmul_rn(ty, m);
-                        cpx zn;
-                        if (p.stage == 4) {
-                            zn.x = __fadd_rn(z0v[q].x, __fdiv_rn(__fmul_rn(__fadd_rn(av[q].x, rx), p.dt), 6.0f));
-                            zn.y = __fadd_rn(z0v[q].y, __fdiv_rn(__fmul_rn(__fadd_rn(av[q].y, ry), p.dt), 6.0f));
-                            p.z0[e] = zn;
-                        } else {
-                            // stage 1: acc = r1 ; stages 2,3: acc += 2 r
-                            const cpx an = (p.stage == 1) ? mk(rx, ry)
-                                                          : mk(__fadd_rn(av[q].x, __fmul_rn(2.0f, rx)),
-                                                               __fadd_rn(av[q].y, __fmul_rn(2.0f, ry)));
-                            p.acc[e] = an;
-                            zn.x = __fadd_rn(z0v[q].x, __fmul_rn(rx, p.dt_stage));
-                            zn.y = __fadd_rn(z0v[q].y, __fmul_rn(ry, p.dt_stage));
-                            p.zk[e] = zn;
-                        }
-                        if (KEEP) v[it][k] = zn;
-                    }
-                }
-            }
+            for (int k = 0; k < 16; ++k) p.z0[e0 + (size_t)(k * G) * srow] = v[it][k];
         }
-    }
-
-    // ------------------------------------------------------------------ plain inverse
-    if (MODE == COL_INV) {
+    } else {
 #pragma unroll
         for (int it = 0; it < NIT; ++it) {
             const cpx *src = p.inv_in + moff + j0 + c[it];
@@ -301,59 +205,11 @@ col_kernel(const ColParams p)
             for (int k = 0; k < 16; ++k) v[it][k] = cswap(__ldg(src + (size_t)(t[it] + k * G) * p.pitch));
         }
         col_fft<NX, W, NIT>(v, sm, t, c, tw);
+        cpx *out = p.t_out[0] + moff;
 #pragma unroll
         for (int it = 0; it < NIT; ++it) {
 #pragma unroll
-            for (int k = 0; k < 16; ++k) *col_out_addr<NX, PEER>(p, 0, p.t_out[0] + moff, t[it], j0 + c[it], k) = cswap(v[it][k]);
-        }
-    }
-
-    // ------------------------------------------------------------------ prologue + 4 inverse
-    if (MODE == COL_STEP || MODE == COL_PRO) {
-        // the state this thread just wrote (stage 4 / PRO: z0, else zk): kept in registers (KEEP) or
-        // re-read from L1/L2
-        const cpx *zsrc = (MODE == COL_PRO || p.stage == 4) ? p.z0 : p.zk;
-        if (KEEP) {
-#pragma unroll
-            for (int k = 0; k < 16; ++k) zkeep[k] = v[0][k];
-        }
-#pragma unroll 1
-        for (int f = 0; f < 4; ++f) {
-            if (!KEEP) {
-#pragma unroll
-                for (int it = 0; it < NIT; ++it) {
-                    const cpx *src = zsrc + soff + (size_t)t[it] * srow + c[it];
-#pragma unroll
-                    for (int k = 0; k < 16; ++k) v[it][k] = src[(size_t)(k * G) * srow];
-                }
-            }
-#pragma unroll
-            for (int it = 0; it < NIT; ++it) {
-                const int j = p.j_base + j0 + c[it];
-                const float ky = __ldg(p.ky + j);
-                const float ky2 = ky * ky;
-#pragma unroll
-                for (int k = 0; k < 16; ++k) {
-                    const int i = t[it] + k * G;
-                    const cpx z = KEEP ? zkeep[k] : v[it][k];
-                    const float kx = (float)signed_row<NX>(t[it], k) * p.kxscale;
-                    // f = 0: i kx Z, 1: i ky Z, 2: i ky Psi (u before negation), 3: i kx Psi (v);
-                    // Psi = Z / -(kx^2+ky^2), (0,0) entry divides by 1                 (fftwfop.cpp:43,112-117)
-                    float kk = (f == 0 || f == 3) ? kx : ky;
-                    if (f >= 2) {
-                        const float li = (i == 0 && j == 0) ? 1.0f : -fmaf(kx, kx, ky2);
-                        kk = __fdividef(kk, li);
-                    }
-                    v[it][k] = mk(z.x * kk, -z.y * kk);       // swap(i kk z) = swap(-z.y kk, z.x kk)
-                }
-            }
-            col_fft<NX, W, NIT>(v, sm, t, c, tw);
-            cpx *outp = p.t_out[f];
-#pragma unroll
-            for (int it = 0; it < NIT; ++it) {
-#pragma unroll
-                for (int k = 0; k < 16; ++k) *col_out_addr<NX, PEER>(p, f, outp + moff, t[it], j0 + c[it], k) = cswap(v[it][k]);
-            }
+            for (int k = 0; k < 16; ++k) *(out + pair_base(t[it], j0 + c[it], p.pitch) + (size_t)(k * G) * p.pitch) = cswap(v[it][k]);
         }
     }
 }

@@ -4,9 +4,9 @@
 // Same fusion as colt_kernel<COL_STEP / COL_PRO> (reference loops main.cpp:148,237,240-243,246-251,286-312 and
 // fftwfop.cpp:87-124).  Why a kernel of its own: a column of 16384 complex values is 128 KB -- a two-column TMA tile
 // does not fit in shared memory, a one-column tile has 16-byte rows (the TMA engine then runs at a quarter of its
-// rate), and the first-generation kernel holds two butterflies per thread (NX / 16 = 1024 butterflies on 512 threads):
-// it spills 280 bytes per thread and issues 8-byte accesses (profiles/r02_16384_gen1_ncu_full_summary.txt: 174 M
-// local-memory sectors, 613 M global sectors for 335 M sectors of payload, stall_lg 2.9, 29 % issue slots used).
+// rate), and the first-generation kernel (since removed) held two butterflies per thread (NX / 16 = 1024 butterflies on
+// 512 threads): it spilled 280 bytes per thread and issued 8-byte accesses (profiles/r02_16384_gen1_ncu_full_summary.txt:
+// 174 M local-memory sectors, 613 M global sectors for 335 M sectors of payload, stall_lg 2.9, 29 % issue slots used).
 // Here a thread owns the rows {2m, 2m+1, 2m + NX/2 ... } that one 16-byte piece of the pair layout holds:
 //   forward  (decimation in time):  E = FFT_{NX/2}(x[2n]), O = FFT_{NX/2}(x[2n+1])  -- the two rows of the piece (m = n);
 //            X[k] = E[k] + W^k O[k], X[k + NX/2] = E[k] - W^k O[k]   (W = exp(-2 pi i / NX)): natural order, so the

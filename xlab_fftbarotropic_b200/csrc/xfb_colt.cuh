@@ -1,8 +1,8 @@
 // xfb_colt.cuh -- K-COL of the stepper, second generation: persistent CTAs, every strided (transposed) access
 // done by the TMA engine.
 //
-// Same fusion as col_kernel<COL_STEP / COL_PRO> (xfb_col.cuh; reference loops main.cpp:148,237,240-243,
-// 246-251,286-312 and fftwfop.cpp:87-124), different data movement:
+// The fusion of COL_STEP / COL_PRO listed in xfb_col.cuh (reference loops main.cpp:148,237,240-243,
+// 246-251,286-312 and fftwfop.cpp:87-124), with this data movement:
 //   * a tile is TW adjacent spectral columns x all NX rows.  In the pair layout of the exchange arrays a tile
 //     row pair is one contiguous piece of TW*2 complex values (32 bytes for TW = 2: whole sectors), so a
 //     tile is a 2-D TMA box {TW*2, NX/2}: cp.async.bulk.tensor.2d loads the y-transformed tendency into the

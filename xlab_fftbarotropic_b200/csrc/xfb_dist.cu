@@ -115,19 +115,6 @@ static int build_panel_table(xfb_handle h, cpx *const *recv_of_rank)
         for (int c = 0; c < h->nchunks; ++c) tab[q * h->nchunks + c] = recv_of_rank[q] + (size_t)5 * h->hpad + col_off(h, h->rank, c, 0);
     if (dev_alloc((void **)&h->panel_base_c, sizeof(cpx *) * n)) return XFB_E_CUDA;
     CK(cudaMemcpy(h->panel_base_c, tab.data(), sizeof(cpx *) * n, cudaMemcpyHostToDevice));
-    // Fused column -> row exchange, OPT-IN (XFB_SLAB_FUSED_COL=1): K-COL stores each product row straight into the
-    // receive array tr[f] of the rank that owns the row (array 1 + f of that rank's receive block), at the block of
-    // panels (me, 0 .. nchunks-1).  Served by the first-generation column kernel (the line lengths > 8192 run on it).
-    // Measured on 2 GPUs at 16384^2 it is SLOWER than writing locally and pushing contiguous blocks (41.2 vs 38.1 ms per
-    // step): a one-column tile stores 16-byte pieces, fine for the local L2 but small NVLink packets; the push moves
-    // 2 KB runs.  Kept as an A/B knob (tests/test_slab.py checks it bit for bit).
-    static const bool col_on_knob = getenv("XFB_SLAB_FUSED_COL") && atoi(getenv("XFB_SLAB_FUSED_COL")) != 0;
-    static const bool gen1 = getenv("XFB_COL_GEN1") && atoi(getenv("XFB_COL_GEN1")) != 0;
-    const int G = h->nx / 16;
-    h->fused_col = col_on_knob && (h->nx == 16384 || (gen1 && (h->nx == 512 || h->nx == 1024))) && h->rows % G == 0 &&
-                   (h->rows & (h->rows - 1)) == 0;
-    for (int q = 0; q < h->nranks; ++q)
-        for (int f = 0; f < 4; ++f) h->peer_tr[q][f] = recv_of_rank[q] + (size_t)(1 + f) * h->hpad + row_off(h, h->rank, 0, 0);
     return 0;
 }
 
@@ -231,7 +218,6 @@ static int exchange(Team *T, int dir, cpx *const *row_ptrs_of_rank, cpx *const *
             return flush();
         }
         const int ncs = h0->ncopy;
-        static const bool one_d = getenv("XFB_SLAB_1D") && atoi(getenv("XFB_SLAB_1D")) != 0;     // A/B: plain 1-D copies
         CK(cudaEventRecord(h0->ev_fork, st));
         for (int s = 0; s < ncs; ++s) CK(cudaStreamWaitEvent(h0->copy_stream[s], h0->ev_fork, 0));
         const int pieces = (T->nranks - 1 >= ncs) ? 1 : ncs / (T->nranks - 1);
@@ -249,21 +235,12 @@ static int exchange(Team *T, int dir, cpx *const *row_ptrs_of_rank, cpx *const *
                     // array 0 of the receive block = jint_recv ; chunks c0..c1-1 are rows*cw apart here, NX*cw apart there
                     const cpx *src = row_ptrs_of_rank[0] + row_off(h0, q, c0, r0) + e0;
                     cpx *dst = peer + (size_t)abase * h0->hpad + col_off(h0, me, c0, r0) + e0;
-                    if (one_d) {
-                        for (int c = c0; c < c1; ++c)
-                            CK(cudaMemcpyAsync(dst + (size_t)(c - c0) * h0->nx * h0->pitch, src + (size_t)(c - c0) * h0->rows * h0->pitch,
-                                               wbytes, cudaMemcpyDeviceToDevice, cs));
-                    } else
                     CK(cudaMemcpy2DAsync(dst, sizeof(cpx) * (size_t)h0->nx * h0->pitch, src, sizeof(cpx) * (size_t)h0->rows * h0->pitch,
                                          wbytes, (size_t)(c1 - c0), cudaMemcpyDeviceToDevice, cs));
                 } else {
                     // arrays 1..4 of the receive block = tr[0..3] (or tr[0] alone, na == 1)
                     for (int c = c0; c < c1; ++c) {
-                        if (na == 4 && one_d) {
-                            for (int a = 0; a < 4; ++a)
-                                CK(cudaMemcpyAsync(peer + (size_t)(abase + a) * h0->hpad + row_off(h0, me, c, r0) + e0,
-                                                   col_ptrs_of_rank[a] + col_off(h0, q, c, r0) + e0, wbytes, cudaMemcpyDeviceToDevice, cs));
-                        } else if (na == 4) {
+                        if (na == 4) {
                             const cpx *src = col_ptrs_of_rank[0] + col_off(h0, q, c, r0) + e0;     // t[0]; t[1..3] follow hpad apart
                             cpx *dst = peer + (size_t)abase * h0->hpad + row_off(h0, me, c, r0) + e0;
                             CK(cudaMemcpy2DAsync(dst, sizeof(cpx) * h0->hpad, src, sizeof(cpx) * h0->hpad, wbytes, 4,
@@ -343,14 +320,6 @@ static int launch_col_chunk(xfb_handle h, int mode, int chunk, int stage, float 
         c.self_piece0 = h->rank * (h->rows / 2);
         c.self_pieces = h->rows / 2;
         for (int f = 0; f < 4; ++f) c.self_out[f] = (tracer ? h->trc[f & 1] : h->tr[f]) + row_off(h, h->rank, chunk, 0);
-    }
-    if (h->fused_col && mode != COL_FWD && !tracer) {
-        c.peer_rows = h->rows;
-        c.peer_rows_shift = 0;
-        while ((1 << c.peer_rows_shift) < h->rows) ++c.peer_rows_shift;
-        c.peer_chunk_off = (long long)chunk * h->rows * h->pitch;          // panels (me, chunk): rows * cw elements each
-        for (int q = 0; q < h->nranks; ++q)
-            for (int f = 0; f < 4; ++f) c.peer_out[q * 4 + f] = h->peer_tr[q][f];
     }
     CKL(h, launch_col(h->nx, mode, c, 1, h->stream));
     return 0;
@@ -442,19 +411,6 @@ static int cols_then_exchange(Team *T, F produce, GC col_of, GR row_of, int na, 
     cpx *rp[16 * 4], *cp[16 * 4];
     for (int l = 0; l < T->nlocal; ++l)
         for (int a = 0; a < na; ++a) { rp[l * na + a] = row_of(T->local[l], a); cp[l * na + a] = col_of(T->local[l], a); }
-    if (h0->fused_col && abase == 1) {
-        // fused exchange: the kernels have stored into the owners' receive arrays themselves; what is left is the barrier
-        for (int l = 0; l < T->nlocal; ++l)
-            for (int c = 0; c < C; ++c)
-                if (int e = produce(T->local[l], c)) return e;
-        if (T->loopback) return 0;
-        CK(cudaEventRecord(h0->ev_chunk[0], h0->stream));
-        CK(cudaStreamWaitEvent(h0->comm_stream, h0->ev_chunk[0], 0));
-        if (int e = phase_barrier(T, h0->comm_stream)) return e;
-        CK(cudaEventRecord(h0->ev_comm[1], h0->comm_stream));
-        CK(cudaStreamWaitEvent(h0->stream, h0->ev_comm[1], 0));
-        return 0;
-    }
     if (T->loopback) {
         for (int l = 0; l < T->nlocal; ++l)
             for (int c = 0; c < C; ++c)
@@ -886,7 +842,7 @@ extern "C" int xfb_slab_transport(xfb_handle h)
 extern "C" int xfb_slab_fused(xfb_handle h)
 {
     if (!h || h->nranks <= 1) return 0;
-    return (h->panel_base ? 1 : 0) | (h->fused_col ? 2 : 0);       // bit 0: row -> column in K-ROW, bit 1: column -> row in K-COL
+    return h->panel_base ? 1 : 0;
 }
 
 extern "C" int xfb_profile_read_a2a(xfb_handle h, double *a2a_ms, long long *exchanges)

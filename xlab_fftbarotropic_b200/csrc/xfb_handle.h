@@ -88,8 +88,6 @@ struct xfb_handle_s {
     xfb::cpx **panel_base;          // fused row->column exchange: device table [nranks * nchunks] of the places in the ranks'
                                     // receive arrays where K-ROW writes its output panels directly (null: exchange by pushes)
     bool self_direct;               // two-level K-COL stores this rank's own row pairs straight into its tr[] arrays (no self-copy in the push)
-    bool fused_col;                 // fused column->row exchange: K-COL stores its product rows straight into the owners' receive arrays
-    xfb::cpx *peer_tr[16][4];       // [rank][f]: block of rank's receive array tr[f] that holds THIS rank's column chunks
     xfb::cpx **panel_base_c;        // the same table for the tracer's tendency (array 5 of the receive blocks)
     cudaStream_t comm_stream;
     cudaStream_t copy_stream[4];    // p2p transport: the pushes of one exchange are spread over several copy engines

@@ -19,12 +19,11 @@ template <int NY, int MODE, bool DIST>
 static int launch_row_t(const RowParams &p, cudaStream_t st)
 {
     typedef RowCfg<NY> C;
-    constexpr int smem = (MODE == ROW_JAC) ? C::SMEM_JAC : C::SMEM;
     static PerDeviceInt cfg;
     int err = 0;
-    if (cfg.get([&](int *e) { return resident_ctas(row_kernel<NY, MODE, DIST>, C::THREADS, smem, 0, e); }, &err) <= 0) return err;
+    if (cfg.get([&](int *e) { return resident_ctas(row_kernel<NY, MODE, DIST>, C::THREADS, C::SMEM, 0, e); }, &err) <= 0) return err;
     const int blocks = (p.nrows + C::LPC - 1) / C::LPC;
-    row_kernel<NY, MODE, DIST><<<blocks, C::THREADS, smem, st>>>(p);
+    row_kernel<NY, MODE, DIST><<<blocks, C::THREADS, C::SMEM, st>>>(p);
     return (int)cudaGetLastError();
 }
 
@@ -67,7 +66,6 @@ static int launch_pair_tmem(const RowParams &p, cudaStream_t st)
 }
 
 // ROW_JAC for lines of 16384 points: two-level pair kernel (xfb_rowpair2l.cuh), TMA-staged and persistent.
-// XFB_ROW_2L=0 (or XFB_ROW_SINGLE=1) keeps the first-generation one-row-per-line kernel (A/B knob).
 template <int NY, bool DIST>
 static int launch_pair2l(const RowParams &p, cudaStream_t st)
 {
@@ -86,50 +84,33 @@ static int launch_pair2l(const RowParams &p, cudaStream_t st)
     return (int)cudaGetLastError();
 }
 
-static bool use_two_level_rows()
-{
-    static const bool off = (getenv("XFB_ROW_2L") && atoi(getenv("XFB_ROW_2L")) == 0) ||
-                            (getenv("XFB_ROW_SINGLE") && atoi(getenv("XFB_ROW_SINGLE")) != 0);
-    return !off;
-}
-
 static bool use_tmem_parks(int ny)
 {
     static const int forced = getenv("XFB_ROW_TMEM") ? (atoi(getenv("XFB_ROW_TMEM")) != 0 ? 1 : 0) : -1;
     return forced >= 0 ? forced == 1 : ny >= 4096;
 }
 
-// XFB_ROW_SINGLE=1 forces the one-row-per-line kernel (tuning / A-B knob); 16384 always uses it
-static bool use_pair_kernel(int ny)
-{
-    static const bool forced_single = getenv("XFB_ROW_SINGLE") && atoi(getenv("XFB_ROW_SINGLE")) != 0;
-    return ny <= 8192 && !forced_single;
-}
-
+// lines of up to 8192 points run on the pair kernels; 16384-point lines on the two-level kernel (JAC) and on
+// row_kernel (the plain transforms)
 template <int NY>
 static int launch_row_n(int mode, const RowParams &p, cudaStream_t st)
 {
     const bool dist = p.cw > 0;
     if constexpr (NY <= 8192) {
-        if (use_pair_kernel(NY)) {
-            switch (mode) {
-            case ROW_R2C: return dist ? launch_pair_t<NY, ROW_R2C, true>(p, st) : launch_pair_t<NY, ROW_R2C, false>(p, st);
-            case ROW_C2R: return dist ? launch_pair_t<NY, ROW_C2R, true>(p, st) : launch_pair_t<NY, ROW_C2R, false>(p, st);
-            case ROW_JAC:
-                if (!dist && use_tmem_parks(NY)) return launch_pair_tmem<NY>(p, st);
-                return dist ? launch_pair_t<NY, ROW_JAC, true>(p, st) : launch_pair_t<NY, ROW_JAC, false>(p, st);
-            case ROW_DIAG: return dist ? (int)cudaErrorInvalidValue : launch_pair_t<NY, ROW_DIAG, false>(p, st);
-            }
-            return (int)cudaErrorInvalidValue;
+        switch (mode) {
+        case ROW_R2C: return dist ? launch_pair_t<NY, ROW_R2C, true>(p, st) : launch_pair_t<NY, ROW_R2C, false>(p, st);
+        case ROW_C2R: return dist ? launch_pair_t<NY, ROW_C2R, true>(p, st) : launch_pair_t<NY, ROW_C2R, false>(p, st);
+        case ROW_JAC:
+            if (!dist && use_tmem_parks(NY)) return launch_pair_tmem<NY>(p, st);
+            return dist ? launch_pair_t<NY, ROW_JAC, true>(p, st) : launch_pair_t<NY, ROW_JAC, false>(p, st);
+        case ROW_DIAG: return dist ? (int)cudaErrorInvalidValue : launch_pair_t<NY, ROW_DIAG, false>(p, st);
         }
-    }
-    if constexpr (NY == 16384) {
-        if (mode == ROW_JAC && use_two_level_rows()) return dist ? launch_pair2l<NY, true>(p, st) : launch_pair2l<NY, false>(p, st);
-    }
-    switch (mode) {
-    case ROW_R2C: return dist ? launch_row_t<NY, ROW_R2C, true>(p, st) : launch_row_t<NY, ROW_R2C, false>(p, st);
-    case ROW_C2R: return dist ? launch_row_t<NY, ROW_C2R, true>(p, st) : launch_row_t<NY, ROW_C2R, false>(p, st);
-    case ROW_JAC: return dist ? launch_row_t<NY, ROW_JAC, true>(p, st) : launch_row_t<NY, ROW_JAC, false>(p, st);
+    } else {
+        switch (mode) {
+        case ROW_R2C: return dist ? launch_row_t<NY, ROW_R2C, true>(p, st) : launch_row_t<NY, ROW_R2C, false>(p, st);
+        case ROW_C2R: return dist ? launch_row_t<NY, ROW_C2R, true>(p, st) : launch_row_t<NY, ROW_C2R, false>(p, st);
+        case ROW_JAC: return dist ? launch_pair2l<NY, true>(p, st) : launch_pair2l<NY, false>(p, st);
+        }
     }
     return (int)cudaErrorInvalidValue;
 }

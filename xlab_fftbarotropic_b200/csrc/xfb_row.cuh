@@ -1,11 +1,10 @@
-// xfb_row.cuh -- K-ROW: transforms along y (the contiguous direction), one line per group of
-// NY/32 threads.  Replaces, for one row i of the grid:
+// xfb_row.cuh -- K-ROW: the line transforms along y (the contiguous direction) shared by every K-ROW kernel,
+// and row_kernel, one line per group of NY/32 threads, which replaces for one row i of the grid:
 //   R2C : the last-dimension half of fftwf_plan_dft_r2c_2d   (/root/reference/src/main.cpp:126-127,237,256)
 //   C2R : the last-dimension half of fftwf_plan_dft_c2r_2d + fftwf_backward_normalize
 //         (main.cpp:129-135,37-41)
-//   JAC : four C2R (dvortdx, dvortdy, u, v: main.cpp:154,168,200,214), `u = -u` (:201), the
-//         Jacobian + source loop (:225-227) and the R2C of the tendency (:237), chained in
-//         registers -- the physical-space fields never touch HBM.
+// row_kernel serves 16384-point lines only (operator tier, record path, slab handles); shorter lines run on the pair
+// kernels (xfb_rowpair.cuh), and the stepper's JAC at 16384 on the two-level kernel (xfb_rowpair2l.cuh).
 // A real line of NY points is transformed as a complex line of L = NY/2 points plus the
 // standard split/merge step of a half-length real transform.
 //
@@ -53,17 +52,11 @@ template <int NY>
 struct RowCfg {
     static constexpr int L = NY / 2;
     static constexpr int G = L / 16;                         // threads per line
-    // both lines of a row pair in one CTA wherever the shared memory allows it (NY <= 8192)
-#ifdef XFB_ROW_LPC1
-    static constexpr int THREADS = (G >= 128) ? G : 128;
-#else
+    // both lines of a row pair in one CTA wherever the shared memory allows it (NY <= 8192); row_kernel is instantiated
+    // at NY = 16384 only, where THREADS = G = 512 and LPC = 1
     static constexpr int THREADS = (G >= 512) ? G : (2 * G >= 128) ? 2 * G : 128;
-#endif
     static constexpr int LPC = THREADS / G;                  // lines per CTA
     static constexpr int SMEM = LPC * LinePlan<L>::PADDED * (int)sizeof(cpx);
-    // JAC parks -u (then -u * dvortdx) and v in shared memory between the four inverse transforms, so
-    // no physical-space field is live in registers across a transform
-    static constexpr int SMEM_JAC = SMEM + 2 * LPC * L * (int)sizeof(cpx);
     static constexpr int MINB = (THREADS >= 512) ? 1 : (THREADS >= 256) ? 2 : 4;
 };
 
@@ -181,6 +174,7 @@ template <int NY, int MODE, bool DIST>
 __global__ void __launch_bounds__(RowCfg<NY>::THREADS, RowCfg<NY>::MINB)
 row_kernel(const RowParams p)
 {
+    static_assert(MODE == ROW_R2C || MODE == ROW_C2R, "row_kernel has the plain transforms only");
     typedef RowCfg<NY> C;
     constexpr int L = C::L, G = C::G;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -205,62 +199,12 @@ row_kernel(const RowParams p)
         for (int q = 0; q < 16; ++q) v[q] = __ldg(x + t + q * G);
         cpx *out = p.spec_out + line_base(row, DIST ? p.cw : p.pitch);
         r2c_line<NY, DIST>(v, out, p, live ? p.pitch : 0, sm, t, wt, tw, bar);   // a clamped duplicate row rewrites identical values
-    } else if (MODE == ROW_C2R) {
+    } else {
         c2r_line<NY, DIST>(v, p.spec_in[0] + line_base(row, DIST ? p.cw : p.pitch), p, sm, t, wt, tw, bar);
         float2 *x = reinterpret_cast<float2 *>(p.real_out + (size_t)row * NY);
         const float s = p.negate ? -p.scale : p.scale;
 #pragma unroll
         for (int q = 0; q < 16; ++q) x[t + q * G] = mk(v[q].y * s, v[q].x * s);
-    } else {
-        const size_t off = line_base(row, DIST ? p.cw : p.pitch);
-        cpx *park0 = reinterpret_cast<cpx *>(smem_raw) + (size_t)C::LPC * LinePlan<L>::PADDED + (size_t)lane_line * (2 * L);
-        // pull the lines that are not needed first into L2 while the first transform runs: the two lines of
-        // a row pair share one contiguous region of 2 * pitch elements, each line's threads fetch half of it
-        if (!DIST) {
-            const int region_bytes = 2 * p.pitch * (int)sizeof(cpx);
-            const size_t pair_off = (size_t)(row >> 1) * (size_t)(2 * p.pitch);
-            for (int o = (t + (row & 1) * G) * 128; o < region_bytes; o += 2 * G * 128) {
-                prefetch_l2(reinterpret_cast<const char *>(p.spec_in[0] + pair_off) + o);
-                prefetch_l2(reinterpret_cast<const char *>(p.spec_in[3] + pair_off) + o);
-                prefetch_l2(reinterpret_cast<const char *>(p.spec_in[1] + pair_off) + o);
-            }
-        }
-        // One code path for the four inverse transforms (keeps the kernel inside the instruction cache):
-        //   f = 0: a = c2r(T_u)/GRIDS = -u      -> park0 = a              (main.cpp:200-201)
-        //   f = 1: dvortdx                      -> park0 = a * dvortdx    (main.cpp:154,226)
-        //   f = 2: v                            -> park1 = v              (main.cpp:214)
-        //   f = 3: dvortdy                      -> park1 = v * dvortdy    (main.cpp:168,226)
-#pragma unroll 1
-        for (int f = 0; f < 4; ++f) {
-            const int src_field = (f == 0) ? 2 : (f == 1) ? 0 : (f == 2) ? 3 : 1;
-            c2r_line<NY, DIST>(v, p.spec_in[src_field] + off, p, sm, t, wt, tw, bar);
-            cpx *park = park0 + (f >> 1) * L;
-            if (f & 1) {
-#pragma unroll
-                for (int q = 0; q < 16; ++q) {
-                    const cpx a = park[q * G + t];
-                    park[q * G + t] = mk(a.x * (v[q].y * p.scale), a.y * (v[q].x * p.scale));
-                }
-            } else {
-#pragma unroll
-                for (int q = 0; q < 16; ++q) park[q * G + t] = mk(v[q].y * p.scale, v[q].x * p.scale);
-            }
-        }
-        cpx J[16];
-#pragma unroll
-        for (int q = 0; q < 16; ++q) {
-            const cpx j1 = park0[q * G + t], j2 = park0[L + q * G + t];
-            J[q] = mk(j1.x - j2.x, j1.y - j2.y);
-        }
-        if (p.real_in != nullptr) {
-            const float2 *s = reinterpret_cast<const float2 *>(p.real_in + (size_t)row * NY);
-#pragma unroll
-            for (int q = 0; q < 16; ++q) {
-                const float2 sv = __ldg(s + t + q * G);
-                J[q] = mk(J[q].x + sv.x, J[q].y + sv.y);
-            }
-        }
-        r2c_line<NY, DIST>(J, p.spec_out + off, p, live ? p.pitch : 0, sm, t, wt, tw, bar);
     }
 }
 

@@ -4,8 +4,8 @@
 //
 // Same reference loops as xfb_rowpair.cuh: main.cpp:126-135,154,168,200-201,214,225-227,237 and
 // fftwf_backward_normalize (:37-41).  Why a kernel of its own: a 16384-point line does not fit 512 threads x 16 values;
-// the first-generation row_kernel<16384> addresses the pair layout with 8-byte loads at stride 16 and touches every
-// spectral element twice (k and its mirror): 572 M global sectors for 134 M sectors of payload, stall_lg 2.4, 42 % of the
+// the first-generation JAC kernel (since removed) addressed the pair layout with 8-byte loads at stride 16 and touched
+// every spectral element twice (k and its mirror): 572 M global sectors for 134 M sectors of payload, stall_lg 2.4, 42 % of the
 // issue slots used (profiles/r02_16384_gen1_ncu_full_summary.txt).  Here, like the 8192 kernel:
 //   * persistent CTAs; the pair's contiguous region of a field (2 * pitch complex values, 131 KB) is fetched by
 //     cp.async.bulk into ONE staging buffer in two halves with an mbarrier each, a field ahead of its use;
