@@ -114,6 +114,12 @@ int xfb_get_diagnostics(xfb_handle h, int member, float *tfil, float *deform);
  * handles: every rank bins its rows, ONE ncclAllReduce sums the 2 * nbins values, every rank receives the whole-domain
  * histograms; collective. */
 int xfb_get_keff_hist(xfb_handle h, int member, int nbins, float cmin, float cmax, double *area, double *grad2);
+/* quadratic invariants of the current state and their isotropic shell spectra (no reference counterpart;
+ * definitions in DESIGN.md).  which = XFB_VORT (vorticity) or XFB_TRACER (the passive tracer, same forms).
+ * totals[3] = {E, Z, P}: domain means, float64.  nshells == 0: totals only (e, z may be NULL); else e[nshells],
+ * z[nshells] = shell sums of E and Z.  Host pointers only.  Reads the state only: later steps are unaffected.
+ * Slab-decomposed handles: collective, every rank receives the whole-domain result. */
+int xfb_get_energy_spectrum(xfb_handle h, int member, int which, int nshells, double *totals, double *e, double *z);
 
 /* ---- passive tracer (SURVEY.md section 8 (f-4); the reference has none) -------------------------
  * dc/dt = -u c_x - v c_y + kappa lap(c), advanced by xfb_step together with the vorticity: every Runge-Kutta stage
@@ -166,6 +172,7 @@ int xfb_loopback_step(xfb_loopback t, int nsteps, float dt);
 int xfb_loopback_get_field(xfb_loopback t, int which, float *out);
 int xfb_loopback_get_diagnostics(xfb_loopback t, float *tfil, float *deform);
 int xfb_loopback_get_keff_hist(xfb_loopback t, int nbins, float cmin, float cmax, double *area, double *grad2);
+int xfb_loopback_get_energy_spectrum(xfb_loopback t, int which, int nshells, double *totals, double *e, double *z);
 long long xfb_loopback_launch_count(xfb_loopback t);
 
 /* ---- introspection --------------------------------------------------------------------------*/

@@ -1,6 +1,6 @@
 """In-tree build of the CUDA library (sm_100a only) and of the host C++ programs.
 
-  libxfb.so        csrc/xfb_row.cu + xfb_col.cu + xfb_api.cu + xfb_dist.cu + xfb_generic.cu  (the C ABI of include/xfb.h)
+  libxfb.so        csrc/xfb_row.cu + xfb_col.cu + xfb_api.cu + xfb_dist.cu + xfb_generic.cu + xfb_spectra.cu  (the C ABI of include/xfb.h)
 
 nvcc cross-compiles without a GPU; the .so is git-ignored but travels with gpurun snapshots.
 """
@@ -20,7 +20,7 @@ LIB = os.path.join(HERE, "libxfb.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
-CUDA_SOURCES = ["xfb_row.cu", "xfb_col.cu", "xfb_api.cu", "xfb_dist.cu", "xfb_generic.cu"]
+CUDA_SOURCES = ["xfb_row.cu", "xfb_col.cu", "xfb_api.cu", "xfb_dist.cu", "xfb_generic.cu", "xfb_spectra.cu"]
 HEADERS = ["xfb_fft.cuh", "xfb_row.cuh", "xfb_rowpair.cuh", "xfb_rowpair2l.cuh", "xfb_col.cuh", "xfb_colt.cuh", "xfb_col2l.cuh", "xfb_internal.h", "xfb_handle.h", os.path.join(ROOT, "include", "xfb.h")]
 
 

@@ -6,6 +6,7 @@ device is present xfb_create fails with XFB_E_CUDA.
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -27,6 +28,7 @@ SYMBOLS = [
     "xfb_loopback_create", "xfb_loopback_destroy", "xfb_loopback_set_vorticity", "xfb_loopback_set_source",
     "xfb_loopback_step", "xfb_loopback_get_field", "xfb_loopback_launch_count", "xfb_loopback_get_diagnostics",
     "xfb_loopback_get_keff_hist", "xfb_loopback_set_tracer",
+    "xfb_get_energy_spectrum", "xfb_loopback_get_energy_spectrum",
 ]
 
 _lib = None
@@ -65,6 +67,8 @@ def load():
     L.xfb_wait_field.argtypes = [vp, ci]
     L.xfb_get_keff_hist.argtypes = [vp, ci, ci, cf, cf, vp, vp]
     L.xfb_get_tracer_keff_hist.argtypes = [vp, ci, ci, cf, cf, vp, vp]
+    L.xfb_get_energy_spectrum.argtypes = [vp, ci, ci, ci, vp, vp, vp]
+    L.xfb_loopback_get_energy_spectrum.argtypes = [vp, ci, ci, vp, vp, vp]
     L.xfb_set_tracer.argtypes = [vp, ci, vp, cf]
     L.xfb_invert_pres.argtypes = [vp, vp, vp, C.c_size_t, C.c_size_t, cf, cf]
     L.xfb_launch_count.restype = C.c_longlong
@@ -105,6 +109,32 @@ def slab_partition(nx, ny, nranks, nchunks, rank):
     if rc != 0:
         raise XfbError(f"xfb error {rc}: {L.xfb_last_error().decode()}")
     return dict(zip(("row0", "rows", "col0", "cols", "chunk_cols", "pitch_global"), (x.value for x in v)))
+
+
+def shells_all(nx, ny, lx, ly=None) -> int:
+    """Number of isotropic shells that holds every mode of an nx x ny grid: the shell of (nx/2, ny/2) plus one
+    (DESIGN.md section 3; pure host arithmetic)."""
+    ly = lx if ly is None else ly
+    lx, ly = float(np.float32(lx)), float(np.float32(ly))
+    ip, j = nx // 2, ny // 2
+    if lx == ly:
+        m = ip * ip + j * j
+        s = math.isqrt(m)
+        return s + (1 if m > s * s + s else 0) + 1
+    big = max(lx, ly)
+    a, b = ip * (big / lx), j * (big / ly)
+    return int(math.floor(math.sqrt(a * a + b * b) + 0.5)) + 1
+
+
+def _energy_spectrum(L, call, nshells, nx, ny, lx, ly):
+    n = shells_all(nx, ny, lx, ly) if nshells is None else int(nshells)
+    totals = np.zeros(3, np.float64)
+    e = np.zeros(n, np.float64)
+    z = np.zeros(n, np.float64)
+    rc = call(_ptr(totals), _ptr(e) if n else None, _ptr(z) if n else None, n)
+    if rc != 0:
+        raise XfbError(f"xfb error {rc}: {L.xfb_last_error().decode()}")
+    return totals, e, z
 
 
 def nccl_unique_id() -> bytes:
@@ -242,6 +272,12 @@ class Backend:
         self._ck(self._L.xfb_get_keff_hist(self._h, member, nbins, cmin, cmax, _ptr(area), _ptr(g2)))
         return area, g2
 
+    def energy_spectrum(self, nshells=None, which=VORT, member=0):
+        """-> (totals [E, Z, P], e[nshells], z[nshells]): domain-mean kinetic energy, enstrophy, palinstrophy and the
+        shell sums of E and Z (float64); nshells=None: every shell (shells_all).  which = VORT or TRACER."""
+        return _energy_spectrum(self._L, lambda t, e, z, n: self._L.xfb_get_energy_spectrum(self._h, member, which, n, t, e, z),
+                                nshells, self.nx, self.ny, self.lx, self.ly)
+
     # passive tracer: advected by xfb_step with the flow of each stage; read back with get_field(TRACER)
     def set_tracer(self, c, kappa, member=0):
         c = np.ascontiguousarray(c, dtype=np.float32).reshape(self.nx, self.ny)
@@ -337,7 +373,7 @@ class LoopbackTeam:
     on a single GPU; same kernels as the NCCL path, the exchange is a set of device copies)."""
 
     def __init__(self, n: int, nranks: int, nchunks: int = 1, lx: float = 600000.0, nu: float = 6.5, device: int = 0):
-        self.n = n
+        self.n, self.lx = n, lx
         self._L = load()
         self._t = C.c_void_p()
         self._ck(self._L.xfb_loopback_create(C.byref(self._t), n, n, lx, lx, nu, device, nranks, nchunks))
@@ -391,6 +427,11 @@ class LoopbackTeam:
         g2 = np.zeros(nbins, np.float64)
         self._ck(self._L.xfb_loopback_get_keff_hist(self._t, nbins, cmin, cmax, _ptr(area), _ptr(g2)))
         return area, g2
+
+    def energy_spectrum(self, nshells=None, which=VORT):
+        """whole-domain (totals, e, z) as Backend.energy_spectrum"""
+        return _energy_spectrum(self._L, lambda t, e, z, n: self._L.xfb_loopback_get_energy_spectrum(self._t, which, n, t, e, z),
+                                nshells, self.n, self.n, self.lx, self.lx)
 
     @property
     def launch_count(self):

@@ -14,7 +14,11 @@
 //      file -- and writes <field>_step_N.bin for m = 0, <field>_step_N.m<m>.bin otherwise),
 //   -G <gpus> (the members are spread over that many devices starting at -g, no communication),
 //   -S <ranks> (ONE grid slab-decomposed over that many GPUs: the process forks one rank per device, the ranks exchange
-//      over NVLink (xfb_create_dist), each reads and writes its own rows of the field files; same files and log).
+//      over NVLink (xfb_create_dist), each reads and writes its own rows of the field files; same files and log),
+//   -E (at every record step, per member: the domain means E, Z, P appended to <output>/integrals.txt as
+//      `step time member E Z P`, and the isotropic shell spectra written to <output>/spectrum_step_N.txt -- .m<m>.txt for
+//      members other than 0 -- one `s k[1/m] E(s) Z(s)` line per shell; neither goes into `log`.  A non-finite total
+//      stops the run with exit status 1 once the record files already issued are written).
 // Record output is asynchronous (SURVEY.md 8f-2): at a record step the five fields are formed on the GPU and copied
 // to pinned host buffers on a second stream (xfb_get_field_async) while the next stretch of steps already runs; a
 // writer thread waits for each buffer, calls writeField and appends the `log` line -- same files, same order as the
@@ -50,11 +54,41 @@ using namespace VORT_SRC_READER;
         }                                                                  \
     } while (0)
 
+// -E: number of shells that holds every mode of an n x n grid (the shell of (n/2, n/2) plus one, integer rule)
+static int all_shells(int n)
+{
+    const long long m = 2LL * (n / 2) * (n / 2);
+    long long s = (long long)std::sqrt((double)m);
+    while (s * s > m) --s;
+    while ((s + 1) * (s + 1) <= m) ++s;
+    return (int)(s + (m > s * s + s ? 1 : 0) + 1);
+}
+
+// -E at one record step for one member: spectrum file, integrals line; returns 1 if a total is not finite
+static int write_energy(const std::string &output, FILE *integrals, int step, float dt, int member, float L, const double *tot,
+                        const std::vector<double> &e, const std::vector<double> &z)
+{
+    char name[1024];
+    if (member == 0) std::snprintf(name, sizeof(name), "%s/spectrum_step_%d.txt", output.c_str(), step);
+    else std::snprintf(name, sizeof(name), "%s/spectrum_step_%d.m%d.txt", output.c_str(), step, member);
+    if (FILE *f = std::fopen(name, "w")) {
+        std::fprintf(f, "# s  k[1/m]  E(s)  Z(s)   (step %d, member %d; shell sums of E = <u^2+v^2>/2 and Z = <zeta^2>/2)\n", step, member);
+        const double dk = 2.0 * M_PI / (double)L;
+        for (size_t k = 0; k < e.size(); ++k) std::fprintf(f, "%zu %.9g %.17g %.17g\n", k, dk * (double)k, e[k], z[k]);
+        std::fclose(f);
+    }
+    if (integrals) {
+        std::fprintf(integrals, "%d %.17g %d %.17g %.17g %.17g\n", step, (double)step * dt, member, tot[0], tot[1], tot[2]);
+        std::fflush(integrals);
+    }
+    return (std::isfinite(tot[0]) && std::isfinite(tot[1]) && std::isfinite(tot[2])) ? 0 : 1;
+}
+
 struct SlabOpts {
     std::string input, output, init_file;
     int npts, record_step, total_steps, device, ranks;
     float L, NU, dt;
-    bool diagnostics, quiet;
+    bool diagnostics, quiet, energy;
 };
 
 // one rank of `-S <ranks>`: local rows [row0, row0 + rows) of every file
@@ -80,6 +114,13 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
         close(fd);
     }
     FILE *log_fd = rank == 0 ? std::fopen("log", "w") : nullptr;
+    FILE *integrals = nullptr;
+    if (o.energy && rank == 0) {
+        std::snprintf(filename, sizeof(filename), "%s/integrals.txt", o.output.c_str());
+        integrals = std::fopen(filename, "w");
+    }
+    const int nsh = o.energy ? all_shells(n) : 0;
+    std::vector<double> es(nsh), zs(nsh);
     CHECK(xfb_set_vorticity(h, 0, buf.data()));
     if (rank == 0) std::printf("Initialization complete.\n");
     auto record = [&](const char *stem, int which, int step) -> int {
@@ -104,6 +145,20 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
                 std::fprintf(stderr, "main.out: %s\n", xfb_last_error());
                 return 1;
             }
+            if (o.energy) {
+                double tot[3];
+                CHECK(xfb_get_energy_spectrum(h, 0, XFB_VORT, nsh, tot, es.data(), zs.data()));      // collective
+                const bool bad = !(std::isfinite(tot[0]) && std::isfinite(tot[1]) && std::isfinite(tot[2]));
+                if (rank == 0) write_energy(o.output, integrals, step, o.dt, 0, o.L, tot, es, zs);
+                if (bad) {
+                    if (rank == 0) std::fprintf(stderr, "main.out: non-finite energy/enstrophy at step %d (member 0)\n", step);
+                    if (integrals) std::fclose(integrals);
+                    if (log_fd) std::fclose(log_fd);
+                    xfb_sync(h);
+                    xfb_destroy(h);
+                    return 1;
+                }
+            }
         }
         const int next_record = (step / o.record_step + 1) * o.record_step;
         const int chunk = (next_record < o.total_steps ? next_record : o.total_steps) - step;
@@ -114,6 +169,7 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
     }
     CHECK(xfb_sync(h));
     if (log_fd) std::fclose(log_fd);
+    if (integrals) std::fclose(integrals);
     xfb_destroy(h);
     if (rank == 0) std::printf("Program ends. Congrats!\n");
     return 0;
@@ -164,10 +220,10 @@ int main(int argc, char *args[])
     RECIPE_TYPE recipe_type = EMPTY;
     int npts = 768, record_step = 100, total_steps = -1, device = 0, members = 1, ngpus = 1, slab_ranks = 0;
     float L = 600000.0f, NU = 6.5f, dt = 3.0f;
-    bool diagnostics = false, quiet = false;
+    bool diagnostics = false, quiet = false, energy = false;
 
     int opt;
-    while ((opt = getopt(argc, args, "I:O:o:i:s:f:n:d:t:r:L:N:g:c:k:b:G:S:Dq")) != EOF) {
+    while ((opt = getopt(argc, args, "I:O:o:i:s:f:n:d:t:r:L:N:g:c:k:b:G:S:DEq")) != EOF) {
         switch (opt) {
         case 'I': input = optarg; break;
         case 'O': case 'o': output = optarg; break;
@@ -187,6 +243,7 @@ int main(int argc, char *args[])
         case 'G': ngpus = std::atoi(optarg); break;
         case 'S': slab_ranks = std::atoi(optarg); break;
         case 'D': diagnostics = true; break;
+        case 'E': energy = true; break;
         case 'q': quiet = true; break;
         }
     }
@@ -215,12 +272,21 @@ int main(int argc, char *args[])
             std::fprintf(stderr, "main.out: -S (slab decomposition) runs one member without forcing or tracer\n");
             return 1;
         }
-        SlabOpts so{input, output, init_file, npts, record_step, total_steps, device, slab_ranks, L, NU, dt, diagnostics, quiet};
+        SlabOpts so{input, output, init_file, npts, record_step, total_steps, device, slab_ranks, L, NU, dt, diagnostics, quiet,
+                    energy};
         return run_slab(so);
     }
 
     FILE *log_fd = std::fopen("log", "w");                        // main.cpp:97, in the CWD
     if (log_fd == NULL) perror("Open log file");
+    FILE *integrals = nullptr;                                      // -E
+    if (energy) {
+        const std::string name = output + "/integrals.txt";
+        integrals = std::fopen(name.c_str(), "w");
+        if (!integrals) perror("Open integrals.txt");
+    }
+    const int nsh = energy ? all_shells(npts) : 0;
+    std::vector<double> es(nsh), zs(nsh);
 
     // ensemble members in blocks over the devices: handle d holds members [first[d], first[d] + count[d])
     std::vector<xfb_handle> hs(ngpus, nullptr);
@@ -358,6 +424,24 @@ int main(int argc, char *args[])
                 shutdown_writer();
                 return 1;
             }
+            for (int m = 0; energy && m < members; ++m) {
+                int lm = 0;
+                xfb_handle hm = owner(m, &lm);
+                double tot[3];
+                if (xfb_get_energy_spectrum(hm, lm, XFB_VORT, nsh, tot, es.data(), zs.data()) != 0) {
+                    std::fprintf(stderr, "main.out: %s\n", xfb_last_error());
+                    shutdown_writer();
+                    return 1;
+                }
+                if (write_energy(output, integrals, step, dt, m, L, tot, es, zs)) {
+                    std::fprintf(stderr, "main.out: non-finite energy/enstrophy at step %d (member %d)\n", step, m);
+                    wait_writer();                 // the record files already issued reach the disk
+                    shutdown_writer();
+                    if (integrals) std::fclose(integrals);
+                    if (log_fd) std::fclose(log_fd);
+                    return 1;
+                }
+            }
         }
         int chunk = 1;
         if (recipe_type == EMPTY) {
@@ -404,6 +488,7 @@ int main(int argc, char *args[])
     for (float *pb : pinned) xfb_host_free(pb);
     xfb_host_free(src);
     if (log_fd) std::fclose(log_fd);
+    if (integrals) std::fclose(integrals);
     for (xfb_handle hd : hs) xfb_destroy(hd);
     (void)h;
     std::printf("Program ends. Congrats!\n");

@@ -332,7 +332,7 @@ int xfb::destroy_impl(xfb_handle h)
         cudaStreamDestroy(h->rec_stream);
     }
     void *ptrs[] = {h->tw, h->kx, h->ky, h->kx2, h->ky2, h->z0, h->zk, h->acc, h->jint, h->t_block, h->src, h->dg, h->real_a,
-                    h->real_b, h->real_c, h->spec_a, h->spec_b, h->ref_a, h->ref_b, h->recv_block, h->sync_buf, h->c0, h->ck, h->cacc, h->cjint, h->tc[0], h->panel_base, h->panel_base_c};
+                    h->real_b, h->real_c, h->spec_a, h->spec_b, h->ref_a, h->ref_b, h->recv_block, h->sync_buf, h->espec, h->c0, h->ck, h->cacc, h->cjint, h->tc[0], h->panel_base, h->panel_base_c};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (auto pool : {h->ev_row, h->ev_col, h->ev_a2a})
@@ -1136,6 +1136,32 @@ extern "C" int xfb_get_tracer_keff_hist(xfb_handle h, int member, int nbins, flo
         return dist_tracer_keff_hist(h, nbins, cmin, cmax, area, grad2);
     }
     return keff_hist_impl(h, member, nbins, cmin, cmax, area, grad2, h->c0);
+}
+
+// Quadratic invariants E, Z, P of the state (vorticity or tracer) and their isotropic shell spectra, reduced on the device
+// from the tile-major (or generic row-major) state in one launch (xfb_spectra.cu); definitions in DESIGN.md section 3.
+static int energy_spectrum_args(xfb_handle h, int member, int which, int nshells, double *totals, double *e, double *z)
+{
+    if (check_member(h, member)) return XFB_E_ARG;
+    if (which != XFB_VORT && which != XFB_TRACER) return fail(XFB_E_ARG, "xfb_get_energy_spectrum: which must be XFB_VORT or XFB_TRACER");
+    if (nshells < 0 || nshells > XFB_SPECTRUM_MAX_SHELLS)
+        return fail(XFB_E_ARG, "xfb_get_energy_spectrum: nshells %d not in 0..%d", nshells, XFB_SPECTRUM_MAX_SHELLS);
+    if (!totals || (nshells > 0 && (!e || !z))) return fail(XFB_E_ARG, "xfb_get_energy_spectrum: null output");
+    if (!h->have_state) return fail(XFB_E_STATE, "xfb_get_energy_spectrum before xfb_set_vorticity");
+    if (which == XFB_TRACER && !h->has_tracer) return fail(XFB_E_STATE, "xfb_get_energy_spectrum: XFB_TRACER before xfb_set_tracer");
+    return 0;
+}
+
+extern "C" int xfb_get_energy_spectrum(xfb_handle h, int member, int which, int nshells, double *totals, double *e, double *z)
+{
+    if (int r = energy_spectrum_args(h, member, which, nshells, totals, e, z)) return r;
+    CK(cudaSetDevice(h->device));
+    if (h->nranks > 1) return dist_energy_spectrum(h, which, nshells, totals, e, z);     // collective
+    if (energy_spectrum_scratch(h)) return XFB_E_CUDA;
+    const cpx *state = (which == XFB_TRACER ? h->c0 : h->z0) + (size_t)member * h->hpad;
+    CK(cudaMemsetAsync(h->espec, 0, sizeof(double) * (3 + 2 * (size_t)nshells), h->stream));
+    if (launch_energy_spectrum(h, state, nshells, h->espec)) return XFB_E_CUDA;
+    return energy_spectrum_finish(h, h->espec, nshells, totals, e, z);
 }
 
 // ------------------------------------------------------------------------------------------------

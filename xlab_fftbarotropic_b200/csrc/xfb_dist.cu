@@ -711,6 +711,19 @@ int dist_get_field(xfb_handle h, int which, float *out_rows)
     return 0;
 }
 
+// quadratic invariants and shell spectra: every rank reduces its own column chunks, one all-reduce of the 3 + 2 * nshells
+// sums (nothing is written that a peer reads: no exchange, no fence); collective
+int dist_energy_spectrum(xfb_handle h, int which, int nshells, double *totals, double *e, double *z)
+{
+    if (h->team->loopback) return fail(XFB_E_STATE, "loopback ranks are driven through xfb_loopback_*");
+    if (energy_spectrum_scratch(h)) return XFB_E_CUDA;
+    const size_t n = 3 + 2 * (size_t)nshells;
+    CK(cudaMemsetAsync(h->espec, 0, sizeof(double) * n, h->stream));
+    if (int r = launch_energy_spectrum(h, which == XFB_TRACER ? h->c0 : h->z0, nshells, h->espec)) return r;
+    NCK(g_nccl.AllReduce(h->espec, h->espec, n, ncclDouble, ncclSum, h->team->comm, h->stream));
+    return energy_spectrum_finish(h, h->espec, nshells, totals, e, z);
+}
+
 void dist_release(xfb_handle h)
 {
     Team *T = h->team;
@@ -1046,6 +1059,27 @@ extern "C" int xfb_loopback_get_keff_hist(xfb_loopback_s *L, int nbins, float cm
     memcpy(area, host.data(), sizeof(double) * nbins);
     memcpy(grad2, host.data() + nbins, sizeof(double) * nbins);
     return 0;
+}
+
+extern "C" int xfb_loopback_get_energy_spectrum(xfb_loopback_s *L, int which, int nshells, double *totals, double *e, double *z)
+{
+    if (!L) return fail(XFB_E_ARG, "null argument");
+    xfb_handle h0 = L->team.local[0];
+    if (which != XFB_VORT && which != XFB_TRACER) return fail(XFB_E_ARG, "xfb_loopback_get_energy_spectrum: which must be XFB_VORT or XFB_TRACER");
+    if (nshells < 0 || nshells > XFB_SPECTRUM_MAX_SHELLS)
+        return fail(XFB_E_ARG, "xfb_loopback_get_energy_spectrum: nshells %d not in 0..%d", nshells, XFB_SPECTRUM_MAX_SHELLS);
+    if (!totals || (nshells > 0 && (!e || !z))) return fail(XFB_E_ARG, "xfb_loopback_get_energy_spectrum: null output");
+    if (!h0->have_state) return fail(XFB_E_STATE, "xfb_loopback_get_energy_spectrum before xfb_loopback_set_vorticity");
+    if (which == XFB_TRACER && !h0->has_tracer) return fail(XFB_E_STATE, "xfb_loopback_get_energy_spectrum: XFB_TRACER before xfb_loopback_set_tracer");
+    CK(cudaSetDevice(h0->device));
+    // all ranks share the device and the stream: their launches add into rank 0's sums (the all-reduce of the NCCL path)
+    if (energy_spectrum_scratch(h0)) return XFB_E_CUDA;
+    CK(cudaMemsetAsync(h0->espec, 0, sizeof(double) * (3 + 2 * (size_t)nshells), h0->stream));
+    for (int r = 0; r < L->team.nranks; ++r) {
+        xfb_handle h = L->team.local[r];
+        if (int e2 = launch_energy_spectrum(h, which == XFB_TRACER ? h->c0 : h->z0, nshells, h0->espec)) return e2;
+    }
+    return energy_spectrum_finish(h0, h0->espec, nshells, totals, e, z);
 }
 
 extern "C" long long xfb_loopback_launch_count(xfb_loopback_s *L)

@@ -31,6 +31,7 @@ struct Team;
 }  // namespace xfb
 
 #define XFB_NREC 8          // record fields in flight (xfb_get_field_async)
+#define XFB_SPECTRUM_MAX_SHELLS 65536   // nshells limit of xfb_get_energy_spectrum
 
 struct xfb_handle_s {
     int nx, ny, hy, pitch, batch, device;
@@ -61,6 +62,7 @@ struct xfb_handle_s {
     cudaEvent_t rec_ready[XFB_NREC], rec_done[XFB_NREC];
     int rec_next;
     xfb::cpx *dg;        // 3 exchange arrays of the fused diagnostics path, allocated on first use
+    double *espec;       // xfb_get_energy_spectrum sums: 3 + 2 * XFB_SPECTRUM_MAX_SHELLS doubles, allocated on first use
     bool warmed;         // one eager step has run (kernels configured)
     void *step_graph;    // cudaGraphExec_t of one RK4 step (8 launches), valid for graph_dt / graph_src
     float graph_dt;
@@ -132,6 +134,13 @@ int generic_step(xfb_handle h, int nsteps, float dt);
 int launch_keff_hist(xfb_handle h, const float *c, const float *gx, const float *gy, long long n, int nbins, float cmin, float cmax,
                      double *d_area, double *d_grad2);
 
+// quadratic invariants and shell spectra (xfb_spectra.cu): one launch adds the raw sums of one state array into
+// d_out[3 + 2 * nshells] (device, zeroed by the caller); _finish copies them to the host and scales them to domain means
+long long shells_all(int nx, int ny, float lx, float ly);
+int energy_spectrum_scratch(xfb_handle h);
+int launch_energy_spectrum(xfb_handle h, const cpx *state, int nshells, double *d_out);
+int energy_spectrum_finish(xfb_handle h, const double *d, int nshells, double *totals, double *e, double *z);
+
 // slab paths (xfb_dist.cu)
 int dist_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2);
 int dist_diagnostics(xfb_handle h, float *tfil_rows, float *deform_rows);
@@ -140,6 +149,7 @@ int dist_set_tracer(xfb_handle h, const float *tracer_rows);
 int dist_tracer_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2);
 int dist_step(xfb_handle h, int nsteps, float dt);
 int dist_get_field(xfb_handle h, int which, float *out_rows);
+int dist_energy_spectrum(xfb_handle h, int which, int nshells, double *totals, double *e, double *z);
 void dist_release(xfb_handle h);
 
 }  // namespace xfb
