@@ -83,24 +83,16 @@ __device__ __forceinline__ size_t pair_base(const int t, const int j, const int 
 // -(kx^2 + ky^2) narrowed to float, summed in float64 like pow(float,2)+pow(float,2) (fftwfop.cpp:42-45)
 __device__ __forceinline__ float lap_coe(const double kx2, const double ky2) { return (float)(-(kx2 + ky2)); }
 
-// signed x wavenumber index of row i = t + k*G (k compile-time): i for i <= NX/2 (Nyquist keeps +), else i - NX
-template <int NX>
+// signed x wavenumber index of row i = slot_pos(t, k) (k compile-time): i for i <= NX/2 (Nyquist keeps +), else i - NX.
+// In both slot orders the slots k < 8 hold rows below NX/2, k > 8 rows above, and k = 8 row NX/2 exactly when the base is 0.
+template <int NX, bool SPLIT = false>
 __device__ __forceinline__ int signed_row(const int t, const int k)
 {
-    constexpr int G = NX / 16;
-    const int i = t + k * G;
+    const int i = slot_pos<NX, SPLIT>(t, k);
     if (k < 8) return i;
-    if (k == 8) return (t == 0) ? i : i - NX;
+    if (k == 8) return (slot_base<NX, SPLIT>(t) == 0) ? i : i - NX;
     return i - NX;
 }
-
-// no-op hooks of col_fft
-struct ColFftNoHook {
-    __device__ __forceinline__ void operator()(int, bool) const {}
-};
-struct ColFftNoPre {
-    __device__ __forceinline__ void operator()() const {}
-};
 
 // hook(e, last): called by every thread after exchange e (0-based) has been read and its closing barrier passed --
 // a CTA-uniform point between two barriers where the caller can slip in unrelated pipelined work.

@@ -163,8 +163,13 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
     int t[1], c[1];
     c[0] = tid % FW;
     t[0] = tid / FW;
+    // NX = 8192 stepper: the forward transform leaves the tendency in the Split8192 order (two shared-memory exchanges instead
+    // of three); the epilogue, the state-array accesses and the parked stage state follow that order and the inverse
+    // transforms take it back to natural order for the staged tile
+    constexpr bool SPLIT = (NX == 8192) && (MODE == COL_STEP || MODE == COL_PRO);
     LineTw<NX> tw[1];
-    tw[0].init(p.tw, p.twn, t[0]);
+    if constexpr (SPLIT) Split8192::init_tw(tw[0], p.tw, p.twn, t[0]);
+    else tw[0].init(p.tw, p.twn, t[0]);
     if (tid == 0) {
         mbar_init(&full, 1);
         for (int i = 0; i < C::RING_SLOTS; ++i) mbar_init(&ring_bar[i], 1);
@@ -272,7 +277,7 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
                 const float kyv = (NG == 1 || cg == 0) ? ky_t0 : ky_t1;
                 const float ky2 = kyv * kyv;
                 const size_t soff = moff + (size_t)(tl * NG + cg) * (size_t)p.st_tile_stride;
-                const size_t e0 = soff + (size_t)t[0] * srow + c[0];
+                const size_t e0 = soff + (size_t)slot_base<NX, SPLIT>(t[0]) * srow + c[0];
                 // Epilogue operands (z0, zk, acc of this column group) in quarters of four rows.  The loads of the first
                 // quarter are issued INSIDE the forward transform, right before its last exchange, so that their L2
                 // latency passes under the exchange's two barriers and the final pass; the loads of quarter q + 1 are
@@ -284,22 +289,23 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
                 auto pre = [&]() {
                     if (MODE == COL_STEP) {
 #pragma unroll
-                        for (int q = 0; q < 4; ++q) qz0[q] = p.z0[e0 + (size_t)(q * G) * srow];
+                        for (int q = 0; q < 4; ++q) qz0[q] = p.z0[e0 + (size_t)slot_off<NX, SPLIT>(q) * srow];
                         if (p.stage != 1) {
 #pragma unroll
                             for (int q = 0; q < 4; ++q) {
-                                qzk[q] = p.zk[e0 + (size_t)(q * G) * srow];
-                                qac[q] = p.acc[e0 + (size_t)(q * G) * srow];
+                                qzk[q] = p.zk[e0 + (size_t)slot_off<NX, SPLIT>(q) * srow];
+                                qac[q] = p.acc[e0 + (size_t)slot_off<NX, SPLIT>(q) * srow];
                             }
                         }
                     }
                 };
                 ColFftNoHook nohook;
-                col_fft<NX, FW, 1, ColFftNoHook, decltype(pre)>(v, F, t, c, tw, false, nohook, pre);
+                if constexpr (SPLIT) fft8192_to_split<FW>(v[0], F, t[0], c[0], tw[0], CtaBar(), false, nohook, pre);
+                else col_fft<NX, FW, 1, ColFftNoHook, decltype(pre)>(v, F, t, c, tw, false, nohook, pre);
                 if (MODE == COL_FWDT) {
                     // plain forward transform of the tile into the tile-major state (xfb_set_vorticity: main.cpp:256)
 #pragma unroll
-                    for (int k = 0; k < 16; ++k) p.z0[e0 + (size_t)(k * G) * srow] = v[0][k];
+                    for (int k = 0; k < 16; ++k) p.z0[e0 + (size_t)slot_off<NX, SPLIT>(k) * srow] = v[0][k];
                 }
                 cpx znew[TKEEP ? 8 : 1];
 #pragma unroll
@@ -307,12 +313,12 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
                     cpx nz0[4], nzk[4], nac[4];
                     if (qd < 3) {
 #pragma unroll
-                        for (int q = 0; q < 4; ++q) nz0[q] = p.z0[e0 + (size_t)((4 * qd + 4 + q) * G) * srow];
+                        for (int q = 0; q < 4; ++q) nz0[q] = p.z0[e0 + (size_t)slot_off<NX, SPLIT>(4 * qd + 4 + q) * srow];
                         if (p.stage != 1) {
 #pragma unroll
                             for (int q = 0; q < 4; ++q) {
-                                nzk[q] = p.zk[e0 + (size_t)((4 * qd + 4 + q) * G) * srow];
-                                nac[q] = p.acc[e0 + (size_t)((4 * qd + 4 + q) * G) * srow];
+                                nzk[q] = p.zk[e0 + (size_t)slot_off<NX, SPLIT>(4 * qd + 4 + q) * srow];
+                                nac[q] = p.acc[e0 + (size_t)slot_off<NX, SPLIT>(4 * qd + 4 + q) * srow];
                             }
                         }
                     }
@@ -323,10 +329,10 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
                         const int k = 4 * qd + q;
-                        const int i = t[0] + k * G;
-                        const size_t e = e0 + (size_t)(k * G) * srow;
+                        const int i = slot_pos<NX, SPLIT>(t[0], k);
+                        const size_t e = e0 + (size_t)slot_off<NX, SPLIT>(k) * srow;
                         const cpx X = v[0][k];
-                        const float kxv = (float)signed_row<NX>(t[0], k) * p.kxscale;
+                        const float kxv = (float)signed_row<NX, SPLIT>(t[0], k) * p.kxscale;
                         const float lap = -fmaf(kxv, kxv, ky2);
                         // dvortdt_c += (vort_c * laplacian_coe) * NU                                  main.cpp:240-243
                         const float tx = __fadd_rn(X.x, __fmul_rn(__fmul_rn(qzk[q].x, lap), p.nu));
@@ -388,9 +394,9 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
         const cpx *zsrc = (MODE == COL_PRO || MODE == COL_DIAG || p.stage == 4) ? p.z0 : p.zk;
         const int NF = (MODE == COL_FWDT) ? 0 : (MODE == COL_DIAG) ? p.nfields : TRACER ? 2 : 4;
         if (KEEP && (MODE == COL_PRO || MODE == COL_DIAG)) {
-            const size_t e0 = moff + (size_t)tl * (size_t)p.st_tile_stride + (size_t)t[0] * srow + c[0];
+            const size_t e0 = moff + (size_t)tl * (size_t)p.st_tile_stride + (size_t)slot_base<NX, SPLIT>(t[0]) * srow + c[0];
 #pragma unroll
-            for (int k = 0; k < 16; ++k) zkeep[k] = zsrc[e0 + (size_t)(k * G) * srow];
+            for (int k = 0; k < 16; ++k) zkeep[k] = zsrc[e0 + (size_t)slot_off<NX, SPLIT>(k) * srow];
         }
 #pragma unroll 1
         for (int f = 0; f < NF; ++f) {
@@ -403,15 +409,16 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
                 if (TKEEP) {
                     tmem_unpark(tpark + (unsigned)(cg * 32), v[0]);
                 } else if (!KEEP) {
-                    const size_t e0 = moff + (size_t)(tl * NG + cg) * (size_t)p.st_tile_stride + (size_t)t[0] * srow + c[0];
+                    const size_t e0 =
+                        moff + (size_t)(tl * NG + cg) * (size_t)p.st_tile_stride + (size_t)slot_base<NX, SPLIT>(t[0]) * srow + c[0];
 #pragma unroll
-                    for (int k = 0; k < 16; ++k) v[0][k] = zsrc[e0 + (size_t)(k * G) * srow];
+                    for (int k = 0; k < 16; ++k) v[0][k] = zsrc[e0 + (size_t)slot_off<NX, SPLIT>(k) * srow];
                 }
 #pragma unroll
                 for (int k = 0; k < 16; ++k) {
-                    const int i = t[0] + k * G;
+                    const int i = slot_pos<NX, SPLIT>(t[0], k);
                     const cpx z = KEEP ? zkeep[k] : v[0][k];
-                    const float kx = (float)signed_row<NX>(t[0], k) * p.kxscale;
+                    const float kx = (float)signed_row<NX, SPLIT>(t[0], k) * p.kxscale;
                     if (MODE == COL_DIAG) {
                         // p.stage 0: psi_xy, psi_xx, psi_yy = (kx ky, kx^2, ky^2) Z / (kx^2+ky^2)   [(i kx)(i ky) Z/-(k^2) ...]
                         // p.stage 1: zeta, zeta_x, zeta_y   = (1, i kx, i ky) Z
@@ -453,8 +460,16 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
                 }
                 // S is about to be overwritten: the bulk store of the previous field (or tile) must have read it.
                 // Thread 0 waits inside the transform, before its last exchange barrier (col_fft, drain_tma).
-                if (TRING) col_fft<NX, FW, 1, ColtRing<NX>>(v, F, t, c, tw, cg == 0, rs);
-                else col_fft<NX, FW, 1>(v, F, t, c, tw, cg == 0);
+                if constexpr (SPLIT) {
+                    ColFftNoHook nohook;
+                    ColFftNoPre nopre;
+                    if (TRING) fft8192_from_split<FW>(v[0], F, t[0], c[0], tw[0], CtaBar(), cg == 0, rs, nopre);
+                    else fft8192_from_split<FW>(v[0], F, t[0], c[0], tw[0], CtaBar(), cg == 0, nohook, nopre);
+                } else if (TRING) {
+                    col_fft<NX, FW, 1, ColtRing<NX>>(v, F, t, c, tw, cg == 0, rs);
+                } else {
+                    col_fft<NX, FW, 1>(v, F, t, c, tw, cg == 0);
+                }
                 cpx *dst = S + s_base + 2 * (col ^ swz);
 #pragma unroll
                 for (int k = 0; k < 16; ++k) dst[k * G * TW] = cswap(v[0][k]);

@@ -477,4 +477,173 @@ __device__ __forceinline__ void line_fft(cpx (&v)[16], cpx *sm, const int t, con
     rem_pass<L>(v, tw);
 }
 
+// no-op hooks of col_fft and of the split 8192-point transforms below
+struct ColFftNoHook {
+    __device__ __forceinline__ void operator()(int, bool) const {}
+};
+struct ColFftNoPre {
+    __device__ __forceinline__ void operator()() const {}
+};
+
+// ---- 8192-point lines with two exchanges: the radix-2 stage across lane pairs ------------------------------------------
+// line_fft<8192> is R16 -> ex -> R16 -> ex -> R16 -> ex -> R2; the third exchange only regroups the data for the radix-2
+// butterflies (j, j + 4096).  Here the third radix-16 pass is run by a remapped thread: thread t (warp w, lane l, lane half
+// h = l >> 4) does the pass of the Stockham thread tau = 256 h + 16 w + (l & 15), so it ends up with E[j0 + 256 s] (h = 0) or
+// O[j0 + 256 s] (h = 1), j0 = 16 w + (l & 15), s = 0..15: the two halves of every radix-2 butterfly sit in lanes l and l ^ 16.
+// Lane h = 1 runs that pass with its twiddle base negated, which rotates its outputs by 8 slots (O[j0 + 256 ((s + 8) & 15)]
+// in slot s), so both lanes send slot 8 + i and keep slot i; 8 complex values cross each way (16 shfl.xor per thread), and
+// lane h owns the butterflies s = 8 h + i, i = 0..7.  The result is in the SPLIT order of Split8192::pos: slot k of thread t
+// holds X[j0 + 2048 h + 256 (k & 7) + 4096 (k >> 3)].
+//   fft8192_to_split   : input at t + 512 k (natural), output in the split order
+//   fft8192_from_split : the transposed algorithm (lane-pair stage first, butterflies before twiddles), input in the split
+//                        order, output at t + 512 k
+// Both are forward transforms and use the twiddle bases of Split8192::init_tw.  The line's threads must be aligned to warps
+// (t % 32 = lane), which holds for every 512-thread line.  tests/test_fft8192_lane_split_model.py models the addressing.
+struct Split8192 {
+    static constexpr int L = 8192, G = 512;
+    __device__ static __forceinline__ int half(const int t) { return (t >> 4) & 1; }
+    __device__ static __forceinline__ int j0(const int t) { return ((t >> 5) << 4) | (t & 15); }
+    // the Stockham thread whose third radix-16 pass thread t runs
+    __device__ static __forceinline__ int tau(const int t) { return (half(t) << 8) | j0(t); }
+    // position of slot k of thread t: base(t) + off(k)
+    __device__ static __forceinline__ int base(const int t) { return j0(t) + (half(t) << 11); }
+    __host__ __device__ static constexpr int off(const int k) { return ((k & 7) << 8) + ((k >> 3) << 12); }
+    // b[1] = exp(-2 pi i (t mod 16) / 256) as LineTw (tau mod 16 = t mod 16), b[2] = (-1)^h exp(-2 pi i j0 / 4096) for the
+    // third pass, b[0] = exp(-2 pi i base(t) / 8192) for the lane-pair stage (times W32^i for butterfly s = 8 h + i)
+    __device__ static __forceinline__ void init_tw(LineTw<L> &tw, const cpx *__restrict__ tab, const int twn, const int t)
+    {
+        tw.b[1] = __ldg(tab + (size_t)(t & 15) * (twn / 256));
+        const cpx b2 = __ldg(tab + (size_t)j0(t) * (twn / 4096));
+        tw.b[2] = half(t) ? mk(-b2.x, -b2.y) : b2;
+        tw.b[0] = __ldg(tab + (size_t)base(t) * (twn / L));
+    }
+};
+
+// slot k of thread t of a transformed line of length L: position t + k * L/16, or Split8192 order
+template <int L, bool SPLIT>
+__device__ __forceinline__ int slot_base(const int t) { return SPLIT ? Split8192::base(t) : t; }
+template <int L, bool SPLIT>
+__host__ __device__ __forceinline__ constexpr int slot_off(const int k) { return SPLIT ? Split8192::off(k) : k * (L / 16); }
+template <int L, bool SPLIT>
+__device__ __forceinline__ int slot_pos(const int t, const int k) { return slot_base<L, SPLIT>(t) + slot_off<L, SPLIT>(k); }
+
+// W32^i = exp(-2 pi i i / 32), i = 0..7
+#define XFB_C32 0.98078528040323044913f
+#define XFB_S32 0.19509032201612826785f
+#define XFB_C32_3 0.83146961230254523708f
+#define XFB_S32_3 0.55557023301960222474f
+__device__ __forceinline__ cpx lane_pair_twiddle(const cpx wb, const int i)
+{
+    const float CQ[8] = {1.f, XFB_C32, XFB_C16, XFB_C32_3, XFB_C8, XFB_S32_3, XFB_S16, XFB_S32};
+    const float SQ[8] = {0.f, -XFB_S32, -XFB_S16, -XFB_S32_3, -XFB_C8, -XFB_C32_3, -XFB_C16, -XFB_C32};
+    return (i == 0) ? wb : cmul(wb, mk(CQ[i], SQ[i]));
+}
+__device__ __forceinline__ cpx shfl_xor16(const cpx a)
+{
+    return mk(__shfl_xor_sync(0xffffffffu, a.x, 16), __shfl_xor_sync(0xffffffffu, a.y, 16));
+}
+
+// the exchange patterns of exchange_read / exchange_write, the other way round (transposed transforms)
+template <int G, int W>
+__device__ __forceinline__ void exchange_write_strided(const cpx (&v)[16], cpx *sm, const int t, const int c)
+{
+    static_assert(G % 16 == 0, "constant offsets need G % 16 == 0");
+    cpx *dst = sm + padpos(t) * W + c;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) dst[k * (G + G / 16) * W] = v[k];
+}
+template <int W>
+__device__ __forceinline__ void exchange_read_stockham(cpx (&v)[16], const cpx *sm, const int t, const int c, const int ns)
+{
+    const int base = (t / ns) * ns * 16 + (t % ns);
+    const cpx *src = sm + padpos(base) * W + c;
+#pragma unroll
+    for (int s = 0; s < 16; ++s) v[s] = src[(s * ns + ((s * ns) >> 4)) * W];
+}
+
+// hook(e, last) after exchange e has been read and its closing barrier passed; pre() right before the writes of the last
+// exchange; drain_tma: thread 0 waits for the bulk stores reading shared memory before the last exchange's first barrier
+// (the same points as col_fft)
+template <int W, typename Bar, class Hook, class Pre>
+__device__ __forceinline__ void fft8192_to_split(cpx (&v)[16], cpx *sm, const int t, const int c, const LineTw<8192> &tw,
+                                                 const Bar &bar, const bool drain_tma, Hook &hook, Pre &pre)
+{
+    constexpr int G = Split8192::G;
+    pass16_compute<8192>(v, 0, tw);
+    exchange_write<W>(v, sm, t, c, 1);
+    bar.sync();
+    exchange_read<G, W>(v, sm, t, c);
+    bar.sync();
+    hook(0, false);
+    pass16_compute<8192>(v, 1, tw);
+    pre();
+    exchange_write<W>(v, sm, t, c, 16);
+    if (drain_tma && threadIdx.x == 0) tma_wait_read_all();
+    bar.sync();
+    exchange_read<G, W>(v, sm, Split8192::tau(t), c);
+    bar.sync();
+    hook(1, true);
+    pass16_compute<8192>(v, 2, tw);
+    // lane h: e = E (own slot i for h = 0, received for h = 1), o = O; butterfly s = 8 h + i -> slots i, 8 + i
+    const bool hi = Split8192::half(t);
+    const cpx wb = launder(tw.b[0]);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const cpx r = shfl_xor16(v[8 + i]);
+        const cpx e = hi ? r : v[i], o = hi ? v[i] : r;
+        const cpx b = cmul(o, lane_pair_twiddle(wb, i));
+        v[i] = cadd(e, b);
+        v[8 + i] = csub(e, b);
+    }
+}
+
+template <int W, typename Bar, class Hook, class Pre>
+__device__ __forceinline__ void fft8192_from_split(cpx (&v)[16], cpx *sm, const int t, const int c, const LineTw<8192> &tw,
+                                                   const Bar &bar, const bool drain_tma, Hook &hook, Pre &pre)
+{
+    constexpr int G = Split8192::G;
+    // transposed radix-2 butterflies (E' = x_j + x_(j+4096), O' = w^j (x_j - x_(j+4096))); lane h keeps E' (h = 0) or O'
+    // (h = 1) in slot i and receives the partner's in slot 8 + i: the rotated order the transposed third pass expects
+    const bool hi = Split8192::half(t);
+    const cpx wb = launder(tw.b[0]);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const cpx a = cadd(v[i], v[8 + i]), b = cmul(csub(v[i], v[8 + i]), lane_pair_twiddle(wb, i));
+        v[i] = hi ? b : a;
+        v[8 + i] = shfl_xor16(hi ? a : b);
+    }
+    dft16(v);
+    apply_twiddles16(v, launder(tw.b[2]));
+    exchange_write_strided<G, W>(v, sm, Split8192::tau(t), c);
+    bar.sync();
+    exchange_read_stockham<W>(v, sm, t, c, 16);
+    bar.sync();
+    hook(0, false);
+    dft16(v);
+    apply_twiddles16(v, launder(tw.b[1]));
+    pre();
+    exchange_write_strided<G, W>(v, sm, t, c);
+    if (drain_tma && threadIdx.x == 0) tma_wait_read_all();
+    bar.sync();
+    exchange_read_stockham<W>(v, sm, t, c, 1);
+    bar.sync();
+    hook(1, true);
+    dft16(v);
+}
+
+template <int W, typename Bar>
+__device__ __forceinline__ void fft8192_to_split(cpx (&v)[16], cpx *sm, const int t, const int c, const LineTw<8192> &tw, const Bar &bar)
+{
+    ColFftNoHook hook;
+    ColFftNoPre pre;
+    fft8192_to_split<W>(v, sm, t, c, tw, bar, false, hook, pre);
+}
+template <int W, typename Bar>
+__device__ __forceinline__ void fft8192_from_split(cpx (&v)[16], cpx *sm, const int t, const int c, const LineTw<8192> &tw, const Bar &bar)
+{
+    ColFftNoHook hook;
+    ColFftNoPre pre;
+    fft8192_from_split<W>(v, sm, t, c, tw, bar, false, hook, pre);
+}
+
 }  // namespace xfb

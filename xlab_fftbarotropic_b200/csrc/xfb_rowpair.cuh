@@ -77,12 +77,14 @@ __device__ __forceinline__ void c2r_pair_staged(cpx (&v)[16], cpx *sm, const int
 }
 
 // v[q] = (a[n], b[n]) -> half spectra of both rows written to the pair at PBout (+ zeroed pad columns)
-template <int NY, bool DIST, typename Bar, bool RELEASE = false>
+// SPLIT (NY = 8192): v arrives in the Split8192 order and is transformed by fft8192_from_split, natural order out
+template <int NY, bool DIST, typename Bar, bool RELEASE = false, bool SPLIT = false>
 __device__ __forceinline__ void r2c_pair(cpx (&v)[16], cpx *__restrict__ PBout, const RowParams &p, const int pitch, cpx *sm,
                                          const int t, const LineTw<NY> &tw, const Bar &bar)
 {
     constexpr int G = NY / 16;
-    line_fft<NY, 1>(v, sm, t, 0, tw, bar);
+    if constexpr (SPLIT) fft8192_from_split<1>(v, sm, t, 0, tw, bar);
+    else line_fft<NY, 1>(v, sm, t, 0, tw, bar);
 #pragma unroll
     for (int q = 0; q < 16; ++q) sm[padpos(t + q * G)] = v[q];
     bar.sync();
@@ -233,8 +235,12 @@ rowpair_jac_tmem_kernel(const RowParams p)
     unsigned long long *mbar = &mbar_all[2 * lane_pair];
     const int npairs = p.nrows >> 1;
 
+    // NY = 8192: the inverse transforms leave their products in the Split8192 order (two shared-memory exchanges instead of
+    // three), the forward transform of J takes them from there
+    constexpr bool SPLIT = (NY == 8192);
     LineTw<NY> tw;
-    tw.init(p.tw, p.twn, t);
+    if constexpr (SPLIT) Split8192::init_tw(tw, p.tw, p.twn, t);
+    else tw.init(p.tw, p.twn, t);
     typedef typename RowBarSel<(G >= 32 && C::PPC > 1)>::type Bar;
     const Bar bar = RowBarSel<(G >= 32 && C::PPC > 1)>::make(1 + lane_pair, G);
 
@@ -292,7 +298,8 @@ rowpair_jac_tmem_kernel(const RowParams p)
         }
         bar.sync();                 // everyone has read this staging buffer: refill it two fields ahead
         XFB_FETCH(n + 2);
-        line_fft<NY, 1>(v, sm, t, 0, tw, bar);
+        if constexpr (SPLIT) fft8192_to_split<1>(v, sm, t, 0, tw, bar);
+        else line_fft<NY, 1>(v, sm, t, 0, tw, bar);
         // v = (b[n], a[n]) unscaled, swapped: .y is row 2m, .x row 2m+1.  Tensor-memory traffic in halves of
         // eight values (16 registers) so that nothing spills next to the live butterfly set.
         if (f == 0 || f == 2) {
@@ -334,15 +341,17 @@ rowpair_jac_tmem_kernel(const RowParams p)
         const int pr = XFB_PAIR_OF(g);
         const bool alive = g * C::PPC + lane_pair < npairs;
         if (p.real_in != nullptr) {
-            const float *sa = p.real_in + (size_t)pr * (size_t)(2 * NY), *sb = sa + NY;
+            const float *sa = p.real_in + (size_t)pr * (size_t)(2 * NY) + slot_base<NY, SPLIT>(t), *sb = sa + NY;
 #pragma unroll
-            for (int q = 0; q < 16; ++q) v[q] = mk(v[q].x + __ldg(sa + t + q * G), v[q].y + __ldg(sb + t + q * G));
+            for (int q = 0; q < 16; ++q)
+                v[q] = mk(v[q].x + __ldg(sa + slot_off<NY, SPLIT>(q)), v[q].y + __ldg(sb + slot_off<NY, SPLIT>(q)));
         }
         // the thread index is laundered per pair: otherwise the 24 padded shared-memory positions of the forward
         // transform's tail are hoisted out of the pair loop and spilled (16 local loads per pair on the critical path)
         int tl = t;
         asm volatile("" : "+r"(tl));
-        r2c_pair<NY, false>(v, p.spec_out + (size_t)pr * (size_t)(2 * p.pitch), p, alive ? p.pitch : 0, sm, tl, tw, bar);
+        r2c_pair<NY, false, Bar, false, SPLIT>(v, p.spec_out + (size_t)pr * (size_t)(2 * p.pitch), p, alive ? p.pitch : 0, sm, tl, tw,
+                                               bar);
     }
 #undef XFB_FETCH
 #undef XFB_PAIR_OF
