@@ -133,6 +133,16 @@ int xfb_get_energy_spectrum(xfb_handle h, int member, int which, int nshells, do
 int xfb_set_tracer(xfb_handle h, int member, const float *tracer, float kappa);
 int xfb_get_tracer_keff_hist(xfb_handle h, int member, int nbins, float cmin, float cmax, double *area, double *grad2);
 
+/* ---- linear terms (the reference has only nu lap(zeta)) -------------------------------------------
+ * d(zeta)/dt = -u.grad(zeta) + src + nu lap(zeta) - beta v - mu zeta - nu_h (-lap)^order zeta, v = d(psi)/dx, x the slow
+ * index: beta-plane (beta > 0: f grows with y; Rossby waves propagate westward), linear drag, hyperviscosity.  Per mode
+ * the step adds L(k) Z_k inside the dealiasing mask, L(k) = -mu - nu_h k^(2 order) + i beta kx / k^2 (DESIGN.md section 3).
+ * Acts on every member of the handle; the passive tracer keeps kappa lap(c) only.  order 1..8, mu >= 0, nu_h >= 0, all
+ * finite (beta may be negative), and nu_h k_c^(2 order) must be a normal float (k_c: the grid's largest wavenumber), else
+ * XFB_E_ARG.  All zeros switches the terms off.  Slab-decomposed handles: per rank, no communication -- every rank must
+ * pass the same values. */
+int xfb_set_linear_terms(xfb_handle h, float beta, float mu, float nu_h, int order);
+
 /* ---- pressure inversion: replaces the loop body of src/invert_pres.cpp:132-187 ---------------*/
 int xfb_invert_pres(xfb_handle h, const float *psi, float *pres, size_t ref_x, size_t ref_y, float rho, float f);
 
@@ -168,6 +178,7 @@ int xfb_loopback_destroy(xfb_loopback t);
 int xfb_loopback_set_vorticity(xfb_loopback t, const float *vort);
 int xfb_loopback_set_source(xfb_loopback t, const float *src);
 int xfb_loopback_set_tracer(xfb_loopback t, const float *tracer, float kappa);
+int xfb_loopback_set_linear_terms(xfb_loopback t, float beta, float mu, float nu_h, int order);
 int xfb_loopback_step(xfb_loopback t, int nsteps, float dt);
 int xfb_loopback_get_field(xfb_loopback t, int which, float *out);
 int xfb_loopback_get_diagnostics(xfb_loopback t, float *tfil, float *deform);

@@ -29,6 +29,7 @@ SYMBOLS = [
     "xfb_loopback_step", "xfb_loopback_get_field", "xfb_loopback_launch_count", "xfb_loopback_get_diagnostics",
     "xfb_loopback_get_keff_hist", "xfb_loopback_set_tracer",
     "xfb_get_energy_spectrum", "xfb_loopback_get_energy_spectrum",
+    "xfb_set_linear_terms", "xfb_loopback_set_linear_terms",
 ]
 
 _lib = None
@@ -70,6 +71,8 @@ def load():
     L.xfb_get_energy_spectrum.argtypes = [vp, ci, ci, ci, vp, vp, vp]
     L.xfb_loopback_get_energy_spectrum.argtypes = [vp, ci, ci, vp, vp, vp]
     L.xfb_set_tracer.argtypes = [vp, ci, vp, cf]
+    L.xfb_set_linear_terms.argtypes = [vp, cf, cf, cf, ci]
+    L.xfb_loopback_set_linear_terms.argtypes = [vp, cf, cf, cf, ci]
     L.xfb_invert_pres.argtypes = [vp, vp, vp, C.c_size_t, C.c_size_t, cf, cf]
     L.xfb_launch_count.restype = C.c_longlong
     L.xfb_launch_count.argtypes = [vp]
@@ -237,6 +240,11 @@ class Backend:
         else:
             s = np.ascontiguousarray(s, dtype=np.float32).reshape(self.nx, self.ny)
             self._ck(self._L.xfb_set_source(self._h, member, _ptr(s)))
+
+    def set_linear_terms(self, beta=0.0, mu=0.0, nu_h=0.0, order=4):
+        """-beta v - mu zeta - nu_h (-lap)^order zeta added to the vorticity tendency of every member (DESIGN.md
+        section 3); all zeros switches them off.  Slab ranks: every rank passes the same values."""
+        self._ck(self._L.xfb_set_linear_terms(self._h, float(beta), float(mu), float(nu_h), int(order)))
 
     def step(self, nsteps, dt):
         self._ck(self._L.xfb_step(self._h, int(nsteps), float(dt)))
@@ -407,6 +415,10 @@ class LoopbackTeam:
     def set_tracer(self, c, kappa):
         c = np.ascontiguousarray(c, dtype=np.float32).reshape(self.n, self.n)
         self._ck(self._L.xfb_loopback_set_tracer(self._t, _ptr(c), float(kappa)))
+
+    def set_linear_terms(self, beta=0.0, mu=0.0, nu_h=0.0, order=4):
+        """Backend.set_linear_terms on every rank"""
+        self._ck(self._L.xfb_loopback_set_linear_terms(self._t, float(beta), float(mu), float(nu_h), int(order)))
 
     def step(self, nsteps, dt):
         self._ck(self._L.xfb_loopback_step(self._t, int(nsteps), float(dt)))

@@ -19,6 +19,10 @@
 //      `step time member E Z P`, and the isotropic shell spectra written to <output>/spectrum_step_N.txt -- .m<m>.txt for
 //      members other than 0 -- one `s k[1/m] E(s) Z(s)` line per shell; neither goes into `log`.  A non-finite total
 //      stops the run with exit status 1 once the record files already issued are written).
+//   -B <beta> -R <mu> -H <nu_h> -P <order=4> (linear terms of the vorticity equation, xfb_set_linear_terms: beta-plane
+//      [1/(m s)], linear drag [1/s], hyperviscosity nu_h (-lap)^order [m^(2 order)/s], order 1..8; on every handle of the
+//      run, -b, -G and -S ranks included.  An invalid value stops with exit status 1 before any step.  Without these
+//      flags the run is the reference's equation and its output is unchanged).
 // Record output is asynchronous (SURVEY.md 8f-2): at a record step the five fields are formed on the GPU and copied
 // to pinned host buffers on a second stream (xfb_get_field_async) while the next stretch of steps already runs; a
 // writer thread waits for each buffer, calls writeField and appends the `log` line -- same files, same order as the
@@ -84,11 +88,34 @@ static int write_energy(const std::string &output, FILE *integrals, int step, fl
     return (std::isfinite(tot[0]) && std::isfinite(tot[1]) && std::isfinite(tot[2])) ? 0 : 1;
 }
 
+// -B -R -H -P: the linear terms, applied to every handle the run creates
+struct LinOpts {
+    bool set;
+    float beta, mu, nu_h;
+    int order;
+};
+
+static int set_linear(xfb_handle h, const LinOpts &lin)
+{
+    return lin.set ? xfb_set_linear_terms(h, lin.beta, lin.mu, lin.nu_h, lin.order) : 0;
+}
+
+// a finite float option value; false on trailing characters or an unparsable / non-finite value
+static bool parse_float(const char *s, float *out)
+{
+    char *end = nullptr;
+    const double v = std::strtod(s, &end);
+    if (end == s || *end != '\0' || !std::isfinite(v) || !std::isfinite((float)v)) return false;
+    *out = (float)v;
+    return true;
+}
+
 struct SlabOpts {
     std::string input, output, init_file;
     int npts, record_step, total_steps, device, ranks;
     float L, NU, dt;
     bool diagnostics, quiet, energy;
+    LinOpts lin;
 };
 
 // one rank of `-S <ranks>`: local rows [row0, row0 + rows) of every file
@@ -99,6 +126,7 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
     while (nchunks > 1 && ((n / o.ranks) % nchunks != 0 || ((n / o.ranks) / nchunks) % 2 != 0)) nchunks /= 2;
     xfb_handle h = nullptr;
     CHECK(xfb_create_dist(&h, n, n, o.L, o.L, o.NU, o.device + rank, rank, o.ranks, nchunks, id128));
+    CHECK(set_linear(h, o.lin));                                   // per rank, the same values everywhere
     CHECK(xfb_slab_partition(n, n, o.ranks, nchunks, rank, &row0, &rows, nullptr, nullptr, nullptr, nullptr));
     const size_t local = (size_t)rows * n;
     const off_t off = (off_t)row0 * n * (off_t)sizeof(float);
@@ -221,9 +249,11 @@ int main(int argc, char *args[])
     int npts = 768, record_step = 100, total_steps = -1, device = 0, members = 1, ngpus = 1, slab_ranks = 0;
     float L = 600000.0f, NU = 6.5f, dt = 3.0f;
     bool diagnostics = false, quiet = false, energy = false;
+    LinOpts lin{false, 0.0f, 0.0f, 0.0f, 4};
+    bool bad_lin = false;
 
     int opt;
-    while ((opt = getopt(argc, args, "I:O:o:i:s:f:n:d:t:r:L:N:g:c:k:b:G:S:DEq")) != EOF) {
+    while ((opt = getopt(argc, args, "I:O:o:i:s:f:n:d:t:r:L:N:g:c:k:b:G:S:B:R:H:P:DEq")) != EOF) {
         switch (opt) {
         case 'I': input = optarg; break;
         case 'O': case 'o': output = optarg; break;
@@ -245,7 +275,22 @@ int main(int argc, char *args[])
         case 'D': diagnostics = true; break;
         case 'E': energy = true; break;
         case 'q': quiet = true; break;
+        case 'B': lin.set = true; bad_lin |= !parse_float(optarg, &lin.beta); break;
+        case 'R': lin.set = true; bad_lin |= !parse_float(optarg, &lin.mu) || lin.mu < 0.0f; break;
+        case 'H': lin.set = true; bad_lin |= !parse_float(optarg, &lin.nu_h) || lin.nu_h < 0.0f; break;
+        case 'P': {
+            lin.set = true;
+            char *end = nullptr;
+            const long v = std::strtol(optarg, &end, 10);
+            if (end == optarg || *end != '\0' || v < 1 || v > 8) bad_lin = true;
+            else lin.order = (int)v;
+            break;
         }
+        }
+    }
+    if (bad_lin) {
+        std::fprintf(stderr, "main.out: -B <beta> -R <mu> -H <nu_h> -P <order>: finite numbers, mu >= 0, nu_h >= 0, order 1..8\n");
+        return 1;
     }
     if (total_steps < 0) total_steps = (int)(60 * 60 / dt);          // configuration.hpp:36
     if (record_step < 1) record_step = 1;
@@ -273,7 +318,7 @@ int main(int argc, char *args[])
             return 1;
         }
         SlabOpts so{input, output, init_file, npts, record_step, total_steps, device, slab_ranks, L, NU, dt, diagnostics, quiet,
-                    energy};
+                    energy, lin};
         return run_slab(so);
     }
 
@@ -295,6 +340,7 @@ int main(int argc, char *args[])
         first[d] = (int)((long long)members * d / ngpus);
         count[d] = (int)((long long)members * (d + 1) / ngpus) - first[d];
         CHECK(xfb_create(&hs[d], npts, npts, L, L, NU, count[d], device + d));
+        CHECK(set_linear(hs[d], lin));
     }
     auto owner = [&](int m, int *local) { int d = 0; while (m >= first[d] + count[d]) ++d; *local = m - first[d]; return hs[d]; };
     xfb_handle h = hs[0];

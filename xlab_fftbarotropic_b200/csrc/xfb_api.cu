@@ -1,5 +1,6 @@
 // xfb_api.cu -- the C ABI declared in include/xfb.h: handle, tables, operator tier, stepper.
 // No CPU fallback lives here: every entry point needs a CUDA device and says so when it fails.
+#include <cfloat>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -496,6 +497,7 @@ void xfb::fill_col(xfb_handle h, ColParams &p, int chunk)
     p.mask_kd_i = (int)h->mask_kd;
     p.st_tile_stride = col_tile_width(h->nx); p.st_row_stride = h->pitch;      // row-major unless the stepper says otherwise
     p.kxscale = (acosf(-1.0f) * 2.0f) / h->lx;
+    p.lin = h->lin;
 }
 
 // real [nx][ny] (device) -> padded spectrum (device), via `tmp` (padded)
@@ -698,6 +700,44 @@ extern "C" int xfb_set_tracer(xfb_handle h, int member, const float *tracer, flo
     h->kappa = kappa;
     h->tcf_valid = false;
     if (!is_device_ptr(tracer)) CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+// Linear terms of the vorticity equation (DESIGN.md section 3): -beta v - mu zeta - nu_h (-lap)^order zeta, added per mode as
+// L(k) Z_k next to the nu term inside the dealiasing mask of every Runge-Kutta stage.  The passive tracer keeps its kappa
+// lap(c) only.  With a non-zero term the stepper runs the LIN instances of its K-COL kernels (and of gen_stage on the
+// generic grids); all zeros switches back to the default kernels.  A change drops the captured step graph, which bakes
+// the kernel parameters in.
+extern "C" int xfb_set_linear_terms(xfb_handle h, float beta, float mu, float nu_h, int order)
+{
+    if (!h) return fail(XFB_E_ARG, "null handle");
+    if (!std::isfinite(beta) || !std::isfinite(mu) || !std::isfinite(nu_h))
+        return fail(XFB_E_ARG, "xfb_set_linear_terms: beta, mu and nu_h must be finite");
+    if (mu < 0.0f || nu_h < 0.0f) return fail(XFB_E_ARG, "xfb_set_linear_terms: mu and nu_h must be >= 0");
+    if (order < 1 || order > 8) return fail(XFB_E_ARG, "xfb_set_linear_terms: order %d not in 1..8", order);
+    LinCoef L;
+    memset(&L, 0, sizeof(L));
+    if (beta != 0.0f || mu != 0.0f || nu_h != 0.0f) {
+        // hyperviscosity as ch (k^2 / k_c^2)^order with the largest wavenumber of the grid, k_c^2 = kx(nx/2)^2 + ky(ny/2)^2
+        // (the float expressions of the wavenumber tables): (k^2 / k_c^2)^order <= 1 never overflows, whatever the size
+        // and domain length; ch = nu_h k_c^(2 order) is formed in float64 and must be a normal float
+        const float TWOPI = acosf(-1.0f) * 2.0f;
+        const double kxc = (double)(TWOPI * ((float)(h->nx / 2)) / h->lx), kyc = (double)(TWOPI * ((float)(h->ny / 2)) / h->ly);
+        const double kc2 = kxc * kxc + kyc * kyc;
+        const double ch = (double)nu_h * std::pow(kc2, (double)order);
+        if (!std::isfinite(ch) || ch > (double)FLT_MAX || (nu_h != 0.0f && ch < (double)FLT_MIN))
+            return fail(XFB_E_ARG, "xfb_set_linear_terms: nu_h * k_c^%d = %g is out of float range", 2 * order, ch);
+        L.beta = beta; L.mu = mu; L.ch = (float)ch; L.inv_kc2 = (float)(1.0 / kc2); L.order = order; L.on = 1;
+    }
+    if (memcmp(&L, &h->lin, sizeof(L)) != 0) {
+        // the captured step (fused or generic path) has the old coefficients baked in
+        if (h->step_graph) {
+            CK(cudaSetDevice(h->device));
+            cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph);
+            h->step_graph = nullptr;
+        }
+        h->lin = L;
+    }
     return 0;
 }
 

@@ -68,13 +68,13 @@ static int make_pair_map(CUtensorMap *m, const void *base, long long rows, int p
     return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
 }
 
-template <int NX, int MODE>
+template <int NX, int MODE, bool LIN = false>
 static int launch_colt_t(const ColParams &p, int batch, cudaStream_t st)
 {
     typedef ColTCfg<NX> C;
     static PerDeviceInt cfg;
     int err = 0;
-    const int resident = cfg.get([&](int *e) { return resident_ctas(colt_kernel<NX, MODE>, C::THREADS, C::SMEM, 0, e); }, &err);
+    const int resident = cfg.get([&](int *e) { return resident_ctas(colt_kernel<NX, MODE, LIN>, C::THREADS, C::SMEM, 0, e); }, &err);
     if (resident <= 0) return err;
     ColTMaps maps;
     const long long rows = (long long)NX * batch;
@@ -93,18 +93,18 @@ static int launch_colt_t(const ColParams &p, int batch, cudaStream_t st)
     }
     const int tiles_per_member = p.pitch / C::TW, tiles_total = tiles_per_member * batch;
     const int blocks = tiles_total < resident ? tiles_total : resident;
-    colt_kernel<NX, MODE><<<blocks, C::THREADS, C::SMEM, st>>>(p, maps, tiles_per_member, tiles_total);
+    colt_kernel<NX, MODE, LIN><<<blocks, C::THREADS, C::SMEM, st>>>(p, maps, tiles_per_member, tiles_total);
     return (int)cudaGetLastError();
 }
 
 // two-level K-COL (xfb_col2l.cuh): columns of 16384 points (and 4096 under XFB_COL_2L=1, a test knob)
-template <int NX, int MODE>
+template <int NX, int MODE, bool LIN = false>
 static int launch_col2l_t(const ColParams &p, int batch, cudaStream_t st)
 {
     typedef Col2LCfg<NX> C;
     static PerDeviceInt cfg;
     int err = 0;
-    const int resident = cfg.get([&](int *e) { return resident_ctas(col2l_kernel<NX, MODE>, C::THREADS, C::SMEM, C::TCOLS, e); }, &err);
+    const int resident = cfg.get([&](int *e) { return resident_ctas(col2l_kernel<NX, MODE, LIN>, C::THREADS, C::SMEM, C::TCOLS, e); }, &err);
     if (resident <= 0) return err;
     CUtensorMap jmap = CUtensorMap();
     if (MODE == COL_STEP || MODE == COL_TSTEP)      // one-column boxes of the tendency: 2 elements (one 16-byte piece) x BOXR row pairs
@@ -120,7 +120,7 @@ static int launch_col2l_t(const ColParams &p, int batch, cudaStream_t st)
         const int fewer = resident - spare;
         if ((ncols + fewer - 1) / fewer == (ncols + resident - 1) / resident) blocks = ncols < fewer ? ncols : fewer;
     }
-    col2l_kernel<NX, MODE><<<blocks, C::THREADS, C::SMEM, st>>>(p, jmap, ncols);
+    col2l_kernel<NX, MODE, LIN><<<blocks, C::THREADS, C::SMEM, st>>>(p, jmap, ncols);
     return (int)cudaGetLastError();
 }
 
@@ -131,7 +131,8 @@ static int launch_colt_n(int mode, const ColParams &p, int batch, cudaStream_t s
     if (mode == COL_FWDT) return launch_colt_t<NX, COL_FWDT>(p, batch, st);
     if (mode == COL_TSTEP) return launch_colt_t<NX, COL_TSTEP>(p, batch, st);
     if (mode == COL_TPRO) return launch_colt_t<NX, COL_TPRO>(p, batch, st);
-    return mode == COL_STEP ? launch_colt_t<NX, COL_STEP>(p, batch, st) : launch_colt_t<NX, COL_PRO>(p, batch, st);
+    if (mode == COL_STEP) return p.lin.on ? launch_colt_t<NX, COL_STEP, true>(p, batch, st) : launch_colt_t<NX, COL_STEP>(p, batch, st);
+    return launch_colt_t<NX, COL_PRO>(p, batch, st);
 }
 
 template <int NX, int W, int MODE>
@@ -167,10 +168,15 @@ int launch_col(int nx, int mode, const ColParams &p, int batch, cudaStream_t st)
         }
         return (int)cudaErrorInvalidValue;
     }
-    // the stepper's modes: two-level kernel on 16384-point columns, TMA-staged persistent kernel on shorter ones
+    // the stepper's modes: two-level kernel on 16384-point columns, TMA-staged persistent kernel on shorter ones;
+    // COL_STEP with a non-zero linear term (p.lin.on, xfb_set_linear_terms) runs the LIN instance of the same kernel
     if ((mode == COL_STEP || mode == COL_PRO) && col_two_level(nx)) {
-        if (nx == 16384)
+        const bool lin = (mode == COL_STEP) && p.lin.on;
+        if (nx == 16384) {
+            if (lin) return launch_col2l_t<16384, COL_STEP, true>(p, batch, st);
             return mode == COL_STEP ? launch_col2l_t<16384, COL_STEP>(p, batch, st) : launch_col2l_t<16384, COL_PRO>(p, batch, st);
+        }
+        if (lin) return launch_col2l_t<4096, COL_STEP, true>(p, batch, st);
         return mode == COL_STEP ? launch_col2l_t<4096, COL_STEP>(p, batch, st) : launch_col2l_t<4096, COL_PRO>(p, batch, st);
     }
     if (nx == 16384) {      // passive tracer on the 16384 grid; the diagnostics modes have no 16384 kernel

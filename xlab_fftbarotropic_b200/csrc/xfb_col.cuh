@@ -23,6 +23,32 @@ namespace xfb {
 // (diffusivity in p.nu) and state update, but only the two gradient products i kx C, i ky C leave for K-ROW.
 enum { COL_FWD = 0, COL_INV = 1, COL_STEP = 2, COL_PRO = 3, COL_DIAG = 4, COL_FWDT = 5, COL_TSTEP = 6, COL_TPRO = 7 };
 
+// Linear terms of the vorticity equation (xfb_set_linear_terms, DESIGN.md section 3): beta-plane, linear drag and
+// hyperviscosity.  Per mode L(k) = -mu - ch (k^2 / k_c^2)^order + i beta kx / k^2 multiplies the stage state inside the
+// dealiasing mask; only the LIN instances of the stepper's K-COL and gen_stage read these fields.
+struct LinCoef {
+    float beta, mu;
+    float ch;             // nu_h * k_c^(2 order), formed in float64 on the host (k_c^2 = kx(nx/2)^2 + ky(ny/2)^2)
+    float inv_kc2;        // 1 / k_c^2: (k^2 / k_c^2) <= 1 on the grid, so no power of it overflows
+    int order;            // 1..8
+    int on;               // non-zero: some term is non-zero and the stepper runs the LIN instances
+};
+
+// L(k) z for one mode: kx the signed x wavenumber, k2 = kx^2 + ky^2 (0 only at (0,0), where kx = 0 and the beta term
+// vanishes through the fmaxf guard)
+__device__ __forceinline__ cpx lin_term(const LinCoef &L, const float kx, const float k2, const cpx z)
+{
+    const float b = __fdividef(L.beta * kx, fmaxf(k2, 1.17549435e-38f));
+    // (k^2 / k_c^2)^order as a uniform loop: the fewest live registers of the forms tried (binary powering with selects or
+    // predicated multiplies spilled more in the 8192 K-COL)
+    const float x = k2 * L.inv_kc2;
+    float xp = x;
+#pragma unroll 1
+    for (int o = 1; o < L.order; ++o) xp *= x;
+    const float a = fmaf(-L.ch, xp, -L.mu);
+    return mk(a * z.x - b * z.y, a * z.y + b * z.x);
+}
+
 struct ColParams {
     const cpx *jint;      // FWD/STEP: y-transformed lines, pair layout (see xfb_row.cuh): (i, j) at ((i>>1)*pitch + j)*2 + (i&1)
     cpx *z0;              // spectral state at the start of the step (FWD writes it)
@@ -59,6 +85,7 @@ struct ColParams {
     // at the block of this launch's chunk), so the exchange has no self-copy to do; self_pieces == 0: everything to t_out
     int self_piece0, self_pieces;
     cpx *self_out[4];
+    LinCoef lin;          // COL_STEP: the linear terms (lin.on selects the LIN instances)
 };
 
 template <int NX, int W>

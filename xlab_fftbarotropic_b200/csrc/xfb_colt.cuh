@@ -135,11 +135,13 @@ struct ColtRing {
     }
 };
 
-template <int NX, int MODE_>
+// LIN: COL_STEP with the linear terms of p.lin in the epilogue (a separate instance: the default one keeps its registers)
+template <int NX, int MODE_, bool LIN = false>
 __global__ void __launch_bounds__(ColTCfg<NX>::THREADS, ColTCfg<NX>::MINB)
 colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int tiles_per_member, const int tiles_total)
 {
     typedef ColTCfg<NX> C;
+    static_assert(!LIN || MODE_ == COL_STEP, "the linear terms act on the vorticity step only");
     // the tracer modes are the stepper's modes with two products instead of four
     constexpr bool TRACER = (MODE_ == COL_TSTEP || MODE_ == COL_TPRO);
     constexpr int MODE = (MODE_ == COL_TSTEP) ? COL_STEP : (MODE_ == COL_TPRO) ? COL_PRO : MODE_;
@@ -335,8 +337,13 @@ colt_kernel(const ColParams p, const __grid_constant__ ColTMaps maps, const int 
                         const float kxv = (float)signed_row<NX, SPLIT>(t[0], k) * p.kxscale;
                         const float lap = -fmaf(kxv, kxv, ky2);
                         // dvortdt_c += (vort_c * laplacian_coe) * NU                                  main.cpp:240-243
-                        const float tx = __fadd_rn(X.x, __fmul_rn(__fmul_rn(qzk[q].x, lap), p.nu));
-                        const float ty2 = __fadd_rn(X.y, __fmul_rn(__fmul_rn(qzk[q].y, lap), p.nu));
+                        float tx = __fadd_rn(X.x, __fmul_rn(__fmul_rn(qzk[q].x, lap), p.nu));
+                        float ty2 = __fadd_rn(X.y, __fmul_rn(__fmul_rn(qzk[q].y, lap), p.nu));
+                        if constexpr (LIN) {                                 // + L(k) Z_k (DESIGN.md section 3)
+                            const cpx l = lin_term(p.lin, kxv, -lap, qzk[q]);
+                            tx = __fadd_rn(tx, l.x);
+                            ty2 = __fadd_rn(ty2, l.y);
+                        }
                         // dealiasing mask (fftwfop.cpp:57-68)
                         const int ii = (i <= NX / 2) ? i : NX - i;
                         const float m = (ii * ii + j * j >= p.mask_kd_i) ? 0.0f : 1.0f;

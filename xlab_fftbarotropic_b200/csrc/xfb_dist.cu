@@ -998,6 +998,15 @@ extern "C" int xfb_loopback_set_tracer(xfb_loopback_s *L, const float *tracer_fu
     return 0;
 }
 
+// the same linear terms on every rank of the team (xfb_set_linear_terms is per rank and needs no communication)
+extern "C" int xfb_loopback_set_linear_terms(xfb_loopback_s *L, float beta, float mu, float nu_h, int order)
+{
+    if (!L) return fail(XFB_E_ARG, "null argument");
+    for (int r = 0; r < L->team.nranks; ++r)
+        if (int e = xfb_set_linear_terms(L->team.local[r], beta, mu, nu_h, order)) return e;
+    return 0;
+}
+
 extern "C" int xfb_loopback_step(xfb_loopback_s *L, int nsteps, float dt)
 {
     if (!L) return fail(XFB_E_ARG, "null argument");

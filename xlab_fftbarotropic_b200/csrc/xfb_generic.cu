@@ -167,16 +167,24 @@ __global__ void gen_jacobian(const float *mu, const float *zx, const float *v, c
 }
 
 // rk = mask * (T + nu * lap * Z_k); RK bookkeeping exactly as the fused epilogue (xfb_colt.cuh)   main.cpp:240-251,296-312
+// LIN: + L(k) Z_k inside the mask (xfb_set_linear_terms; kx from the gradx table, k^2 = -lap)
+template <bool LIN>
 __global__ void gen_stage(const cpx *T, cpx *z0, cpx *zk, cpx *acc, const int nx, const int hy, const double *kx2, const double *ky2,
-                          const double mask_kd, const float nu, const float dt, const float dt_stage, const int stage)
+                          const double mask_kd, const float nu, const float dt, const float dt_stage, const int stage,
+                          const float *kx, const LinCoef lin)
 {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (long long)nx * hy) return;
     const int i = (int)(idx / hy), j = (int)(idx % hy);
     const cpx zkv = (stage == 1) ? z0[idx] : zk[idx];
     const float lap = lap_coe(kx2[i], ky2[j]);
-    const float tx = __fadd_rn(T[idx].x, __fmul_rn(__fmul_rn(zkv.x, lap), nu));
-    const float ty = __fadd_rn(T[idx].y, __fmul_rn(__fmul_rn(zkv.y, lap), nu));
+    float tx = __fadd_rn(T[idx].x, __fmul_rn(__fmul_rn(zkv.x, lap), nu));
+    float ty = __fadd_rn(T[idx].y, __fmul_rn(__fmul_rn(zkv.y, lap), nu));
+    if constexpr (LIN) {
+        const cpx l = lin_term(lin, kx[i], -lap, zkv);
+        tx = __fadd_rn(tx, l.x);
+        ty = __fadd_rn(ty, l.y);
+    }
     const long long ii = (i <= nx / 2) ? i : nx - i;
     const float m = ((double)(ii * ii + (long long)j * j) >= mask_kd) ? 0.0f : 1.0f;
     const float rx = __fmul_rn(tx, m), ry = __fmul_rn(ty, m);
@@ -319,8 +327,12 @@ static int generic_one_step(xfb_handle h, float dt)
             if (launch_pw(h, OP_GRADX, psi, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fd, scale, 0)) return XFB_E_CUDA;     // :212-214
             GLAUNCH(h, (gen_jacobian<<<gb, 256, 0, h->stream>>>(fc, fa, fd, fb, src, fa, n)));                                  // :225-227
             if (generic_fwd2d(h, fa, tmp2, T)) return XFB_E_CUDA;                                                                // :237
-            GLAUNCH(h, (gen_stage<<<hb, 256, 0, h->stream>>>(T, z0, zk, acc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd, h->nu, dt,
-                                                              (k == 3) ? dt : dt / 2.0f, k)));
+            if (h->lin.on)
+                GLAUNCH(h, (gen_stage<true><<<hb, 256, 0, h->stream>>>(T, z0, zk, acc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd, h->nu,
+                                                                        dt, (k == 3) ? dt : dt / 2.0f, k, h->kx, h->lin)));
+            else
+                GLAUNCH(h, (gen_stage<false><<<hb, 256, 0, h->stream>>>(T, z0, zk, acc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd, h->nu,
+                                                                         dt, (k == 3) ? dt : dt / 2.0f, k, h->kx, h->lin)));
             if (h->has_tracer) {
                 // passive tracer (xfb_set_tracer): the same loops with c for vort and kappa for NU; -u, v of this
                 // stage are still in fc, fd
@@ -330,8 +342,8 @@ static int generic_one_step(xfb_handle h, float dt)
                 if (launch_pw(h, OP_GRADY, c, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fb, scale, 0)) return XFB_E_CUDA;
                 GLAUNCH(h, (gen_jacobian<<<gb, 256, 0, h->stream>>>(fc, fa, fd, fb, nullptr, fa, n)));
                 if (generic_fwd2d(h, fa, tmp2, h->cjint)) return XFB_E_CUDA;
-                GLAUNCH(h, (gen_stage<<<hb, 256, 0, h->stream>>>(h->cjint, c0, ck, cacc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd,
-                                                                  h->kappa, dt, (k == 3) ? dt : dt / 2.0f, k)));
+                GLAUNCH(h, (gen_stage<false><<<hb, 256, 0, h->stream>>>(h->cjint, c0, ck, cacc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd,
+                                                                         h->kappa, dt, (k == 3) ? dt : dt / 2.0f, k, h->kx, LinCoef())));
             }
         }
     }
@@ -341,7 +353,7 @@ static int generic_one_step(xfb_handle h, float dt)
 // nsteps RK4 steps.  A step is 72 short launches per member (124 with the tracer) on grids that live in L2 -- launch
 // gaps, not kernels, bound it --, so like the fused stepper (xfb_step) the step is captured once into a CUDA graph and
 // replayed; the first step of a handle runs eagerly, XFB_NO_GRAPH=1 keeps the eager path.  The graph bakes in dt, the
-// source pointer and the tracer's state (xfb_set_tracer drops it).
+// source pointer, the tracer's state (xfb_set_tracer drops it) and the linear terms (xfb_set_linear_terms drops it).
 int generic_step(xfb_handle h, int nsteps, float dt)
 {
     static const bool no_graph = getenv("XFB_NO_GRAPH") && atoi(getenv("XFB_NO_GRAPH")) != 0;

@@ -72,6 +72,7 @@ struct xfb_handle_s {
     xfb::cpx *c0, *ck, *cacc, *cjint, *tc[2];
     float kappa;
     bool has_tracer, tcf_valid;     // tcf_valid: tc[0..1] hold the gradient products of the current c0
+    xfb::LinCoef lin;    // beta-plane, linear drag, hyperviscosity (xfb_set_linear_terms); all zero: off
     void *generic;       // non-null: grid served by the generic mixed-radix path (xfb_generic.cu), reference layout everywhere
     // ---- slab decomposition (xfb_dist.cu); nranks == 1 otherwise ------------------------------------
     // rank r holds physical rows [r*rows, (r+1)*rows) and the spectral columns of panels r*nchunks ..
