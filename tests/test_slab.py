@@ -35,6 +35,25 @@ def test_partition_covers_grid(n, p, c):
     assert parts[0]["pitch_global"] - (n // 2 + 1) < 4 * p * c + 4, "padding stays small"
 
 
+@pytest.mark.parametrize("nx,ny,p,c", [(512, 2048, 4, 2), (2048, 256, 2, 4), (256, 1024, 8, 1), (16384, 1024, 8, 4),
+                                       (16384, 256, 8, 8), (256, 16384, 2, 16)])
+def test_partition_covers_rectangular_grid(nx, ny, p, c):
+    """rows come from nx, columns (of the ny / 2 + 1 wide half spectrum) from ny"""
+    import xlab_fftbarotropic_b200 as xfb
+    parts = [xfb.slab_partition(nx, ny, p, c, r) for r in range(p)]
+    assert sum(q["rows"] for q in parts) == nx
+    assert [q["row0"] for q in parts] == [r * (nx // p) for r in range(p)]
+    assert all(q["rows"] % (2 * c) == 0 for q in parts)
+    cw = parts[0]["chunk_cols"]
+    assert cw % 4 == 0 and all(q["chunk_cols"] == cw and q["cols"] == c * cw for q in parts)
+    assert [q["col0"] for q in parts] == [r * c * cw for r in range(p)]
+    assert parts[0]["pitch_global"] == p * c * cw >= ny // 2 + 1
+    assert parts[0]["pitch_global"] - (ny // 2 + 1) < 4 * p * c + 4
+    # the transposed grid splits its own rows and columns
+    t = xfb.slab_partition(ny, nx, p, c, 0)
+    assert t["rows"] == ny // p and t["pitch_global"] >= nx // 2 + 1
+
+
 def test_partition_rejects_bad_arguments():
     import xlab_fftbarotropic_b200 as xfb
     with pytest.raises(xfb.XfbError):

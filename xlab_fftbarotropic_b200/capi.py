@@ -326,15 +326,18 @@ class SlabBackend(Backend):
     """One rank of a slab-decomposed grid (one process per GPU, NCCL all-to-all).  Fields are the LOCAL rows."""
 
     def __init__(self, n: int, rank: int, nranks: int, unique_id: bytes, nchunks: int = 8, lx: float = 600000.0,
-                 nu: float = 6.5, device: int = 0):
-        self.nx, self.ny, self.hy, self.batch = n, n, n // 2 + 1, 1
-        self.lx, self.ly, self.nu = lx, lx, nu
+                 nu: float = 6.5, device: int = 0, ny: int | None = None, ly: float | None = None):
+        """n x ny grid (ny = n by default) on an lx x ly domain (ly = lx by default); n rows are split over the ranks"""
+        ny = n if ny is None else ny
+        ly = lx if ly is None else ly
+        self.nx, self.ny, self.hy, self.batch = n, ny, ny // 2 + 1, 1
+        self.lx, self.ly, self.nu = lx, ly, nu
         self.rank, self.nranks = rank, nranks
-        self.part = slab_partition(n, n, nranks, nchunks, rank) if nranks > 1 else dict(row0=0, rows=n)
+        self.part = slab_partition(n, ny, nranks, nchunks, rank) if nranks > 1 else dict(row0=0, rows=n)
         self.rows = self.part["rows"]
         self._L = load()
         self._h = C.c_void_p()
-        self._ck(self._L.xfb_create_dist(C.byref(self._h), n, n, lx, lx, nu, device, rank, nranks, nchunks, unique_id))
+        self._ck(self._L.xfb_create_dist(C.byref(self._h), n, ny, lx, ly, nu, device, rank, nranks, nchunks, unique_id))
 
     def set_vorticity(self, f, member=0):
         if not isinstance(f, (int, np.integer)):
@@ -380,11 +383,15 @@ class LoopbackTeam:
     """All ranks of a slab decomposition in one process on one device (verification of the slab indexing
     on a single GPU; same kernels as the NCCL path, the exchange is a set of device copies)."""
 
-    def __init__(self, n: int, nranks: int, nchunks: int = 1, lx: float = 600000.0, nu: float = 6.5, device: int = 0):
-        self.n, self.lx = n, lx
+    def __init__(self, n: int, nranks: int, nchunks: int = 1, lx: float = 600000.0, nu: float = 6.5, device: int = 0,
+                 ny: int | None = None, ly: float | None = None):
+        """n x ny grid (ny = n by default) on an lx x ly domain (ly = lx by default); n rows are split over the ranks"""
+        ny = n if ny is None else ny
+        ly = lx if ly is None else ly
+        self.nx, self.ny, self.lx, self.ly = n, ny, lx, ly
         self._L = load()
         self._t = C.c_void_p()
-        self._ck(self._L.xfb_loopback_create(C.byref(self._t), n, n, lx, lx, nu, device, nranks, nchunks))
+        self._ck(self._L.xfb_loopback_create(C.byref(self._t), n, ny, lx, ly, nu, device, nranks, nchunks))
 
     def _ck(self, rc):
         if rc != 0:
@@ -402,18 +409,18 @@ class LoopbackTeam:
             pass
 
     def set_vorticity(self, f):
-        f = np.ascontiguousarray(f, dtype=np.float32).reshape(self.n, self.n)
+        f = np.ascontiguousarray(f, dtype=np.float32).reshape(self.nx, self.ny)
         self._ck(self._L.xfb_loopback_set_vorticity(self._t, _ptr(f)))
 
     def set_source(self, s):
         if s is None:
             self._ck(self._L.xfb_loopback_set_source(self._t, None))
         else:
-            s = np.ascontiguousarray(s, dtype=np.float32).reshape(self.n, self.n)
+            s = np.ascontiguousarray(s, dtype=np.float32).reshape(self.nx, self.ny)
             self._ck(self._L.xfb_loopback_set_source(self._t, _ptr(s)))
 
     def set_tracer(self, c, kappa):
-        c = np.ascontiguousarray(c, dtype=np.float32).reshape(self.n, self.n)
+        c = np.ascontiguousarray(c, dtype=np.float32).reshape(self.nx, self.ny)
         self._ck(self._L.xfb_loopback_set_tracer(self._t, _ptr(c), float(kappa)))
 
     def set_linear_terms(self, beta=0.0, mu=0.0, nu_h=0.0, order=4):
@@ -424,13 +431,13 @@ class LoopbackTeam:
         self._ck(self._L.xfb_loopback_step(self._t, int(nsteps), float(dt)))
 
     def get_field(self, which):
-        out = np.empty((self.n, self.n), np.float32)
+        out = np.empty((self.nx, self.ny), np.float32)
         self._ck(self._L.xfb_loopback_get_field(self._t, which, _ptr(out)))
         return out
 
     def diagnostics(self):
-        t = np.empty((self.n, self.n), np.float32)
-        d = np.empty((self.n, self.n), np.float32)
+        t = np.empty((self.nx, self.ny), np.float32)
+        d = np.empty((self.nx, self.ny), np.float32)
         self._ck(self._L.xfb_loopback_get_diagnostics(self._t, _ptr(t), _ptr(d)))
         return t, d
 
@@ -443,7 +450,7 @@ class LoopbackTeam:
     def energy_spectrum(self, nshells=None, which=VORT):
         """whole-domain (totals, e, z) as Backend.energy_spectrum"""
         return _energy_spectrum(self._L, lambda t, e, z, n: self._L.xfb_loopback_get_energy_spectrum(self._t, which, n, t, e, z),
-                                nshells, self.n, self.n, self.lx, self.lx)
+                                nshells, self.nx, self.ny, self.lx, self.ly)
 
     @property
     def launch_count(self):
