@@ -83,3 +83,26 @@ def test_source_and_pressure_on_768(xfb, orc):
     po = o.invert_pres(psi, 3, 5, 1.0, 1e-5)
     assert rel_l2(pb, po) < 1e-4
     b.close()
+
+
+def test_field_ids_outside_the_header_are_rejected(xfb):
+    """xfb_get_field / xfb_get_field_async take the field ids of include/xfb.h only: any other id fails with "bad field
+    id" on the unfused record path (generic grids), whatever chains the library keeps for its own use.  Both entry points
+    report a failure of the field computation as XFB_E_CUDA, the code they have always returned for it."""
+    import ctypes as C
+    n = 96
+    b = xfb.Backend(n)
+    b.set_vorticity(fields.elliptic(n))
+    L = b._L
+    out = np.empty((n, n), np.float32)
+    p = C.c_void_p()
+    assert L.xfb_host_alloc(C.byref(p), n * n) == 0
+    t = C.c_int()
+    for which in (-1, 10, 11, 12, 13, 42):
+        assert L.xfb_get_field(b._h, 0, which, out.ctypes.data_as(C.c_void_p)) == -3, which
+        assert b"bad field id" in L.xfb_last_error()
+        assert L.xfb_get_field_async(b._h, 0, which, p, C.byref(t)) == -3, which
+        assert b"bad field id" in L.xfb_last_error()
+    assert np.isfinite(b.get_field(xfb.capi.DEFORM)).all()          # the handle is still usable
+    L.xfb_host_free(p)
+    b.close()

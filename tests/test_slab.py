@@ -241,6 +241,20 @@ def test_loopback_diagnostics_and_keff_histograms():
 
 
 @pytest.mark.gpu
+def test_loopback_rejects_field_ids_outside_the_header():
+    """xfb_loopback_get_field takes the field ids of include/xfb.h only (XFB_SRC is not a team field): XFB_E_ARG"""
+    import xlab_fftbarotropic_b200 as xfb
+    n = 256
+    team = xfb.LoopbackTeam(n, 2)
+    team.set_vorticity(fields.elliptic(n))
+    for which in (-1, xfb.capi.SRC, 10, 11, 12, 13):
+        with pytest.raises(xfb.XfbError, match="error -1: bad field id"):
+            team.get_field(which)
+    assert np.isfinite(team.get_field(xfb.capi.TFIL)).all()
+    team.close()
+
+
+@pytest.mark.gpu
 def test_loopback_16384_two_level_kernels():
     """the slab path at the grid bench.py measures (BASELINE.json configs[4]): two-level K-ROW fed by one bulk copy per
     panel, two-level K-COL storing this rank's own row pairs straight into its receive arrays (no self-copy in the

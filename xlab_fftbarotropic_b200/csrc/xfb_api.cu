@@ -315,6 +315,13 @@ extern "C" int xfb_create(xfb_handle *out, int nx, int ny, float lx, float ly, f
     return create_impl(out, nx, ny, lx, ly, nu, batch, device, 0, 1, 1);
 }
 
+// the captured step bakes in dt, the source pointer, the tracer and the linear terms: a change of the last two drops it
+static void drop_step_graph(xfb_handle h)
+{
+    if (h->step_graph) cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph);
+    h->step_graph = nullptr;
+}
+
 int xfb::destroy_impl(xfb_handle h)
 {
     if (!h) return 0;
@@ -322,7 +329,7 @@ int xfb::destroy_impl(xfb_handle h)
     cudaStreamSynchronize(h->stream);
     if (h->comm_stream) cudaStreamSynchronize(h->comm_stream);
     generic_destroy(h);
-    if (h->step_graph) cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph);
+    drop_step_graph(h);
     if (h->rec_stream) {
         cudaStreamSynchronize(h->rec_stream);
         for (int i = 0; i < XFB_NREC; ++i) {
@@ -412,7 +419,7 @@ extern "C" void *xfb_stream(xfb_handle h) { return h ? (void *)h->stream : nullp
 // ------------------------------------------------------------------------------------------------
 // staging helpers: bring a caller buffer to the device / back
 // ------------------------------------------------------------------------------------------------
-static int stage_in(xfb_handle h, const void *user, void *dev_scratch, size_t bytes, const void **dev)
+int xfb::stage_in(xfb_handle h, const void *user, void *dev_scratch, size_t bytes, const void **dev)
 {
     if (is_device_ptr(user)) { *dev = user; return 0; }
     CK(cudaMemcpyAsync(dev_scratch, user, bytes, cudaMemcpyHostToDevice, h->stream));
@@ -420,14 +427,13 @@ static int stage_in(xfb_handle h, const void *user, void *dev_scratch, size_t by
     return 0;
 }
 
-// returns the device buffer the result should be produced in
-static void *stage_out_target(const void *user, void *dev_scratch) { return is_device_ptr(user) ? (void *)user : dev_scratch; }
+void *xfb::stage_out_target(const void *user, void *dev_scratch) { return is_device_ptr(user) ? (void *)user : dev_scratch; }
 
-static int stage_out(xfb_handle h, void *user, const void *dev, size_t bytes)
+int xfb::stage_out(xfb_handle h, void *user, const void *dev, size_t bytes, bool wait)
 {
     if ((const void *)user != dev) {
         CK(cudaMemcpyAsync(user, dev, bytes, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
+        if (wait) CK(cudaStreamSynchronize(h->stream));
     }
     return 0;
 }
@@ -651,6 +657,23 @@ extern "C" int xfb_set_source(xfb_handle h, int member, const float *src)
     return 0;
 }
 
+int xfb::tracer_state_alloc(xfb_handle h)
+{
+    if (h->c0) return 0;
+    const size_t sb = sizeof(cpx) * h->hpad * h->batch;
+    cpx **state[] = {&h->c0, &h->ck, &h->cacc, &h->cjint};
+    for (auto pp : state) {
+        if (dev_alloc((void **)pp, sb)) return XFB_E_CUDA;
+        CK(cudaMemsetAsync(*pp, 0, sb, h->stream));
+    }
+    if (!h->generic) {
+        if (dev_alloc((void **)&h->tc[0], 2 * sb)) return XFB_E_CUDA;
+        CK(cudaMemsetAsync(h->tc[0], 0, 2 * sb, h->stream));
+        h->tc[1] = h->tc[0] + h->hpad * h->batch;
+    }
+    return 0;
+}
+
 // Passive tracer (SURVEY.md section 8 (f-4)): dc/dt = -u c_x - v c_y + kappa lap(c), advanced inside xfb_step by the
 // velocity of the same Runge-Kutta stage with the vorticity equation's own operation order (dealiased tendency, same
 // evolve / final combine).  The reference has no tracer; the definition is the oracle's (barotropic_oracle.c
@@ -663,19 +686,7 @@ extern "C" int xfb_set_tracer(xfb_handle h, int member, const float *tracer, flo
     if (!fused_diag_ok(h) && !h->generic && h->nranks == 1 && h->nx != 16384)
         return fail(XFB_E_SIZE, "the passive tracer needs the fused kernels (power-of-two grids), a generic mixed-radix grid, or a slab-decomposed handle");
     CK(cudaSetDevice(h->device));
-    const size_t sb = sizeof(cpx) * h->hpad * h->batch;
-    if (!h->c0) {
-        cpx **state[] = {&h->c0, &h->ck, &h->cacc, &h->cjint};
-        for (auto pp : state) {
-            if (dev_alloc((void **)pp, sb)) return XFB_E_CUDA;
-            CK(cudaMemsetAsync(*pp, 0, sb, h->stream));
-        }
-        if (!h->generic) {
-            if (dev_alloc((void **)&h->tc[0], 2 * sb)) return XFB_E_CUDA;
-            CK(cudaMemsetAsync(h->tc[0], 0, 2 * sb, h->stream));
-            h->tc[1] = h->tc[0] + h->hpad * h->batch;
-        }
-    }
+    if (tracer_state_alloc(h)) return XFB_E_CUDA;
     const void *din;
     if (stage_in(h, tracer, h->real_a, sizeof(float) * h->grids, &din)) return XFB_E_CUDA;
     if (h->nranks > 1) {
@@ -692,10 +703,7 @@ extern "C" int xfb_set_tracer(xfb_handle h, int member, const float *tracer, flo
         if (launch_pw(h, OP_COPY, h->spec_b, h->pitch, h->c0 + (size_t)member * h->hpad, h->pitch, h->pitch, 0, h->tw_state))
             return XFB_E_CUDA;
     }
-    if (!h->has_tracer || h->kappa != kappa) {
-        // the captured step has no tracer launches / another diffusivity baked in
-        if (h->step_graph) { cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph); h->step_graph = nullptr; }
-    }
+    if (!h->has_tracer || h->kappa != kappa) drop_step_graph(h);     // it has no tracer launches / another diffusivity baked in
     h->has_tracer = true;
     h->kappa = kappa;
     h->tcf_valid = false;
@@ -731,11 +739,8 @@ extern "C" int xfb_set_linear_terms(xfb_handle h, float beta, float mu, float nu
     }
     if (memcmp(&L, &h->lin, sizeof(L)) != 0) {
         // the captured step (fused or generic path) has the old coefficients baked in
-        if (h->step_graph) {
-            CK(cudaSetDevice(h->device));
-            cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph);
-            h->step_graph = nullptr;
-        }
+        if (h->step_graph) CK(cudaSetDevice(h->device));
+        drop_step_graph(h);
         h->lin = L;
     }
     return 0;
@@ -748,7 +753,7 @@ extern "C" int xfb_step(xfb_handle h, int nsteps, float dt)
     if (!h->have_state) return fail(XFB_E_STATE, "xfb_step before xfb_set_vorticity");
     CK(cudaSetDevice(h->device));
     if (h->nranks > 1) return dist_step(h, nsteps, dt);
-    if (h->generic) return generic_step(h, nsteps, dt);
+    if (h->generic) return step_replay(h, nsteps, dt, false, [&]() { return generic_one_step(h, dt); });
     ColParams c; fill_col(h, c);
     c.jint = h->jint; c.z0 = h->z0; c.zk = h->zk; c.acc = h->acc;
     c.st_tile_stride = (long long)h->nx * h->tw_state; c.st_row_stride = h->tw_state;     // tile-major state
@@ -776,8 +781,7 @@ extern "C" int xfb_step(xfb_handle h, int nsteps, float dt)
             h->tcf_valid = true;
         }
     }
-    const int launches_per_step = tracer ? 16 : 8;
-    auto one_step = [&]() -> int {
+    return step_replay(h, nsteps, dt, true, [&]() -> int {
         for (int k = 1; k <= 4; ++k) {
             if (h->profiling) cudaEventRecord(next_event(h->ev_row, h->ev_row_used), h->stream);
             CKL(h, launch_row(h->ny, ROW_JAC, r, h->stream));
@@ -796,26 +800,34 @@ extern "C" int xfb_step(xfb_handle h, int nsteps, float dt)
             if (h->profiling) cudaEventRecord(next_event(h->ev_col, h->ev_col_used), h->stream);
         }
         return 0;
-    };
-    // The eight launches of a step are captured once into a CUDA graph and replayed: on small grids (one launch is
-    // 15-25 us at 512^2 / 1024^2) the launch gaps are a tenth of the step.  The first step of a handle runs eagerly
-    // (it also configures the kernels), per-kernel profiling and XFB_NO_GRAPH=1 keep the eager path.
+    });
+}
+
+// The launches of a step are captured once into a CUDA graph and replayed: on small grids (one launch is 15-25 us at
+// 512^2 / 1024^2 on the fused path; the generic path issues 72 short launches per member) the launch gaps are a large
+// part of the step.  The first step of a handle runs eagerly (it also configures the kernels); XFB_NO_GRAPH=1, and
+// per-kernel profiling of the fused step (its events), keep the eager path.  The graph is captured again when dt or
+// the source pointer changes; xfb_set_tracer and xfb_set_linear_terms drop it.
+int xfb::step_replay(xfb_handle h, int nsteps, float dt, bool eager_if_profiling, const std::function<int()> &one_step)
+{
     static const bool no_graph = getenv("XFB_NO_GRAPH") && atoi(getenv("XFB_NO_GRAPH")) != 0;
+    const bool eager_all = no_graph || (eager_if_profiling && h->profiling);
     int s = 0;
-    if (nsteps > 0 && (!h->warmed || h->profiling || no_graph)) {
-        const int eager = (h->profiling || no_graph) ? nsteps : 1;
+    if (nsteps > 0 && (!h->warmed || eager_all)) {
+        const int eager = eager_all ? nsteps : 1;
         for (; s < eager; ++s)
             if (int e = one_step()) return e;
         h->warmed = true;
     }
     if (s < nsteps) {
-        const void *src_now = (const void *)r.real_in;
+        const void *src_now = h->has_src ? (const void *)h->src : nullptr;
         if (!h->step_graph || h->graph_dt != dt || h->graph_src != src_now) {
-            if (h->step_graph) { cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph); h->step_graph = nullptr; }
+            drop_step_graph(h);
             cudaGraph_t g = nullptr;
             CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeRelaxed));
             const long long l0 = h->launches;
             const int e = one_step();
+            const int per_step = (int)(h->launches - l0);
             h->launches = l0;
             cudaError_t ce = cudaStreamEndCapture(h->stream, &g);
             if (e) { if (g) cudaGraphDestroy(g); return e; }
@@ -824,14 +836,49 @@ extern "C" int xfb_step(xfb_handle h, int nsteps, float dt)
             ce = cudaGraphInstantiate(&ge, g, 0);
             cudaGraphDestroy(g);
             if (ce != cudaSuccess) return fail(XFB_E_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(ce));
-            h->step_graph = ge; h->graph_dt = dt; h->graph_src = src_now;
+            h->step_graph = ge; h->graph_dt = dt; h->graph_src = src_now; h->graph_launches = per_step;
         }
         for (; s < nsteps; ++s) {
             CK(cudaGraphLaunch((cudaGraphExec_t)h->step_graph, h->stream));
-            h->launches += launches_per_step;
+            h->launches += h->graph_launches;
         }
     }
     return 0;
+}
+
+const FieldOps *xfb::field_ops(int which)
+{
+    static const FieldOps table[] = {
+        {1, {OP_COPY}, 0},                          // XFB_VORT
+        {1, {OP_INVLAP}, 0},                        // XFB_PSI
+        {2, {OP_INVLAP, OP_GRADY}, 1},              // XFB_U = -psi_y
+        {2, {OP_INVLAP, OP_GRADX}, 0},              // XFB_V = psi_x
+        {0}, {0}, {0},                              // XFB_SRC, XFB_TFIL, XFB_DEFORM
+        {1, {OP_GRADX}, 0},                         // XFB_DVORTDX
+        {1, {OP_GRADY}, 0},                         // XFB_DVORTDY
+        {1, {OP_COPY}, 0},                          // XFB_TRACER (of the tracer's state)
+    };
+    static_assert(sizeof(table) / sizeof(table[0]) == XFB_TRACER + 1, "one entry per field id");
+    if (which < 0 || which > XFB_TRACER || table[which].nops == 0) return nullptr;
+    return &table[which];
+}
+
+const FieldOps xfb::psi_second_ops[3] = {
+    {3, {OP_INVLAP, OP_GRADX, OP_GRADY}, 0},    // psi_xy
+    {3, {OP_INVLAP, OP_GRADX, OP_GRADX}, 0},    // psi_xx
+    {3, {OP_INVLAP, OP_GRADY, OP_GRADY}, 0},    // psi_yy
+};
+
+// operator chain `f` of one member's state array z (tile-major, or row-major on generic grids) -> physical field in
+// `dout` (device), reference normalisation; spec_a and spec_b are the scratch
+static int chain_to_device(xfb_handle h, const cpx *z, const FieldOps &f, float *dout)
+{
+    const float scale = 1.0f / (float)((double)h->nx * (double)h->ny);
+    const int P = h->pitch;
+    if (launch_pw(h, f.ops[0], z, P, h->spec_a, P, P, h->tw_state, 0)) return XFB_E_CUDA;
+    for (int o = 1; o < f.nops; ++o)
+        if (launch_pw(h, f.ops[o], h->spec_a, P, h->spec_a, P, P)) return XFB_E_CUDA;
+    return inv2d(h, h->spec_a, h->spec_b, dout, scale, f.negate);
 }
 
 // derived spectral field of member -> physical field in `dout` (device), reference normalisation
@@ -843,7 +890,6 @@ static int derived_field(xfb_handle h, int member, int which, float *dout, const
     }
     const cpx *z = (state ? state : h->z0) + (size_t)member * h->hpad;
     const float scale = 1.0f / (float)((double)h->nx * (double)h->ny);
-    const int P = h->pitch, T = h->tw_state;
     if (fused_diag_ok(h)) {
         // record fields on the stepper's kernels: one K-COL launch (spectral multiplier + x pass, TMA-staged) and one
         // K-ROW launch (y pass, normalisation, sign); multipliers in float32 (<= 2 ulp from the operator tier's tables)
@@ -853,41 +899,9 @@ static int derived_field(xfb_handle h, int member, int which, float *dout, const
         CKL(h, launch_row(h->ny, ROW_C2R, r, h->stream));
         return 0;
     }
-    switch (which) {
-    case XFB_VORT:
-        if (launch_pw(h, OP_COPY, z, P, h->spec_a, P, P, T, 0)) return XFB_E_CUDA;
-        return inv2d(h, h->spec_a, h->spec_b, dout, scale, 0);
-    case XFB_PSI:
-        if (launch_pw(h, OP_INVLAP, z, P, h->spec_a, P, P, T, 0)) return XFB_E_CUDA;
-        return inv2d(h, h->spec_a, h->spec_b, dout, scale, 0);
-    case XFB_U:
-        if (launch_pw(h, OP_INVLAP, z, P, h->spec_a, P, P, T, 0)) return XFB_E_CUDA;
-        if (launch_pw(h, OP_GRADY, h->spec_a, P, h->spec_a, P, P)) return XFB_E_CUDA;
-        return inv2d(h, h->spec_a, h->spec_b, dout, scale, 1);
-    case XFB_V:
-        if (launch_pw(h, OP_INVLAP, z, P, h->spec_a, P, P, T, 0)) return XFB_E_CUDA;
-        if (launch_pw(h, OP_GRADX, h->spec_a, P, h->spec_a, P, P)) return XFB_E_CUDA;
-        return inv2d(h, h->spec_a, h->spec_b, dout, scale, 0);
-    case XFB_DVORTDX:
-        if (launch_pw(h, OP_GRADX, z, P, h->spec_a, P, P, T, 0)) return XFB_E_CUDA;
-        return inv2d(h, h->spec_a, h->spec_b, dout, scale, 0);
-    case XFB_DVORTDY:
-        if (launch_pw(h, OP_GRADY, z, P, h->spec_a, P, P, T, 0)) return XFB_E_CUDA;
-        return inv2d(h, h->spec_a, h->spec_b, dout, scale, 0);
-    }
-    return fail(XFB_E_ARG, "bad field id %d", which);
-}
-
-// second derivatives of psi for the diagnostics: which = 0 psi_xy, 1 psi_xx, 2 psi_yy
-static int psi_second(xfb_handle h, int member, int which, float *dout)
-{
-    const cpx *z = h->z0 + (size_t)member * h->hpad;
-    const float scale = 1.0f / (float)((double)h->nx * (double)h->ny);
-    const int P = h->pitch;
-    if (launch_pw(h, OP_INVLAP, z, P, h->spec_a, P, P, h->tw_state, 0)) return XFB_E_CUDA;
-    if (launch_pw(h, which == 2 ? OP_GRADY : OP_GRADX, h->spec_a, P, h->spec_a, P, P)) return XFB_E_CUDA;
-    if (launch_pw(h, which == 1 ? OP_GRADX : OP_GRADY, h->spec_a, P, h->spec_a, P, P)) return XFB_E_CUDA;
-    return inv2d(h, h->spec_a, h->spec_b, dout, scale, 0);
+    const FieldOps *f = field_ops(which);
+    if (!f) return fail(XFB_E_ARG, "bad field id %d", which);
+    return chain_to_device(h, z, *f, dout);
 }
 
 // filamentation time and deformation factor from psi_xy, psi_xx, psi_yy
@@ -902,6 +916,31 @@ __global__ void diag_kernel(const float *pxy, const float *pxx, const float *pyy
     else out[i] = (den > 0.0f) ? __fdiv_rn(q, den) : 0.0f;
 }
 
+int xfb::launch_strain(xfb_handle h, const float *pxy, const float *pxx, const float *pyy, float *out, long long n, int which)
+{
+    diag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(pxy, pxx, pyy, out, n, which);
+    CK(cudaGetLastError());
+    h->launches++;
+    return 0;
+}
+
+// Both strain diagnostics of member from ONE set of the three second derivatives of psi, into device buffers; either
+// may be null.  Filamentation time (Rozoff et al. 2006) and deformation factor, README.md:5,7.  The fused pair writes
+// both outputs, so a missing one goes to scratch.  Otherwise psi_xy -> real_b, psi_xx -> real_c, psi_yy -> real_a; an
+// output may be real_a only when it is the sole output (the strain kernel then runs in place).
+static int strain_to_device(xfb_handle h, int member, float *tfil, float *deform)
+{
+    if (fused_diag_ok(h)) return fused_diag(h, member, 0, tfil ? tfil : h->real_c, deform ? deform : h->real_b);
+    const cpx *z = h->z0 + (size_t)member * h->hpad;
+    if (chain_to_device(h, z, psi_second_ops[0], h->real_b) || chain_to_device(h, z, psi_second_ops[1], h->real_c) ||
+        chain_to_device(h, z, psi_second_ops[2], h->real_a))
+        return XFB_E_CUDA;
+    const long long n = (long long)h->grids;
+    if (tfil && launch_strain(h, h->real_b, h->real_c, h->real_a, tfil, n, XFB_TFIL)) return XFB_E_CUDA;
+    if (deform && launch_strain(h, h->real_b, h->real_c, h->real_a, deform, n, XFB_DEFORM)) return XFB_E_CUDA;
+    return 0;
+}
+
 // field `which` of member into the DEVICE buffer dout (grids floats), on the handle's stream
 static int field_to_device(xfb_handle h, int member, int which, float *dout)
 {
@@ -911,19 +950,8 @@ static int field_to_device(xfb_handle h, int member, int which, float *dout)
         CK(cudaMemcpyAsync(dout, h->src + (size_t)member * h->grids, bytes, cudaMemcpyDeviceToDevice, h->stream));
         return 0;
     }
-    if ((which == XFB_TFIL || which == XFB_DEFORM) && fused_diag_ok(h))
-        return fused_diag(h, member, 0, which == XFB_TFIL ? dout : h->real_c, which == XFB_DEFORM ? dout : h->real_b);   // dout may be real_a
-    if (which == XFB_TFIL || which == XFB_DEFORM) {
-        if (psi_second(h, member, 0, h->real_b)) return XFB_E_CUDA;
-        if (psi_second(h, member, 1, h->real_c)) return XFB_E_CUDA;
-        float *pyy = dout;   // psi_yy lands in the output buffer, then is overwritten in place
-        if (psi_second(h, member, 2, pyy)) return XFB_E_CUDA;
-        const long long n = (long long)h->grids;
-        diag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->real_b, h->real_c, pyy, dout, n, which);
-        CK(cudaGetLastError());
-        h->launches++;
-        return 0;
-    }
+    if (which == XFB_TFIL || which == XFB_DEFORM)      // dout may be real_a
+        return strain_to_device(h, member, which == XFB_TFIL ? dout : nullptr, which == XFB_DEFORM ? dout : nullptr);
     return derived_field(h, member, which, dout);
 }
 
@@ -1037,9 +1065,8 @@ static int fused_diag(xfb_handle h, int member, int kind, float *out0, float *ou
     return 0;
 }
 
-// Both strain diagnostics of one member from ONE set of the three second derivatives of psi (xfb_get_field recomputes
-// them per field): filamentation time (Rozoff et al. 2006) and deformation factor, README.md:5,7.  Either output may
-// be NULL.  Host or device pointers.
+// both strain diagnostics of one member (xfb_get_field recomputes the second derivatives of psi per field); either
+// output may be NULL.  Host or device pointers.
 extern "C" int xfb_get_diagnostics(xfb_handle h, int member, float *tfil, float *deform)
 {
     if (check_member(h, member)) return XFB_E_ARG;
@@ -1048,34 +1075,13 @@ extern "C" int xfb_get_diagnostics(xfb_handle h, int member, float *tfil, float 
     CK(cudaSetDevice(h->device));
     if (h->nranks > 1) return dist_diagnostics(h, tfil, deform);          // local rows; collective
     const size_t bytes = sizeof(float) * h->grids;
-    const long long n = (long long)h->grids;
-    if (fused_diag_ok(h)) {
-        float *d0 = (tfil && is_device_ptr(tfil)) ? tfil : h->real_a, *d1 = (deform && is_device_ptr(deform)) ? deform : h->real_b;
-        if (fused_diag(h, member, 0, d0, d1)) return XFB_E_CUDA;
-        if (tfil && d0 != tfil) CK(cudaMemcpyAsync(tfil, d0, bytes, cudaMemcpyDeviceToHost, h->stream));
-        if (deform && d1 != deform) CK(cudaMemcpyAsync(deform, d1, bytes, cudaMemcpyDeviceToHost, h->stream));
-        if ((tfil && d0 != tfil) || (deform && d1 != deform)) CK(cudaStreamSynchronize(h->stream));
-        return 0;
-    }
-    // psi_xy -> real_b, psi_xx -> real_c, psi_yy -> real_a; each result is produced in the caller's buffer when that
-    // is device memory, else in a transform scratch array that is free by then (the input pointers are read before
-    // the output element is written, so diag_kernel may run in place)
-    if (psi_second(h, member, 0, h->real_b) || psi_second(h, member, 1, h->real_c) || psi_second(h, member, 2, h->real_a))
-        return XFB_E_CUDA;
-    float *outs[2] = {tfil, deform};
-    const int which[2] = {XFB_TFIL, XFB_DEFORM};
-    float *scratch = (float *)h->ref_a;          // 2*hgrids floats >= grids floats
-    for (int o = 0; o < 2; ++o) {
-        if (!outs[o]) continue;
-        float *d = is_device_ptr(outs[o]) ? outs[o] : scratch;
-        diag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->real_b, h->real_c, h->real_a, d, n, which[o]);
-        CK(cudaGetLastError());
-        h->launches++;
-        if (d != outs[o]) {
-            CK(cudaMemcpyAsync(outs[o], d, bytes, cudaMemcpyDeviceToHost, h->stream));
-            CK(cudaStreamSynchronize(h->stream));
-        }
-    }
+    // host outputs are produced in the reference-layout scratch arrays (2 * hgrids floats >= grids floats)
+    float *dt = tfil ? (float *)stage_out_target(tfil, h->ref_a) : nullptr;
+    float *dd = deform ? (float *)stage_out_target(deform, h->ref_b) : nullptr;
+    if (strain_to_device(h, member, dt, dd)) return XFB_E_CUDA;
+    if (tfil && stage_out(h, tfil, dt, bytes, false)) return XFB_E_CUDA;
+    if (deform && stage_out(h, deform, dd, bytes, false)) return XFB_E_CUDA;
+    if (dt != tfil || dd != deform) CK(cudaStreamSynchronize(h->stream));      // one wait for the host copies
     return 0;
 }
 
@@ -1126,11 +1132,25 @@ int xfb::launch_keff_hist(xfb_handle h, const float *c, const float *gx, const f
     return 0;
 }
 
+int xfb::keff_hist_args(int nbins, float cmin, float cmax, const double *area, const double *grad2)
+{
+    if (!area || !grad2 || nbins < 1 || nbins > 2048 || !(cmax > cmin)) return fail(XFB_E_ARG, "bad histogram arguments");
+    return 0;
+}
+
+int xfb::keff_hist_finish(xfb_handle h, const double *d, int nbins, double *area, double *grad2)
+{
+    std::vector<double> host(2 * (size_t)nbins);
+    CK(cudaMemcpyAsync(host.data(), d, sizeof(double) * 2 * nbins, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    memcpy(area, host.data(), sizeof(double) * nbins);
+    memcpy(grad2, host.data() + nbins, sizeof(double) * nbins);
+    return 0;
+}
+
 static int keff_hist_impl(xfb_handle h, int member, int nbins, float cmin, float cmax, double *area, double *grad2,
                           const cpx *state)
 {
-    if (!area || !grad2 || nbins < 1 || nbins > 2048 || !(cmax > cmin)) return fail(XFB_E_ARG, "bad histogram arguments");
-    CK(cudaSetDevice(h->device));
     const bool fused = fused_diag_ok(h);
     if (fused) {
         if (fused_diag(h, member, 1, h->real_a, h->real_b, state)) return XFB_E_CUDA;       // c, |grad c|^2
@@ -1143,24 +1163,17 @@ static int keff_hist_impl(xfb_handle h, int member, int nbins, float cmin, float
     CK(cudaMemsetAsync(d, 0, sizeof(double) * 2 * nbins, h->stream));
     if (launch_keff_hist(h, h->real_a, h->real_b, fused ? nullptr : h->real_c, (long long)h->grids, nbins, cmin, cmax, d, d + nbins))
         return XFB_E_CUDA;
-    std::vector<double> host(2 * (size_t)nbins);
-    CK(cudaMemcpyAsync(host.data(), d, sizeof(double) * 2 * nbins, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    memcpy(area, host.data(), sizeof(double) * nbins);
-    memcpy(grad2, host.data() + nbins, sizeof(double) * nbins);
-    return 0;
+    return keff_hist_finish(h, d, nbins, area, grad2);
 }
 
+// slab handles: every rank bins its own rows, one all-reduce of the 2 * nbins sums (SURVEY.md 8e); collective
 extern "C" int xfb_get_keff_hist(xfb_handle h, int member, int nbins, float cmin, float cmax, double *area, double *grad2)
 {
     if (check_member(h, member)) return XFB_E_ARG;
     if (!h->have_state) return fail(XFB_E_STATE, "xfb_get_keff_hist before xfb_set_vorticity");
-    if (h->nranks > 1) {
-        // slab handle: every rank bins its own rows, one all-reduce of the 2 * nbins sums (SURVEY.md 8e); collective
-        if (!area || !grad2 || nbins < 1 || nbins > 2048 || !(cmax > cmin)) return fail(XFB_E_ARG, "bad histogram arguments");
-        CK(cudaSetDevice(h->device));
-        return dist_keff_hist(h, nbins, cmin, cmax, area, grad2);
-    }
+    if (int e = keff_hist_args(nbins, cmin, cmax, area, grad2)) return e;
+    CK(cudaSetDevice(h->device));
+    if (h->nranks > 1) return dist_keff_hist(h, nbins, cmin, cmax, area, grad2, false);
     return keff_hist_impl(h, member, nbins, cmin, cmax, area, grad2, nullptr);
 }
 
@@ -1170,31 +1183,32 @@ extern "C" int xfb_get_tracer_keff_hist(xfb_handle h, int member, int nbins, flo
 {
     if (check_member(h, member)) return XFB_E_ARG;
     if (!h->has_tracer) return fail(XFB_E_STATE, "xfb_get_tracer_keff_hist before xfb_set_tracer");
-    if (h->nranks > 1) {
-        if (!area || !grad2 || nbins < 1 || nbins > 2048 || !(cmax > cmin)) return fail(XFB_E_ARG, "bad histogram arguments");
-        CK(cudaSetDevice(h->device));
-        return dist_tracer_keff_hist(h, nbins, cmin, cmax, area, grad2);
-    }
+    if (int e = keff_hist_args(nbins, cmin, cmax, area, grad2)) return e;
+    CK(cudaSetDevice(h->device));
+    if (h->nranks > 1) return dist_keff_hist(h, nbins, cmin, cmax, area, grad2, true);
     return keff_hist_impl(h, member, nbins, cmin, cmax, area, grad2, h->c0);
 }
 
 // Quadratic invariants E, Z, P of the state (vorticity or tracer) and their isotropic shell spectra, reduced on the device
 // from the tile-major (or generic row-major) state in one launch (xfb_spectra.cu); definitions in DESIGN.md section 3.
-static int energy_spectrum_args(xfb_handle h, int member, int which, int nshells, double *totals, double *e, double *z)
+int xfb::energy_spectrum_args(xfb_handle h, int member, int which, int nshells, const double *totals, const double *e,
+                              const double *z, const char *api)
 {
     if (check_member(h, member)) return XFB_E_ARG;
-    if (which != XFB_VORT && which != XFB_TRACER) return fail(XFB_E_ARG, "xfb_get_energy_spectrum: which must be XFB_VORT or XFB_TRACER");
+    if (which != XFB_VORT && which != XFB_TRACER)
+        return fail(XFB_E_ARG, "%sget_energy_spectrum: which must be XFB_VORT or XFB_TRACER", api);
     if (nshells < 0 || nshells > XFB_SPECTRUM_MAX_SHELLS)
-        return fail(XFB_E_ARG, "xfb_get_energy_spectrum: nshells %d not in 0..%d", nshells, XFB_SPECTRUM_MAX_SHELLS);
-    if (!totals || (nshells > 0 && (!e || !z))) return fail(XFB_E_ARG, "xfb_get_energy_spectrum: null output");
-    if (!h->have_state) return fail(XFB_E_STATE, "xfb_get_energy_spectrum before xfb_set_vorticity");
-    if (which == XFB_TRACER && !h->has_tracer) return fail(XFB_E_STATE, "xfb_get_energy_spectrum: XFB_TRACER before xfb_set_tracer");
+        return fail(XFB_E_ARG, "%sget_energy_spectrum: nshells %d not in 0..%d", api, nshells, XFB_SPECTRUM_MAX_SHELLS);
+    if (!totals || (nshells > 0 && (!e || !z))) return fail(XFB_E_ARG, "%sget_energy_spectrum: null output", api);
+    if (!h->have_state) return fail(XFB_E_STATE, "%sget_energy_spectrum before %sset_vorticity", api, api);
+    if (which == XFB_TRACER && !h->has_tracer)
+        return fail(XFB_E_STATE, "%sget_energy_spectrum: XFB_TRACER before %sset_tracer", api, api);
     return 0;
 }
 
 extern "C" int xfb_get_energy_spectrum(xfb_handle h, int member, int which, int nshells, double *totals, double *e, double *z)
 {
-    if (int r = energy_spectrum_args(h, member, which, nshells, totals, e, z)) return r;
+    if (int r = energy_spectrum_args(h, member, which, nshells, totals, e, z, "xfb_")) return r;
     CK(cudaSetDevice(h->device));
     if (h->nranks > 1) return dist_energy_spectrum(h, which, nshells, totals, e, z);     // collective
     if (energy_spectrum_scratch(h)) return XFB_E_CUDA;

@@ -519,28 +519,18 @@ static int team_step(Team *T, int nsteps, float dt)
     return 0;
 }
 
-__global__ void dist_diag_kernel(const float *pxy, const float *pxx, const float *pyy, float *out, long long n, int which)
-{
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float s1 = __fmul_rn(-2.0f, pxy[i]), s2 = __fsub_rn(pxx[i], pyy[i]), z = __fadd_rn(pxx[i], pyy[i]);
-    const float ss = __fadd_rn(__fmul_rn(s1, s1), __fmul_rn(s2, s2)), zz = __fmul_rn(z, z);
-    const float q = __fsub_rn(ss, zz), den = __fadd_rn(ss, zz);
-    if (which == XFB_TFIL) out[i] = (q > 0.0f) ? __fdiv_rn(2.0f, __fsqrt_rn(q)) : 0.0f;
-    else out[i] = (den > 0.0f) ? __fdiv_rn(q, den) : 0.0f;
-}
-
-// spectral operator chain `ops` applied to the state, inverse 2-D transform, into dout[l] (device, local rows)
-static int team_inverse(Team *T, const int *ops, int nops, int negate, float *const *dout, bool tracer_state = false)
+// operator chain `f` applied to the state (tracer_state: the passive tracer's), inverse 2-D transform, into dout[l]
+// (device, local rows)
+static int team_inverse(Team *T, const FieldOps &f, float *const *dout, bool tracer_state = false)
 {
     int e = cols_then_exchange(
         T,
         [&](xfb_handle h, int c) {
             const size_t off = (size_t)c * h->nx * h->pitch;
             const int P = h->pitch;
-            if (launch_pw(h, ops[0], (tracer_state ? h->c0 : h->z0) + off, P, h->spec_a + off, P, P, h->tw_state, 0, c)) return (int)XFB_E_CUDA;
-            for (int o = 1; o < nops; ++o)
-                if (launch_pw(h, ops[o], h->spec_a + off, P, h->spec_a + off, P, P, 0, 0, c)) return (int)XFB_E_CUDA;
+            if (launch_pw(h, f.ops[0], (tracer_state ? h->c0 : h->z0) + off, P, h->spec_a + off, P, P, h->tw_state, 0, c)) return (int)XFB_E_CUDA;
+            for (int o = 1; o < f.nops; ++o)
+                if (launch_pw(h, f.ops[o], h->spec_a + off, P, h->spec_a + off, P, P, 0, 0, c)) return (int)XFB_E_CUDA;
             return launch_col_chunk(h, COL_INV, c, 0, 0.f, h->spec_a, h->spec_b);
         },
         [](xfb_handle h, int) { return h->spec_b; }, [](xfb_handle h, int) { return h->tr[0]; }, 1);
@@ -548,81 +538,49 @@ static int team_inverse(Team *T, const int *ops, int nops, int negate, float *co
     for (int l = 0; l < T->nlocal; ++l) {
         xfb_handle h = T->local[l];
         const cpx *in[4] = {h->tr[0], nullptr, nullptr, nullptr};
-        if (int e2 = launch_row_chunk(h, ROW_C2R, in, nullptr, nullptr, dout[l], negate, 0, h->rows)) return e2;
+        if (int e2 = launch_row_chunk(h, ROW_C2R, in, nullptr, nullptr, dout[l], f.negate, 0, h->rows)) return e2;
         h->tf_valid = false;                      // tr[0] was scratch
     }
     return team_fence(T);       // tr[0] has been consumed everywhere before anybody's next exchange pushes into it
 }
 
-static int team_get_field(Team *T, int which, float *const *dout)
-{
-    static const int op_vort[] = {OP_COPY}, op_psi[] = {OP_INVLAP}, op_u[] = {OP_INVLAP, OP_GRADY}, op_v[] = {OP_INVLAP, OP_GRADX},
-                     op_zx[] = {OP_GRADX}, op_zy[] = {OP_GRADY}, op_pxy[] = {OP_INVLAP, OP_GRADX, OP_GRADY},
-                     op_pxx[] = {OP_INVLAP, OP_GRADX, OP_GRADX}, op_pyy[] = {OP_INVLAP, OP_GRADY, OP_GRADY};
-    switch (which) {
-    case XFB_VORT: return team_inverse(T, op_vort, 1, 0, dout);
-    case XFB_TRACER:
-        if (!T->local[0]->has_tracer) return fail(XFB_E_STATE, "XFB_TRACER before xfb_set_tracer");
-        return team_inverse(T, op_vort, 1, 0, dout, true);
-    case XFB_PSI: return team_inverse(T, op_psi, 1, 0, dout);
-    case XFB_U: return team_inverse(T, op_u, 2, 1, dout);
-    case XFB_V: return team_inverse(T, op_v, 2, 0, dout);
-    case XFB_DVORTDX: return team_inverse(T, op_zx, 1, 0, dout);
-    case XFB_DVORTDY: return team_inverse(T, op_zy, 1, 0, dout);
-    case XFB_TFIL:
-    case XFB_DEFORM: {
-        float *b[16], *c[16];
-        for (int l = 0; l < T->nlocal; ++l) { b[l] = T->local[l]->real_b; c[l] = T->local[l]->real_c; }
-        if (int e = team_inverse(T, op_pxy, 3, 0, b)) return e;
-        if (int e = team_inverse(T, op_pxx, 3, 0, c)) return e;
-        if (int e = team_inverse(T, op_pyy, 3, 0, dout)) return e;
-        for (int l = 0; l < T->nlocal; ++l) {
-            xfb_handle h = T->local[l];
-            const long long n = (long long)h->grids;
-            dist_diag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(b[l], c[l], dout[l], dout[l], n, which);
-            CK(cudaGetLastError());
-            h->launches++;
-        }
-        return 0;
-    }
-    }
-    return fail(XFB_E_ARG, "bad field id %d", which);
-}
-
-// both strain diagnostics from ONE set of the three second derivatives of psi; either output list may be null
+// both strain diagnostics from ONE set of the three second derivatives of psi (psi_xy -> real_b, psi_xx -> real_c,
+// psi_yy -> real_a); either output list may be null, and an output may be real_a only when it is the sole output
 static int team_diagnostics(Team *T, float *const *tfil, float *const *deform)
 {
-    static const int op_pxy[] = {OP_INVLAP, OP_GRADX, OP_GRADY}, op_pxx[] = {OP_INVLAP, OP_GRADX, OP_GRADX},
-                     op_pyy[] = {OP_INVLAP, OP_GRADY, OP_GRADY};
     float *a[16], *b[16], *c[16];
     for (int l = 0; l < T->nlocal; ++l) { a[l] = T->local[l]->real_a; b[l] = T->local[l]->real_b; c[l] = T->local[l]->real_c; }
-    if (int e = team_inverse(T, op_pxy, 3, 0, b)) return e;
-    if (int e = team_inverse(T, op_pxx, 3, 0, c)) return e;
-    if (int e = team_inverse(T, op_pyy, 3, 0, a)) return e;
+    if (int e = team_inverse(T, psi_second_ops[0], b)) return e;
+    if (int e = team_inverse(T, psi_second_ops[1], c)) return e;
+    if (int e = team_inverse(T, psi_second_ops[2], a)) return e;
     for (int l = 0; l < T->nlocal; ++l) {
         xfb_handle h = T->local[l];
         const long long n = (long long)h->grids;
-        for (int o = 0; o < 2; ++o) {
-            float *out = o == 0 ? (tfil ? tfil[l] : nullptr) : (deform ? deform[l] : nullptr);
-            if (!out) continue;
-            dist_diag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(b[l], c[l], a[l], out, n, o == 0 ? XFB_TFIL : XFB_DEFORM);
-            CK(cudaGetLastError());
-            h->launches++;
-        }
+        if (tfil && launch_strain(h, b[l], c[l], a[l], tfil[l], n, XFB_TFIL)) return XFB_E_CUDA;
+        if (deform && launch_strain(h, b[l], c[l], a[l], deform[l], n, XFB_DEFORM)) return XFB_E_CUDA;
     }
     return 0;
+}
+
+static int team_get_field(Team *T, int which, float *const *dout)
+{
+    if (which == XFB_TRACER && !T->local[0]->has_tracer) return fail(XFB_E_STATE, "XFB_TRACER before xfb_set_tracer");
+    if (which == XFB_TFIL) return team_diagnostics(T, dout, nullptr);
+    if (which == XFB_DEFORM) return team_diagnostics(T, nullptr, dout);
+    const FieldOps *f = field_ops(which);
+    if (!f) return fail(XFB_E_ARG, "bad field id %d", which);
+    return team_inverse(T, *f, dout, which == XFB_TRACER);
 }
 
 // effective-diffusivity histograms: zeta, zeta_x, zeta_y of the local rows, binned per rank into `d[l]` (2 * nbins doubles,
 // device); the caller reduces over the ranks
 static int team_keff_hist(Team *T, int nbins, float cmin, float cmax, double *const *d, bool tracer_state = false)
 {
-    static const int op_vort[] = {OP_COPY}, op_zx[] = {OP_GRADX}, op_zy[] = {OP_GRADY};
     float *a[16], *b[16], *c[16];
     for (int l = 0; l < T->nlocal; ++l) { a[l] = T->local[l]->real_a; b[l] = T->local[l]->real_b; c[l] = T->local[l]->real_c; }
-    if (int e = team_inverse(T, op_vort, 1, 0, a, tracer_state)) return e;
-    if (int e = team_inverse(T, op_zx, 1, 0, b, tracer_state)) return e;
-    if (int e = team_inverse(T, op_zy, 1, 0, c, tracer_state)) return e;
+    if (int e = team_inverse(T, *field_ops(XFB_VORT), a, tracer_state)) return e;
+    if (int e = team_inverse(T, *field_ops(XFB_DVORTDX), b, tracer_state)) return e;
+    if (int e = team_inverse(T, *field_ops(XFB_DVORTDY), c, tracer_state)) return e;
     // the inverses above use the spectral scratch arrays the caller may have taken `d` from: zero it only now
     CK(cudaMemsetAsync(d[0], 0, sizeof(double) * 2 * nbins, T->local[0]->stream));
     for (int l = 1; l < T->nlocal; ++l)
@@ -635,40 +593,26 @@ static int team_keff_hist(Team *T, int nbins, float cmin, float cmax, double *co
 }
 
 // ---- entry points used by xfb_api.cu for NCCL handles ----------------------------------------------------
-static int dist_keff_hist_impl(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2, bool tracer_state);
-int dist_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2)
-{
-    return dist_keff_hist_impl(h, nbins, cmin, cmax, area, grad2, false);
-}
-int dist_tracer_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2)
-{
-    return dist_keff_hist_impl(h, nbins, cmin, cmax, area, grad2, true);
-}
-static int dist_keff_hist_impl(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2, bool tracer_state)
+int dist_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2, bool tracer_state)
 {
     if (h->team->loopback) return fail(XFB_E_STATE, "loopback ranks are driven through xfb_loopback_*");
     double *d = (double *)h->spec_a;                 // free scratch of >= 2 * 2048 doubles once the inverses are done
     if (int e = team_keff_hist(h->team, nbins, cmin, cmax, &d, tracer_state)) return e;
     // one all-reduce of the 2 * nbins partial sums over the ranks (SURVEY.md 8e)
     NCK(g_nccl.AllReduce(d, d, (size_t)2 * nbins, ncclDouble, ncclSum, h->team->comm, h->stream));
-    std::vector<double> host(2 * (size_t)nbins);
-    CK(cudaMemcpyAsync(host.data(), d, sizeof(double) * 2 * nbins, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    memcpy(area, host.data(), sizeof(double) * nbins);
-    memcpy(grad2, host.data() + nbins, sizeof(double) * nbins);
-    return 0;
+    return keff_hist_finish(h, d, nbins, area, grad2);
 }
 
 int dist_diagnostics(xfb_handle h, float *tfil_rows, float *deform_rows)
 {
     if (h->team->loopback) return fail(XFB_E_STATE, "loopback ranks are driven through xfb_loopback_*");
     const size_t bytes = sizeof(float) * h->grids;
-    float *scratch = (float *)h->spec_b;             // >= grids floats, free after the last team_inverse
-    float *dt = tfil_rows ? (is_device_ptr(tfil_rows) ? tfil_rows : scratch) : nullptr;
-    float *dd = deform_rows ? (is_device_ptr(deform_rows) ? deform_rows : (float *)h->jint) : nullptr;
+    // host outputs are produced in spectral scratch (>= grids floats) that the last team_inverse has finished with
+    float *dt = tfil_rows ? (float *)stage_out_target(tfil_rows, h->spec_b) : nullptr;
+    float *dd = deform_rows ? (float *)stage_out_target(deform_rows, h->jint) : nullptr;
     if (int e = team_diagnostics(h->team, dt ? &dt : nullptr, dd ? &dd : nullptr)) return e;
-    if (dt && dt != tfil_rows) CK(cudaMemcpyAsync(tfil_rows, dt, bytes, cudaMemcpyDeviceToHost, h->stream));
-    if (dd && dd != deform_rows) CK(cudaMemcpyAsync(deform_rows, dd, bytes, cudaMemcpyDeviceToHost, h->stream));
+    if (tfil_rows && stage_out(h, tfil_rows, dt, bytes, false)) return XFB_E_CUDA;
+    if (deform_rows && stage_out(h, deform_rows, dd, bytes, false)) return XFB_E_CUDA;
     CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
@@ -676,12 +620,10 @@ int dist_diagnostics(xfb_handle h, float *tfil_rows, float *deform_rows)
 int dist_set_vorticity(xfb_handle h, const float *vort_rows)
 {
     if (h->team->loopback) return fail(XFB_E_STATE, "loopback ranks are driven through xfb_loopback_*");
-    const float *din = vort_rows;
-    if (!is_device_ptr(vort_rows)) {
-        CK(cudaMemcpyAsync(h->real_a, vort_rows, sizeof(float) * h->grids, cudaMemcpyHostToDevice, h->stream));
-        din = h->real_a;
-    }
-    if (int e = team_set_vorticity(h->team, &din)) return e;
+    const void *din;
+    if (stage_in(h, vort_rows, h->real_a, sizeof(float) * h->grids, &din)) return XFB_E_CUDA;
+    const float *rows = (const float *)din;
+    if (int e = team_set_vorticity(h->team, &rows)) return e;
     if (!is_device_ptr(vort_rows)) CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
@@ -702,13 +644,9 @@ int dist_step(xfb_handle h, int nsteps, float dt)
 int dist_get_field(xfb_handle h, int which, float *out_rows)
 {
     if (h->team->loopback) return fail(XFB_E_STATE, "loopback ranks are driven through xfb_loopback_*");
-    float *dout = is_device_ptr(out_rows) ? out_rows : h->real_a;
+    float *dout = (float *)stage_out_target(out_rows, h->real_a);
     if (int e = team_get_field(h->team, which, &dout)) return e;
-    if (dout != out_rows) {
-        CK(cudaMemcpyAsync(out_rows, dout, sizeof(float) * h->grids, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-    }
-    return 0;
+    return stage_out(h, out_rows, dout, sizeof(float) * h->grids);
 }
 
 // quadratic invariants and shell spectra: every rank reduces its own column chunks, one all-reduce of the 3 + 2 * nshells
@@ -883,6 +821,12 @@ struct xfb_loopback_s {
     float *full;             // device scratch, one full field
 };
 
+// rows[r] = rank r's rows of `full` (one whole field on the device, as L->full); all null when `full` is
+static void rank_rows(const xfb_loopback_s *L, float *full, float **rows)
+{
+    for (int r = 0; r < L->team.nranks; ++r) rows[r] = full ? full + (size_t)r * L->team.local[0]->rows * L->ny : nullptr;
+}
+
 extern "C" int xfb_loopback_create(xfb_loopback_s **out, int nx, int ny, float lx, float ly, float nu, int device, int nranks,
                                    int nchunks)
 {
@@ -952,8 +896,8 @@ extern "C" int xfb_loopback_set_vorticity(xfb_loopback_s *L, const float *vort_f
     xfb_handle h0 = L->team.local[0];
     CK(cudaSetDevice(h0->device));
     CK(cudaMemcpyAsync(L->full, vort_full_host, sizeof(float) * (size_t)L->nx * L->ny, cudaMemcpyHostToDevice, h0->stream));
-    const float *rows[16];
-    for (int r = 0; r < L->team.nranks; ++r) rows[r] = L->full + (size_t)r * h0->rows * L->ny;
+    float *rows[16];
+    rank_rows(L, L->full, rows);
     if (int e = team_set_vorticity(&L->team, rows)) return e;
     CK(cudaStreamSynchronize(h0->stream));
     return 0;
@@ -976,23 +920,13 @@ extern "C" int xfb_loopback_set_tracer(xfb_loopback_s *L, const float *tracer_fu
     CK(cudaSetDevice(h0->device));
     for (int r = 0; r < L->team.nranks; ++r) {
         xfb_handle h = L->team.local[r];
-        const size_t sb = sizeof(cpx) * h->hpad;
-        if (!h->c0) {
-            cpx **state[] = {&h->c0, &h->ck, &h->cacc, &h->cjint};
-            for (auto pp : state) {
-                if (dev_alloc((void **)pp, sb)) return XFB_E_CUDA;
-                CK(cudaMemsetAsync(*pp, 0, sb, h->stream));
-            }
-            if (dev_alloc((void **)&h->tc[0], 2 * sb)) return XFB_E_CUDA;
-            CK(cudaMemsetAsync(h->tc[0], 0, 2 * sb, h->stream));
-            h->tc[1] = h->tc[0] + h->hpad;
-        }
+        if (tracer_state_alloc(h)) return XFB_E_CUDA;
         h->has_tracer = true;
         h->kappa = kappa;
     }
     CK(cudaMemcpyAsync(L->full, tracer_full_host, sizeof(float) * (size_t)L->nx * L->ny, cudaMemcpyHostToDevice, h0->stream));
-    const float *rows[16];
-    for (int r = 0; r < L->team.nranks; ++r) rows[r] = L->full + (size_t)r * h0->rows * L->ny;
+    float *rows[16];
+    rank_rows(L, L->full, rows);
     if (int e = team_set_vorticity(&L->team, rows, true)) return e;
     CK(cudaStreamSynchronize(h0->stream));
     return 0;
@@ -1022,7 +956,7 @@ extern "C" int xfb_loopback_get_field(xfb_loopback_s *L, int which, float *out_f
     if (!h0->have_state) return fail(XFB_E_STATE, "xfb_loopback_get_field before xfb_loopback_set_vorticity");
     CK(cudaSetDevice(h0->device));
     float *rows[16];
-    for (int r = 0; r < L->team.nranks; ++r) rows[r] = L->full + (size_t)r * h0->rows * L->ny;
+    rank_rows(L, L->full, rows);
     if (int e = team_get_field(&L->team, which, rows)) return e;
     CK(cudaMemcpyAsync(out_full_host, L->full, sizeof(float) * (size_t)L->nx * L->ny, cudaMemcpyDeviceToHost, h0->stream));
     CK(cudaStreamSynchronize(h0->stream));
@@ -1040,10 +974,8 @@ extern "C" int xfb_loopback_get_diagnostics(xfb_loopback_s *L, float *tfil_full_
     if (tfil_full_host && deform_full_host && dev_alloc((void **)&second, sizeof(float) * n)) return XFB_E_CUDA;
     float *t_rows[16], *d_rows[16];
     float *tbuf = tfil_full_host ? L->full : nullptr, *dbuf = deform_full_host ? (tfil_full_host ? second : L->full) : nullptr;
-    for (int r = 0; r < L->team.nranks; ++r) {
-        t_rows[r] = tbuf ? tbuf + (size_t)r * h0->rows * L->ny : nullptr;
-        d_rows[r] = dbuf ? dbuf + (size_t)r * h0->rows * L->ny : nullptr;
-    }
+    rank_rows(L, tbuf, t_rows);
+    rank_rows(L, dbuf, d_rows);
     int e = team_diagnostics(&L->team, tbuf ? t_rows : nullptr, dbuf ? d_rows : nullptr);
     if (!e && tbuf) e = cudaMemcpyAsync(tfil_full_host, tbuf, sizeof(float) * n, cudaMemcpyDeviceToHost, h0->stream) != cudaSuccess;
     if (!e && dbuf) e = cudaMemcpyAsync(deform_full_host, dbuf, sizeof(float) * n, cudaMemcpyDeviceToHost, h0->stream) != cudaSuccess;
@@ -1054,7 +986,8 @@ extern "C" int xfb_loopback_get_diagnostics(xfb_loopback_s *L, float *tfil_full_
 
 extern "C" int xfb_loopback_get_keff_hist(xfb_loopback_s *L, int nbins, float cmin, float cmax, double *area, double *grad2)
 {
-    if (!L || !area || !grad2 || nbins < 1 || nbins > 2048 || !(cmax > cmin)) return fail(XFB_E_ARG, "bad histogram arguments");
+    if (!L) return fail(XFB_E_ARG, "bad histogram arguments");
+    if (int e = keff_hist_args(nbins, cmin, cmax, area, grad2)) return e;
     xfb_handle h0 = L->team.local[0];
     if (!h0->have_state) return fail(XFB_E_STATE, "xfb_loopback_get_keff_hist before xfb_loopback_set_vorticity");
     CK(cudaSetDevice(h0->device));
@@ -1062,24 +995,14 @@ extern "C" int xfb_loopback_get_keff_hist(xfb_loopback_s *L, int nbins, float cm
     double *d[16];
     for (int r = 0; r < L->team.nranks; ++r) d[r] = (double *)L->full;
     if (int e = team_keff_hist(&L->team, nbins, cmin, cmax, d)) return e;
-    std::vector<double> host(2 * (size_t)nbins);
-    CK(cudaMemcpyAsync(host.data(), d[0], sizeof(double) * 2 * nbins, cudaMemcpyDeviceToHost, h0->stream));
-    CK(cudaStreamSynchronize(h0->stream));
-    memcpy(area, host.data(), sizeof(double) * nbins);
-    memcpy(grad2, host.data() + nbins, sizeof(double) * nbins);
-    return 0;
+    return keff_hist_finish(h0, d[0], nbins, area, grad2);
 }
 
 extern "C" int xfb_loopback_get_energy_spectrum(xfb_loopback_s *L, int which, int nshells, double *totals, double *e, double *z)
 {
     if (!L) return fail(XFB_E_ARG, "null argument");
     xfb_handle h0 = L->team.local[0];
-    if (which != XFB_VORT && which != XFB_TRACER) return fail(XFB_E_ARG, "xfb_loopback_get_energy_spectrum: which must be XFB_VORT or XFB_TRACER");
-    if (nshells < 0 || nshells > XFB_SPECTRUM_MAX_SHELLS)
-        return fail(XFB_E_ARG, "xfb_loopback_get_energy_spectrum: nshells %d not in 0..%d", nshells, XFB_SPECTRUM_MAX_SHELLS);
-    if (!totals || (nshells > 0 && (!e || !z))) return fail(XFB_E_ARG, "xfb_loopback_get_energy_spectrum: null output");
-    if (!h0->have_state) return fail(XFB_E_STATE, "xfb_loopback_get_energy_spectrum before xfb_loopback_set_vorticity");
-    if (which == XFB_TRACER && !h0->has_tracer) return fail(XFB_E_STATE, "xfb_loopback_get_energy_spectrum: XFB_TRACER before xfb_loopback_set_tracer");
+    if (int r = energy_spectrum_args(h0, 0, which, nshells, totals, e, z, "xfb_loopback_")) return r;
     CK(cudaSetDevice(h0->device));
     // all ranks share the device and the stream: their launches add into rank 0's sums (the all-reduce of the NCCL path)
     if (energy_spectrum_scratch(h0)) return XFB_E_CUDA;

@@ -306,8 +306,10 @@ int generic_inv2d(xfb_handle h, const cpx *spec_in, cpx *tmp, float *real_out, f
     return 0;
 }
 
-// one RK4 step of every member, one kernel per loop of src/main.cpp:286-317
-static int generic_one_step(xfb_handle h, float dt)
+// one RK4 step of every member, one kernel per loop of src/main.cpp:286-317.  A step is 72 short launches per member
+// (124 with the tracer) on grids that live in L2 -- launch gaps, not kernels, bound it --, so xfb_step replays it from a
+// CUDA graph (step_replay) like the fused step.
+int generic_one_step(xfb_handle h, float dt)
 {
     const int P = h->hy;
     const long long n = (long long)h->grids, hn = (long long)h->nx * h->hy;
@@ -345,47 +347,6 @@ static int generic_one_step(xfb_handle h, float dt)
                 GLAUNCH(h, (gen_stage<false><<<hb, 256, 0, h->stream>>>(h->cjint, c0, ck, cacc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd,
                                                                          h->kappa, dt, (k == 3) ? dt : dt / 2.0f, k, h->kx, LinCoef())));
             }
-        }
-    }
-    return 0;
-}
-
-// nsteps RK4 steps.  A step is 72 short launches per member (124 with the tracer) on grids that live in L2 -- launch
-// gaps, not kernels, bound it --, so like the fused stepper (xfb_step) the step is captured once into a CUDA graph and
-// replayed; the first step of a handle runs eagerly, XFB_NO_GRAPH=1 keeps the eager path.  The graph bakes in dt, the
-// source pointer, the tracer's state (xfb_set_tracer drops it) and the linear terms (xfb_set_linear_terms drops it).
-int generic_step(xfb_handle h, int nsteps, float dt)
-{
-    static const bool no_graph = getenv("XFB_NO_GRAPH") && atoi(getenv("XFB_NO_GRAPH")) != 0;
-    int s = 0;
-    if (nsteps > 0 && (!h->warmed || no_graph)) {
-        const int eager = no_graph ? nsteps : 1;
-        for (; s < eager; ++s)
-            if (int e = generic_one_step(h, dt)) return e;
-        h->warmed = true;
-    }
-    if (s < nsteps) {
-        const void *src_now = h->has_src ? (const void *)h->src : nullptr;
-        if (!h->step_graph || h->graph_dt != dt || h->graph_src != src_now) {
-            if (h->step_graph) { cudaGraphExecDestroy((cudaGraphExec_t)h->step_graph); h->step_graph = nullptr; }
-            cudaGraph_t g = nullptr;
-            CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeRelaxed));
-            const long long l0 = h->launches;
-            const int e = generic_one_step(h, dt);
-            const int per_step = (int)(h->launches - l0);
-            h->launches = l0;
-            cudaError_t ce = cudaStreamEndCapture(h->stream, &g);
-            if (e) { if (g) cudaGraphDestroy(g); return e; }
-            if (ce != cudaSuccess) return fail(XFB_E_CUDA, "cudaStreamEndCapture: %s", cudaGetErrorString(ce));
-            cudaGraphExec_t ge = nullptr;
-            ce = cudaGraphInstantiate(&ge, g, 0);
-            cudaGraphDestroy(g);
-            if (ce != cudaSuccess) return fail(XFB_E_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(ce));
-            h->step_graph = ge; h->graph_dt = dt; h->graph_src = src_now; h->graph_launches = per_step;
-        }
-        for (; s < nsteps; ++s) {
-            CK(cudaGraphLaunch((cudaGraphExec_t)h->step_graph, h->stream));
-            h->launches += h->graph_launches;
         }
     }
     return 0;

@@ -4,6 +4,7 @@
 #include <cstdarg>
 #include <cstddef>
 #include <cstdio>
+#include <functional>
 #include <vector>
 
 #include "../../include/xfb.h"
@@ -64,10 +65,10 @@ struct xfb_handle_s {
     xfb::cpx *dg;        // 3 exchange arrays of the fused diagnostics path, allocated on first use
     double *espec;       // xfb_get_energy_spectrum sums: 3 + 2 * XFB_SPECTRUM_MAX_SHELLS doubles, allocated on first use
     bool warmed;         // one eager step has run (kernels configured)
-    void *step_graph;    // cudaGraphExec_t of one RK4 step (8 launches), valid for graph_dt / graph_src
+    void *step_graph;    // cudaGraphExec_t of one RK4 step (step_replay), valid for graph_dt / graph_src
     float graph_dt;
     const void *graph_src;
-    int graph_launches;  // launches one replay of step_graph stands for (generic path; the fused step has 8 or 16)
+    int graph_launches;  // launches one replay of step_graph stands for (counted while it was captured)
     // passive tracer (xfb_set_tracer), allocated on first use: state like z0/zk/acc/jint, two gradient product arrays
     xfb::cpx *c0, *ck, *cacc, *cjint, *tc[2];
     float kappa;
@@ -111,6 +112,23 @@ bool is_device_ptr(const void *p);
 
 enum { OP_GRADX = 0, OP_GRADY = 1, OP_LAP = 2, OP_INVLAP = 3, OP_DEALIAS = 4, OP_COPY = 5 };
 
+// Spectral operator chain of a record field (xfb_api.cu): ops[0] reads the state, the others run in place, then the
+// inverse 2-D transform with sign `negate`.  field_ops(which) takes the field ids of include/xfb.h and returns null for
+// one that is not such a chain (XFB_SRC, XFB_TFIL, XFB_DEFORM) and for any other value.  psi_second_ops are psi_xy,
+// psi_xx and psi_yy, the second derivatives the strain diagnostics combine; they are not field ids a caller can ask for.
+struct FieldOps {
+    int nops, ops[3], negate;
+};
+const FieldOps *field_ops(int which);
+extern const FieldOps psi_second_ops[3];
+
+// caller buffers (xfb_api.cu): a device pointer is used in place, a host pointer goes through `dev_scratch`.
+// stage_in copies host input in; stage_out_target names the buffer a result is produced in; stage_out copies it to the
+// host unless it was produced in place, and then waits for the copy unless `wait` is false (the caller synchronises).
+int stage_in(xfb_handle h, const void *user, void *dev_scratch, size_t bytes, const void **dev);
+void *stage_out_target(const void *user, void *dev_scratch);
+int stage_out(xfb_handle h, void *user, const void *dev, size_t bytes, bool wait = true);
+
 // pointwise spectral operator on one chunk of K-COL-side columns (chunk 0 on one GPU)
 int launch_pw(xfb_handle h, int op, const cpx *in, int in_pitch, cpx *out, int out_pitch, int ncols, int in_tw = 0,
               int out_tw = 0, int chunk = 0);
@@ -128,12 +146,26 @@ int generic_create(xfb_handle h);
 void generic_destroy(xfb_handle h);
 int generic_fwd2d(xfb_handle h, const float *real_in, cpx *tmp, cpx *spec_out);
 int generic_inv2d(xfb_handle h, const cpx *spec_in, cpx *tmp, float *real_out, float scale, int negate);
-int generic_step(xfb_handle h, int nsteps, float dt);
+int generic_one_step(xfb_handle h, float dt);
+
+// nsteps calls of `one_step` (one RK4 step, xfb_api.cu): the first step of a handle runs eagerly, later ones replay a
+// CUDA graph captured from one call; XFB_NO_GRAPH=1, and profiling when `eager_if_profiling`, keep the eager path
+int step_replay(xfb_handle h, int nsteps, float dt, bool eager_if_profiling, const std::function<int()> &one_step);
+
+// passive tracer state (c0, ck, cacc, cjint; tc[0..1] except on generic grids), allocated and zeroed on first use
+int tracer_state_alloc(xfb_handle h);
 
 // histogram of area and |grad c|^2 over tracer bins of `n` points (xfb_api.cu); accumulates into d_area[nbins], d_grad2[nbins]
 // (device, float64, zeroed by the caller); gy == nullptr: gx holds |grad c|^2
 int launch_keff_hist(xfb_handle h, const float *c, const float *gx, const float *gy, long long n, int nbins, float cmin, float cmax,
                      double *d_area, double *d_grad2);
+// the argument check of every histogram entry point, and the copy of the 2 * nbins device sums d to area / grad2 (host)
+int keff_hist_args(int nbins, float cmin, float cmax, const double *area, const double *grad2);
+int keff_hist_finish(xfb_handle h, const double *d, int nbins, double *area, double *grad2);
+
+// filamentation time (which = XFB_TFIL) or deformation factor (XFB_DEFORM) of `n` points from psi_xy, psi_xx, psi_yy
+// (xfb_api.cu); `out` may be any of the inputs: each element is read before it is written
+int launch_strain(xfb_handle h, const float *pxy, const float *pxx, const float *pyy, float *out, long long n, int which);
 
 // quadratic invariants and shell spectra (xfb_spectra.cu): one launch adds the raw sums of one state array into
 // d_out[3 + 2 * nshells] (device, zeroed by the caller); _finish copies them to the host and scales them to domain means
@@ -141,13 +173,16 @@ long long shells_all(int nx, int ny, float lx, float ly);
 int energy_spectrum_scratch(xfb_handle h);
 int launch_energy_spectrum(xfb_handle h, const cpx *state, int nshells, double *d_out);
 int energy_spectrum_finish(xfb_handle h, const double *d, int nshells, double *totals, double *e, double *z);
+// argument and state checks of xfb_get_energy_spectrum (xfb_api.cu); `api` ("xfb_" or "xfb_loopback_") prefixes the entry
+// points the messages name
+int energy_spectrum_args(xfb_handle h, int member, int which, int nshells, const double *totals, const double *e, const double *z,
+                         const char *api);
 
 // slab paths (xfb_dist.cu)
-int dist_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2);
+int dist_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2, bool tracer_state);
 int dist_diagnostics(xfb_handle h, float *tfil_rows, float *deform_rows);
 int dist_set_vorticity(xfb_handle h, const float *vort_rows);
 int dist_set_tracer(xfb_handle h, const float *tracer_rows);
-int dist_tracer_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2);
 int dist_step(xfb_handle h, int nsteps, float dt);
 int dist_get_field(xfb_handle h, int which, float *out_rows);
 int dist_energy_spectrum(xfb_handle h, int which, int nshells, double *totals, double *e, double *z);
