@@ -120,6 +120,20 @@ int xfb_get_keff_hist(xfb_handle h, int member, int nbins, float cmin, float cma
  * z[nshells] = shell sums of E and Z.  Host pointers only.  Reads the state only: later steps are unaffected.
  * Slab-decomposed handles: collective, every rank receives the whole-domain result. */
 int xfb_get_energy_spectrum(xfb_handle h, int member, int which, int nshells, double *totals, double *e, double *z);
+/* spectral budget of the vorticity (no reference counterpart; definitions in DESIGN.md section 3): the rates that the
+ * nonlinear transfer T, the forcing F (xfb_set_source; zero without one) and the dissipation D (nu, mu and the
+ * hyperviscosity of xfb_set_linear_terms) give the energy E and the enstrophy Z of xfb_get_energy_spectrum, per mode
+ * w_j M Re(conj(Z_k) X_k) / Np^2 (over k^2 for E) inside the dealiasing mask M, with X = the r2c of -u.grad(zeta) formed as
+ * the stepper's first Runge-Kutta stage forms it, the r2c of the source, and (-nu k^2 - mu - nu_h k^(2 order)) Z_k.  The
+ * beta term rotates the phase of each mode and adds nothing to E or Z: it is no term of the budget.  totals[6] = domain
+ * sums over all modes, in XFB_BUDGET_* order; nshells == 0: totals only (budget may be NULL), else
+ * budget[q * nshells + s] = the sum of quantity q over shell s (the shells of xfb_get_energy_spectrum, modes beyond
+ * nshells count in the totals only).  Host pointers only.  Vorticity only.  Reads the state and leaves later steps
+ * bit-identical (it may form the products the next step would form first).  Slab-decomposed handles: collective,
+ * every rank receives the whole-domain result. */
+enum { XFB_BUDGET_TE = 0, XFB_BUDGET_FE = 1, XFB_BUDGET_DE = 2, XFB_BUDGET_TZ = 3, XFB_BUDGET_FZ = 4, XFB_BUDGET_DZ = 5,
+       XFB_BUDGET_N = 6 };
+int xfb_get_spectral_budget(xfb_handle h, int member, int nshells, double *totals, double *budget);
 
 /* ---- passive tracer (SURVEY.md section 8 (f-4); the reference has none) -------------------------
  * dc/dt = -u c_x - v c_y + kappa lap(c), advanced by xfb_step together with the vorticity: every Runge-Kutta stage
@@ -184,6 +198,7 @@ int xfb_loopback_get_field(xfb_loopback t, int which, float *out);
 int xfb_loopback_get_diagnostics(xfb_loopback t, float *tfil, float *deform);
 int xfb_loopback_get_keff_hist(xfb_loopback t, int nbins, float cmin, float cmax, double *area, double *grad2);
 int xfb_loopback_get_energy_spectrum(xfb_loopback t, int which, int nshells, double *totals, double *e, double *z);
+int xfb_loopback_get_spectral_budget(xfb_loopback t, int nshells, double *totals, double *budget);
 long long xfb_loopback_launch_count(xfb_loopback t);
 
 /* ---- introspection --------------------------------------------------------------------------*/

@@ -30,7 +30,11 @@ SYMBOLS = [
     "xfb_loopback_get_keff_hist", "xfb_loopback_set_tracer",
     "xfb_get_energy_spectrum", "xfb_loopback_get_energy_spectrum",
     "xfb_set_linear_terms", "xfb_loopback_set_linear_terms",
+    "xfb_get_spectral_budget", "xfb_loopback_get_spectral_budget",
 ]
+
+# rows of Backend.spectral_budget: transfer, forcing and dissipation rates of E, then of Z (include/xfb.h XFB_BUDGET_*)
+BUDGET_TE, BUDGET_FE, BUDGET_DE, BUDGET_TZ, BUDGET_FZ, BUDGET_DZ = range(6)
 
 _lib = None
 
@@ -70,6 +74,8 @@ def load():
     L.xfb_get_tracer_keff_hist.argtypes = [vp, ci, ci, cf, cf, vp, vp]
     L.xfb_get_energy_spectrum.argtypes = [vp, ci, ci, ci, vp, vp, vp]
     L.xfb_loopback_get_energy_spectrum.argtypes = [vp, ci, ci, vp, vp, vp]
+    L.xfb_get_spectral_budget.argtypes = [vp, ci, ci, vp, vp]
+    L.xfb_loopback_get_spectral_budget.argtypes = [vp, ci, vp, vp]
     L.xfb_set_tracer.argtypes = [vp, ci, vp, cf]
     L.xfb_set_linear_terms.argtypes = [vp, cf, cf, cf, ci]
     L.xfb_loopback_set_linear_terms.argtypes = [vp, cf, cf, cf, ci]
@@ -138,6 +144,16 @@ def _energy_spectrum(L, call, nshells, nx, ny, lx, ly):
     if rc != 0:
         raise XfbError(f"xfb error {rc}: {L.xfb_last_error().decode()}")
     return totals, e, z
+
+
+def _spectral_budget(L, call, nshells, nx, ny, lx, ly):
+    n = shells_all(nx, ny, lx, ly) if nshells is None else int(nshells)
+    totals = np.zeros(6, np.float64)
+    budget = np.zeros((6, n), np.float64)
+    rc = call(_ptr(totals), _ptr(budget) if n else None, n)
+    if rc != 0:
+        raise XfbError(f"xfb error {rc}: {L.xfb_last_error().decode()}")
+    return totals, budget
 
 
 def nccl_unique_id() -> bytes:
@@ -284,6 +300,13 @@ class Backend:
         """-> (totals [E, Z, P], e[nshells], z[nshells]): domain-mean kinetic energy, enstrophy, palinstrophy and the
         shell sums of E and Z (float64); nshells=None: every shell (shells_all).  which = VORT or TRACER."""
         return _energy_spectrum(self._L, lambda t, e, z, n: self._L.xfb_get_energy_spectrum(self._h, member, which, n, t, e, z),
+                                nshells, self.nx, self.ny, self.lx, self.ly)
+
+    def spectral_budget(self, nshells=None, member=0):
+        """-> (totals[6], budget[6, nshells]): rates of E and Z from the nonlinear transfer, the forcing and the
+        dissipation, rows in BUDGET_* order (T_E, F_E, D_E, T_Z, F_Z, D_Z), domain sums and shell sums of the shells of
+        energy_spectrum (float64); nshells=None: every shell.  Leaves later steps unchanged."""
+        return _spectral_budget(self._L, lambda t, b, n: self._L.xfb_get_spectral_budget(self._h, member, n, t, b),
                                 nshells, self.nx, self.ny, self.lx, self.ly)
 
     # passive tracer: advected by xfb_step with the flow of each stage; read back with get_field(TRACER)
@@ -450,6 +473,11 @@ class LoopbackTeam:
     def energy_spectrum(self, nshells=None, which=VORT):
         """whole-domain (totals, e, z) as Backend.energy_spectrum"""
         return _energy_spectrum(self._L, lambda t, e, z, n: self._L.xfb_loopback_get_energy_spectrum(self._t, which, n, t, e, z),
+                                nshells, self.nx, self.ny, self.lx, self.ly)
+
+    def spectral_budget(self, nshells=None):
+        """whole-domain (totals, budget) as Backend.spectral_budget"""
+        return _spectral_budget(self._L, lambda t, b, n: self._L.xfb_loopback_get_spectral_budget(self._t, n, t, b),
                                 nshells, self.nx, self.ny, self.lx, self.ly)
 
     @property

@@ -19,6 +19,11 @@
 //      `step time member E Z P`, and the isotropic shell spectra written to <output>/spectrum_step_N.txt -- .m<m>.txt for
 //      members other than 0 -- one `s k[1/m] E(s) Z(s)` line per shell; neither goes into `log`.  A non-finite total
 //      stops the run with exit status 1 once the record files already issued are written).
+//   -T (at every record step, per member: the spectral budget of xfb_get_spectral_budget -- the rates of E and Z from the
+//      nonlinear transfer T, the forcing F (the source the handle holds) and the dissipation D -- written to
+//      <output>/budget_step_N.txt (.m<m>.txt for members other than 0), one `s k[1/m] T_E F_E D_E T_Z F_Z D_Z Pi_E Pi_Z`
+//      line per shell with the fluxes Pi(s) = -sum_{s' <= s} T(s'), and the domain totals appended to <output>/budget.txt
+//      as `step time member T_E F_E D_E T_Z F_Z D_Z`; neither goes into `log`).
 //   -B <beta> -R <mu> -H <nu_h> -P <order=4> (linear terms of the vorticity equation, xfb_set_linear_terms: beta-plane
 //      [1/(m s)], linear drag [1/s], hyperviscosity nu_h (-lap)^order [m^(2 order)/s], order 1..8; on every handle of the
 //      run, -b, -G and -S ranks included.  An invalid value stops with exit status 1 before any step.  Without these
@@ -88,6 +93,36 @@ static int write_energy(const std::string &output, FILE *integrals, int step, fl
     return (std::isfinite(tot[0]) && std::isfinite(tot[1]) && std::isfinite(tot[2])) ? 0 : 1;
 }
 
+// -T at one record step for one member: budget file with the fluxes formed here, totals line
+static void write_budget(const std::string &output, FILE *totals_file, int step, float dt, int member, float L, const double *tot,
+                         const std::vector<double> &b)
+{
+    const size_t nsh = b.size() / XFB_BUDGET_N;
+    char name[1024];
+    if (member == 0) std::snprintf(name, sizeof(name), "%s/budget_step_%d.txt", output.c_str(), step);
+    else std::snprintf(name, sizeof(name), "%s/budget_step_%d.m%d.txt", output.c_str(), step, member);
+    if (FILE *f = std::fopen(name, "w")) {
+        std::fprintf(f, "# s  k[1/m]  T_E  F_E  D_E  T_Z  F_Z  D_Z  Pi_E  Pi_Z   (step %d, member %d; shell sums of the rates of "
+                        "E and Z, Pi(s) = -sum of T up to s)\n", step, member);
+        const double dk = 2.0 * M_PI / (double)L;
+        double pe = 0.0, pz = 0.0;
+        for (size_t k = 0; k < nsh; ++k) {
+            pe -= b[XFB_BUDGET_TE * nsh + k];
+            pz -= b[XFB_BUDGET_TZ * nsh + k];
+            std::fprintf(f, "%zu %.9g", k, dk * (double)k);
+            for (int q = 0; q < XFB_BUDGET_N; ++q) std::fprintf(f, " %.17g", b[q * nsh + k]);
+            std::fprintf(f, " %.17g %.17g\n", pe, pz);
+        }
+        std::fclose(f);
+    }
+    if (totals_file) {
+        std::fprintf(totals_file, "%d %.17g %d", step, (double)step * dt, member);
+        for (int q = 0; q < XFB_BUDGET_N; ++q) std::fprintf(totals_file, " %.17g", tot[q]);
+        std::fprintf(totals_file, "\n");
+        std::fflush(totals_file);
+    }
+}
+
 // -B -R -H -P: the linear terms, applied to every handle the run creates
 struct LinOpts {
     bool set;
@@ -114,7 +149,7 @@ struct SlabOpts {
     std::string input, output, init_file;
     int npts, record_step, total_steps, device, ranks;
     float L, NU, dt;
-    bool diagnostics, quiet, energy;
+    bool diagnostics, quiet, energy, budget;
     LinOpts lin;
 };
 
@@ -149,6 +184,12 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
     }
     const int nsh = o.energy ? all_shells(n) : 0;
     std::vector<double> es(nsh), zs(nsh);
+    FILE *budget_file = nullptr;
+    if (o.budget && rank == 0) {
+        std::snprintf(filename, sizeof(filename), "%s/budget.txt", o.output.c_str());
+        budget_file = std::fopen(filename, "w");
+    }
+    std::vector<double> bs(o.budget ? (size_t)XFB_BUDGET_N * all_shells(n) : 0);
     CHECK(xfb_set_vorticity(h, 0, buf.data()));
     if (rank == 0) std::printf("Initialization complete.\n");
     auto record = [&](const char *stem, int which, int step) -> int {
@@ -187,6 +228,11 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
                     return 1;
                 }
             }
+            if (o.budget) {
+                double tot[XFB_BUDGET_N];
+                CHECK(xfb_get_spectral_budget(h, 0, (int)(bs.size() / XFB_BUDGET_N), tot, bs.data()));      // collective
+                if (rank == 0) write_budget(o.output, budget_file, step, o.dt, 0, o.L, tot, bs);
+            }
         }
         const int next_record = (step / o.record_step + 1) * o.record_step;
         const int chunk = (next_record < o.total_steps ? next_record : o.total_steps) - step;
@@ -198,6 +244,7 @@ static int slab_rank(const SlabOpts &o, int rank, const char *id128)
     CHECK(xfb_sync(h));
     if (log_fd) std::fclose(log_fd);
     if (integrals) std::fclose(integrals);
+    if (budget_file) std::fclose(budget_file);
     xfb_destroy(h);
     if (rank == 0) std::printf("Program ends. Congrats!\n");
     return 0;
@@ -248,12 +295,12 @@ int main(int argc, char *args[])
     RECIPE_TYPE recipe_type = EMPTY;
     int npts = 768, record_step = 100, total_steps = -1, device = 0, members = 1, ngpus = 1, slab_ranks = 0;
     float L = 600000.0f, NU = 6.5f, dt = 3.0f;
-    bool diagnostics = false, quiet = false, energy = false;
+    bool diagnostics = false, quiet = false, energy = false, budget = false;
     LinOpts lin{false, 0.0f, 0.0f, 0.0f, 4};
     bool bad_lin = false;
 
     int opt;
-    while ((opt = getopt(argc, args, "I:O:o:i:s:f:n:d:t:r:L:N:g:c:k:b:G:S:B:R:H:P:DEq")) != EOF) {
+    while ((opt = getopt(argc, args, "I:O:o:i:s:f:n:d:t:r:L:N:g:c:k:b:G:S:B:R:H:P:DETq")) != EOF) {
         switch (opt) {
         case 'I': input = optarg; break;
         case 'O': case 'o': output = optarg; break;
@@ -274,6 +321,7 @@ int main(int argc, char *args[])
         case 'S': slab_ranks = std::atoi(optarg); break;
         case 'D': diagnostics = true; break;
         case 'E': energy = true; break;
+        case 'T': budget = true; break;
         case 'q': quiet = true; break;
         case 'B': lin.set = true; bad_lin |= !parse_float(optarg, &lin.beta); break;
         case 'R': lin.set = true; bad_lin |= !parse_float(optarg, &lin.mu) || lin.mu < 0.0f; break;
@@ -318,7 +366,7 @@ int main(int argc, char *args[])
             return 1;
         }
         SlabOpts so{input, output, init_file, npts, record_step, total_steps, device, slab_ranks, L, NU, dt, diagnostics, quiet,
-                    energy, lin};
+                    energy, budget, lin};
         return run_slab(so);
     }
 
@@ -332,6 +380,13 @@ int main(int argc, char *args[])
     }
     const int nsh = energy ? all_shells(npts) : 0;
     std::vector<double> es(nsh), zs(nsh);
+    FILE *budget_file = nullptr;                                    // -T
+    if (budget) {
+        const std::string name = output + "/budget.txt";
+        budget_file = std::fopen(name.c_str(), "w");
+        if (!budget_file) perror("Open budget.txt");
+    }
+    std::vector<double> bs(budget ? (size_t)XFB_BUDGET_N * all_shells(npts) : 0);
 
     // ensemble members in blocks over the devices: handle d holds members [first[d], first[d] + count[d])
     std::vector<xfb_handle> hs(ngpus, nullptr);
@@ -488,6 +543,17 @@ int main(int argc, char *args[])
                     return 1;
                 }
             }
+            for (int m = 0; budget && m < members; ++m) {
+                int lm = 0;
+                xfb_handle hm = owner(m, &lm);
+                double tot[XFB_BUDGET_N];
+                if (xfb_get_spectral_budget(hm, lm, (int)(bs.size() / XFB_BUDGET_N), tot, bs.data()) != 0) {
+                    std::fprintf(stderr, "main.out: %s\n", xfb_last_error());
+                    shutdown_writer();
+                    return 1;
+                }
+                write_budget(output, budget_file, step, dt, m, L, tot, bs);
+            }
         }
         int chunk = 1;
         if (recipe_type == EMPTY) {
@@ -535,6 +601,7 @@ int main(int argc, char *args[])
     xfb_host_free(src);
     if (log_fd) std::fclose(log_fd);
     if (integrals) std::fclose(integrals);
+    if (budget_file) std::fclose(budget_file);
     for (xfb_handle hd : hs) xfb_destroy(hd);
     (void)h;
     std::printf("Program ends. Congrats!\n");

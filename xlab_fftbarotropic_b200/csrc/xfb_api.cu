@@ -340,7 +340,7 @@ int xfb::destroy_impl(xfb_handle h)
         cudaStreamDestroy(h->rec_stream);
     }
     void *ptrs[] = {h->tw, h->kx, h->ky, h->kx2, h->ky2, h->z0, h->zk, h->acc, h->jint, h->t_block, h->src, h->dg, h->real_a,
-                    h->real_b, h->real_c, h->spec_a, h->spec_b, h->ref_a, h->ref_b, h->recv_block, h->sync_buf, h->espec, h->c0, h->ck, h->cacc, h->cjint, h->tc[0], h->panel_base, h->panel_base_c};
+                    h->real_b, h->real_c, h->spec_a, h->spec_b, h->ref_a, h->ref_b, h->recv_block, h->sync_buf, h->espec, h->bspec, h->c0, h->ck, h->cacc, h->cjint, h->tc[0], h->panel_base, h->panel_base_c};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (auto pool : {h->ev_row, h->ev_col, h->ev_a2a})
@@ -746,6 +746,15 @@ extern "C" int xfb_set_linear_terms(xfb_handle h, float beta, float mu, float nu
     return 0;
 }
 
+// K-COL parameters of the fused stepper: every member's state (tile-major), tendency and product arrays
+static void stepper_col(xfb_handle h, ColParams &c)
+{
+    fill_col(h, c);
+    c.jint = h->jint; c.z0 = h->z0; c.zk = h->zk; c.acc = h->acc;
+    c.st_tile_stride = (long long)h->nx * h->tw_state; c.st_row_stride = h->tw_state;     // tile-major state
+    for (int f = 0; f < 4; ++f) c.t_out[f] = h->t[f];
+}
+
 extern "C" int xfb_step(xfb_handle h, int nsteps, float dt)
 {
     if (!h) return fail(XFB_E_ARG, "null handle");
@@ -754,10 +763,7 @@ extern "C" int xfb_step(xfb_handle h, int nsteps, float dt)
     CK(cudaSetDevice(h->device));
     if (h->nranks > 1) return dist_step(h, nsteps, dt);
     if (h->generic) return step_replay(h, nsteps, dt, false, [&]() { return generic_one_step(h, dt); });
-    ColParams c; fill_col(h, c);
-    c.jint = h->jint; c.z0 = h->z0; c.zk = h->zk; c.acc = h->acc;
-    c.st_tile_stride = (long long)h->nx * h->tw_state; c.st_row_stride = h->tw_state;     // tile-major state
-    for (int f = 0; f < 4; ++f) c.t_out[f] = h->t[f];
+    ColParams c; stepper_col(h, c);
     c.dt = dt;
     RowParams r; fill_row(h, r, h->nx * h->batch);
     for (int f = 0; f < 4; ++f) r.spec_in[f] = h->t[f];
@@ -1216,6 +1222,86 @@ extern "C" int xfb_get_energy_spectrum(xfb_handle h, int member, int which, int 
     CK(cudaMemsetAsync(h->espec, 0, sizeof(double) * (3 + 2 * (size_t)nshells), h->stream));
     if (launch_energy_spectrum(h, state, nshells, h->espec)) return XFB_E_CUDA;
     return energy_spectrum_finish(h, h->espec, nshells, totals, e, z);
+}
+
+// Spectral budget of the vorticity (DESIGN.md section 3): the tendency N = r2c(-u.grad(zeta)) and the source's spectrum S
+// of one member are formed with the stepper's own transforms into scratch arrays in the state's layout, then one
+// reduction (xfb_spectra.cu) reads state, N and S once.  Scratch: spec_a, spec_b and jint, which the next stage
+// overwrites before reading; the products t[0..3] of the current state are formed as the next step would form them.
+int xfb::spectral_budget_args(xfb_handle h, int member, int nshells, const double *totals, const double *budget, const char *api)
+{
+    if (check_member(h, member)) return XFB_E_ARG;
+    if (nshells < 0 || nshells > XFB_SPECTRUM_MAX_SHELLS)
+        return fail(XFB_E_ARG, "%sget_spectral_budget: nshells %d not in 0..%d", api, nshells, XFB_SPECTRUM_MAX_SHELLS);
+    if (!totals || (nshells > 0 && !budget)) return fail(XFB_E_ARG, "%sget_spectral_budget: null output", api);
+    if (!h->have_state) return fail(XFB_E_STATE, "%sget_spectral_budget before %sset_vorticity", api, api);
+    return 0;
+}
+
+// tendency and source spectrum of one member on one GPU, tile-major (row-major on generic grids); *n, *s name the arrays
+// (*s null without a source)
+static int budget_terms(xfb_handle h, int member, const cpx **n, const cpx **s)
+{
+    const float *src = h->has_src ? h->src + (size_t)member * h->grids : nullptr;
+    *s = nullptr;
+    if (h->generic) {
+        // generic_one_step's stage body without the source, stopping before gen_stage
+        if (generic_tendency(h, h->z0 + (size_t)member * h->hpad, nullptr, h->jint)) return XFB_E_CUDA;
+        *n = h->jint;
+        if (src) {
+            if (fwd2d(h, src, h->spec_a, h->spec_b)) return XFB_E_CUDA;
+            *s = h->spec_b;
+        }
+        return 0;
+    }
+    if (!h->tf_valid) {
+        ColParams c; stepper_col(h, c);
+        CKL(h, launch_col(h->nx, COL_PRO, c, h->batch, h->stream));
+        h->tf_valid = true;
+    }
+    RowParams r; fill_row(h, r, h->nx);
+    for (int f = 0; f < 4; ++f) r.spec_in[f] = h->t[f] + (size_t)member * h->hpad;
+    r.real_in = nullptr;
+    r.spec_out = h->spec_a;
+    CKL(h, launch_row(h->ny, ROW_JAC, r, h->stream));
+    if (h->nx <= 8192 && h->ny <= 8192) {
+        // x pass of the pair-layout tendency straight into tile-major scratch, then the source the way set_vorticity goes
+        ColParams c; fill_col(h, c);
+        c.jint = h->spec_a; c.z0 = h->spec_b; c.zk = c.z0; c.acc = c.z0;
+        c.st_tile_stride = (long long)h->nx * h->tw_state; c.st_row_stride = h->tw_state;
+        CKL(h, launch_col(h->nx, COL_FWDT, c, 1, h->stream));
+        *n = h->spec_b;
+        if (src) {
+            if (fused_forward_to_state(h, src, h->jint)) return XFB_E_CUDA;
+            *s = h->jint;
+        }
+        return 0;
+    }
+    // 16384-point lines: plain x pass into row-major scratch, then the layout conversion (as xfb_set_tracer does)
+    ColParams c; fill_col(h, c);
+    c.jint = h->spec_a; c.z0 = h->spec_b;
+    CKL(h, launch_col(h->nx, COL_FWD, c, 1, h->stream));
+    if (launch_pw(h, OP_COPY, h->spec_b, h->pitch, h->jint, h->pitch, h->pitch, 0, h->tw_state)) return XFB_E_CUDA;
+    *n = h->jint;
+    if (src) {
+        if (fwd2d(h, src, h->spec_a, h->spec_b)) return XFB_E_CUDA;
+        if (launch_pw(h, OP_COPY, h->spec_b, h->pitch, h->spec_a, h->pitch, h->pitch, 0, h->tw_state)) return XFB_E_CUDA;
+        *s = h->spec_a;
+    }
+    return 0;
+}
+
+extern "C" int xfb_get_spectral_budget(xfb_handle h, int member, int nshells, double *totals, double *budget)
+{
+    if (int r = spectral_budget_args(h, member, nshells, totals, budget, "xfb_")) return r;
+    CK(cudaSetDevice(h->device));
+    if (h->nranks > 1) return dist_spectral_budget(h, nshells, totals, budget);      // collective
+    if (spectral_budget_scratch(h)) return XFB_E_CUDA;
+    const cpx *n, *s;
+    if (budget_terms(h, member, &n, &s)) return XFB_E_CUDA;
+    CK(cudaMemsetAsync(h->bspec, 0, sizeof(double) * XFB_BUDGET_N * (1 + (size_t)nshells), h->stream));
+    if (launch_spectral_budget(h, h->z0 + (size_t)member * h->hpad, n, s, nshells, h->bspec)) return XFB_E_CUDA;
+    return spectral_budget_finish(h, h->bspec, nshells, totals, budget);
 }
 
 // ------------------------------------------------------------------------------------------------

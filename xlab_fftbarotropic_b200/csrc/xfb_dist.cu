@@ -299,8 +299,9 @@ static int launch_row_chunk(xfb_handle h, int mode, const cpx *const in[4], cons
 }
 
 // tracer: the same launch on the passive tracer's arrays (state c0 / ck / cacc, tendency cjint_recv, two gradient
-// products tc[0..1], diffusivity kappa); `mode` is then COL_TSTEP / COL_TPRO (or COL_FWD into c0)
-static int launch_col_chunk(xfb_handle h, int mode, int chunk, int stage, float dt, const cpx *inv_in, cpx *inv_out, bool tracer = false)
+// products tc[0..1], diffusivity kappa); `mode` is then COL_TSTEP / COL_TPRO (or COL_FWD into c0).
+// out: COL_INV's output; COL_FWD writes there instead of the state when it is not null
+static int launch_col_chunk(xfb_handle h, int mode, int chunk, int stage, float dt, const cpx *inv_in, cpx *out, bool tracer = false)
 {
     ColParams c;
     fill_col(h, c, chunk);
@@ -313,7 +314,8 @@ static int launch_col_chunk(xfb_handle h, int mode, int chunk, int stage, float 
         if (mode != COL_FWD) c.jint = h->cjint_recv + off;       // COL_FWD: the field just travelled through jint_recv
         for (int f = 0; f < 4; ++f) c.t_out[f] = h->tc[f & 1] + off;
     }
-    if (mode == COL_INV) { c.inv_in = inv_in + off; c.t_out[0] = inv_out + off; }
+    if (mode == COL_INV) { c.inv_in = inv_in + off; c.t_out[0] = out + off; }
+    if (mode == COL_FWD && out) c.z0 = out + off;
     c.dt = dt; c.stage = stage;
     c.dt_stage = (stage == 3) ? dt : dt / 2.0f;          // main.cpp:296,299,302
     if (h->self_direct && (mode == COL_STEP || mode == COL_PRO || mode == COL_TSTEP || mode == COL_TPRO)) {
@@ -519,6 +521,43 @@ static int team_step(Team *T, int nsteps, float dt)
     return 0;
 }
 
+// Spectral budget terms of every local rank, tile-major chunks like the state: the tendency r2c(-u.grad(zeta)) into
+// spec_a (the stepper's K-ROW without the source, its exchange, a plain x pass per chunk) and, when `with_src`, the
+// source's spectrum into spec_b (as team_set_vorticity forms a state; a rank without a source contributes zero rows).
+// The products t[0..3] / tr[0..3] of the current state are formed first if the next step would have to form them.
+static int team_budget_terms(Team *T, bool with_src)
+{
+    xfb_handle h0 = T->local[0];
+    if (!h0->tf_valid) {
+        if (int e = team_products(T, COL_PRO, 0, 0.f)) return e;
+        for (int l = 0; l < T->nlocal; ++l) T->local[l]->tf_valid = true;
+    }
+    for (int pass = 0; pass < (with_src ? 2 : 1); ++pass) {
+        if (pass == 1) {
+            // jint_recv has been read everywhere before the source's rows land in it
+            if (int e = team_fence(T)) return e;
+            for (int l = 0; l < T->nlocal; ++l) {
+                xfb_handle h = T->local[l];
+                if (!h->has_src) CK(cudaMemsetAsync(h->real_a, 0, sizeof(float) * h->grids, h->stream));
+            }
+        }
+        int e = rows_then_exchange(
+            T,
+            [&](xfb_handle h, int r0, int r1) {
+                if (pass == 0) return launch_row_chunk(h, ROW_JAC, h->tr, nullptr, h->jint, nullptr, 0, r0, r1, true);
+                return launch_row_chunk(h, ROW_R2C, nullptr, h->has_src ? h->src : h->real_a, h->jint, nullptr, 0, r0, r1, true);
+            },
+            [](xfb_handle h) { return h->jint; }, [](xfb_handle h) { return h->jint_recv; });
+        if (e) return e;
+        for (int l = 0; l < T->nlocal; ++l) {
+            xfb_handle h = T->local[l];
+            for (int c = 0; c < h->nchunks; ++c)
+                if (int e2 = launch_col_chunk(h, COL_FWD, c, 0, 0.f, nullptr, pass == 0 ? h->spec_a : h->spec_b)) return e2;
+        }
+    }
+    return team_fence(T);       // jint_recv has been consumed everywhere before anybody's next K-ROW stores into it
+}
+
 // operator chain `f` applied to the state (tracer_state: the passive tracer's), inverse 2-D transform, into dout[l]
 // (device, local rows)
 static int team_inverse(Team *T, const FieldOps &f, float *const *dout, bool tracer_state = false)
@@ -660,6 +699,20 @@ int dist_energy_spectrum(xfb_handle h, int which, int nshells, double *totals, d
     if (int r = launch_energy_spectrum(h, which == XFB_TRACER ? h->c0 : h->z0, nshells, h->espec)) return r;
     NCK(g_nccl.AllReduce(h->espec, h->espec, n, ncclDouble, ncclSum, h->team->comm, h->stream));
     return energy_spectrum_finish(h, h->espec, nshells, totals, e, z);
+}
+
+// spectral budget: the terms of every rank (collective exchanges), the reduction of its own column chunks, one all-reduce
+// of the 6 + 6 * nshells sums.  Every rank runs the source pass: no rank knows whether a peer has a source.
+int dist_spectral_budget(xfb_handle h, int nshells, double *totals, double *budget)
+{
+    if (h->team->loopback) return fail(XFB_E_STATE, "loopback ranks are driven through xfb_loopback_*");
+    if (spectral_budget_scratch(h)) return XFB_E_CUDA;
+    if (int r = team_budget_terms(h->team, true)) return r;
+    const size_t n = XFB_BUDGET_N * (1 + (size_t)nshells);
+    CK(cudaMemsetAsync(h->bspec, 0, sizeof(double) * n, h->stream));
+    if (int r = launch_spectral_budget(h, h->z0, h->spec_a, h->spec_b, nshells, h->bspec)) return r;
+    NCK(g_nccl.AllReduce(h->bspec, h->bspec, n, ncclDouble, ncclSum, h->team->comm, h->stream));
+    return spectral_budget_finish(h, h->bspec, nshells, totals, budget);
 }
 
 void dist_release(xfb_handle h)
@@ -1012,6 +1065,25 @@ extern "C" int xfb_loopback_get_energy_spectrum(xfb_loopback_s *L, int which, in
         if (int e2 = launch_energy_spectrum(h, which == XFB_TRACER ? h->c0 : h->z0, nshells, h0->espec)) return e2;
     }
     return energy_spectrum_finish(h0, h0->espec, nshells, totals, e, z);
+}
+
+extern "C" int xfb_loopback_get_spectral_budget(xfb_loopback_s *L, int nshells, double *totals, double *budget)
+{
+    if (!L) return fail(XFB_E_ARG, "null argument");
+    xfb_handle h0 = L->team.local[0];
+    if (int r = spectral_budget_args(h0, 0, nshells, totals, budget, "xfb_loopback_")) return r;
+    CK(cudaSetDevice(h0->device));
+    bool with_src = false;
+    for (int r = 0; r < L->team.nranks; ++r) with_src |= L->team.local[r]->has_src;
+    if (spectral_budget_scratch(h0)) return XFB_E_CUDA;
+    if (int r = team_budget_terms(&L->team, with_src)) return r;
+    // all ranks share the device and the stream: their launches add into rank 0's sums (the all-reduce of the NCCL path)
+    CK(cudaMemsetAsync(h0->bspec, 0, sizeof(double) * XFB_BUDGET_N * (1 + (size_t)nshells), h0->stream));
+    for (int r = 0; r < L->team.nranks; ++r) {
+        xfb_handle h = L->team.local[r];
+        if (int e2 = launch_spectral_budget(h, h->z0, h->spec_a, with_src ? h->spec_b : nullptr, nshells, h0->bspec)) return e2;
+    }
+    return spectral_budget_finish(h0, h0->bspec, nshells, totals, budget);
 }
 
 extern "C" long long xfb_loopback_launch_count(xfb_loopback_s *L)

@@ -306,6 +306,23 @@ int generic_inv2d(xfb_handle h, const cpx *spec_in, cpx *tmp, float *real_out, f
     return 0;
 }
 
+int generic_tendency(xfb_handle h, const cpx *z, const float *src, cpx *T)
+{
+    const int P = h->hy;
+    const long long n = (long long)h->grids;
+    const float scale = 1.0f / (float)((double)h->nx * (double)h->ny);
+    const unsigned gb = (unsigned)((n + 255) / 256);
+    float *fa = h->real_a, *fb = h->real_b, *fc = h->real_c, *fd = (float *)h->t[0];      // dvortdx, dvortdy, -u, v
+    cpx *tmp = h->spec_a, *tmp2 = h->spec_b, *psi = h->t[1];
+    if (launch_pw(h, OP_GRADX, z, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fa, scale, 0)) return XFB_E_CUDA;       // :151-154
+    if (launch_pw(h, OP_GRADY, z, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fb, scale, 0)) return XFB_E_CUDA;       // :165-168
+    if (launch_pw(h, OP_INVLAP, z, P, psi, P, P)) return XFB_E_CUDA;                                                    // :179
+    if (launch_pw(h, OP_GRADY, psi, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fc, scale, 1)) return XFB_E_CUDA;     // :198-201
+    if (launch_pw(h, OP_GRADX, psi, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fd, scale, 0)) return XFB_E_CUDA;     // :212-214
+    GLAUNCH(h, (gen_jacobian<<<gb, 256, 0, h->stream>>>(fc, fa, fd, fb, src, fa, n)));                                  // :225-227
+    return generic_fwd2d(h, fa, tmp2, T);                                                                                // :237
+}
+
 // one RK4 step of every member, one kernel per loop of src/main.cpp:286-317.  A step is 72 short launches per member
 // (124 with the tracer) on grids that live in L2 -- launch gaps, not kernels, bound it --, so xfb_step replays it from a
 // CUDA graph (step_replay) like the fused step.
@@ -319,16 +336,10 @@ int generic_one_step(xfb_handle h, float dt)
         cpx *z0 = h->z0 + (size_t)m * h->hpad, *zk = h->zk + (size_t)m * h->hpad, *acc = h->acc + (size_t)m * h->hpad;
         const float *src = h->has_src ? h->src + (size_t)m * h->grids : nullptr;
         float *fa = h->real_a, *fb = h->real_b, *fc = h->real_c, *fd = (float *)h->t[0];      // dvortdx, dvortdy, -u, v
-        cpx *tmp = h->spec_a, *tmp2 = h->spec_b, *psi = h->t[1], *T = h->jint;
+        cpx *tmp = h->spec_a, *tmp2 = h->spec_b, *T = h->jint;
         for (int k = 1; k <= 4; ++k) {
             const cpx *z = (k == 1) ? z0 : zk;
-            if (launch_pw(h, OP_GRADX, z, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fa, scale, 0)) return XFB_E_CUDA;       // :151-154
-            if (launch_pw(h, OP_GRADY, z, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fb, scale, 0)) return XFB_E_CUDA;       // :165-168
-            if (launch_pw(h, OP_INVLAP, z, P, psi, P, P)) return XFB_E_CUDA;                                                    // :179
-            if (launch_pw(h, OP_GRADY, psi, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fc, scale, 1)) return XFB_E_CUDA;     // :198-201
-            if (launch_pw(h, OP_GRADX, psi, P, tmp, P, P) || generic_inv2d(h, tmp, tmp2, fd, scale, 0)) return XFB_E_CUDA;     // :212-214
-            GLAUNCH(h, (gen_jacobian<<<gb, 256, 0, h->stream>>>(fc, fa, fd, fb, src, fa, n)));                                  // :225-227
-            if (generic_fwd2d(h, fa, tmp2, T)) return XFB_E_CUDA;                                                                // :237
+            if (generic_tendency(h, z, src, T)) return XFB_E_CUDA;
             if (h->lin.on)
                 GLAUNCH(h, (gen_stage<true><<<hb, 256, 0, h->stream>>>(T, z0, zk, acc, h->nx, h->hy, h->kx2, h->ky2, h->mask_kd, h->nu,
                                                                         dt, (k == 3) ? dt : dt / 2.0f, k, h->kx, h->lin)));

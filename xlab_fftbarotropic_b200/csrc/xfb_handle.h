@@ -64,6 +64,7 @@ struct xfb_handle_s {
     int rec_next;
     xfb::cpx *dg;        // 3 exchange arrays of the fused diagnostics path, allocated on first use
     double *espec;       // xfb_get_energy_spectrum sums: 3 + 2 * XFB_SPECTRUM_MAX_SHELLS doubles, allocated on first use
+    double *bspec;       // xfb_get_spectral_budget sums: 6 + 6 * XFB_SPECTRUM_MAX_SHELLS doubles, allocated on first use
     bool warmed;         // one eager step has run (kernels configured)
     void *step_graph;    // cudaGraphExec_t of one RK4 step (step_replay), valid for graph_dt / graph_src
     float graph_dt;
@@ -147,6 +148,9 @@ void generic_destroy(xfb_handle h);
 int generic_fwd2d(xfb_handle h, const float *real_in, cpx *tmp, cpx *spec_out);
 int generic_inv2d(xfb_handle h, const cpx *spec_in, cpx *tmp, float *real_out, float scale, int negate);
 int generic_one_step(xfb_handle h, float dt);
+// the nonlinear tendency r2c(-u.grad(zeta) [+ src]) of the spectral state z (row-major), as one Runge-Kutta stage of
+// generic_one_step forms it, into T; uses real_a, real_b, real_c, t[0], t[1], spec_a and spec_b
+int generic_tendency(xfb_handle h, const cpx *z, const float *src, cpx *T);
 
 // nsteps calls of `one_step` (one RK4 step, xfb_api.cu): the first step of a handle runs eagerly, later ones replay a
 // CUDA graph captured from one call; XFB_NO_GRAPH=1, and profiling when `eager_if_profiling`, keep the eager path
@@ -177,6 +181,13 @@ int energy_spectrum_finish(xfb_handle h, const double *d, int nshells, double *t
 // points the messages name
 int energy_spectrum_args(xfb_handle h, int member, int which, int nshells, const double *totals, const double *e, const double *z,
                          const char *api);
+// spectral budget (xfb_spectra.cu): one launch adds the raw sums of one member into d_out[6 + 6 * nshells] (device, zeroed by
+// the caller) from its state, its nonlinear tendency and its source (null: none), all three in the state's layout; _finish
+// copies them to the host and scales them to rates of domain means; _args checks as energy_spectrum_args does
+int spectral_budget_scratch(xfb_handle h);
+int launch_spectral_budget(xfb_handle h, const cpx *state, const cpx *tend, const cpx *src, int nshells, double *d_out);
+int spectral_budget_finish(xfb_handle h, const double *d, int nshells, double *totals, double *budget);
+int spectral_budget_args(xfb_handle h, int member, int nshells, const double *totals, const double *budget, const char *api);
 
 // slab paths (xfb_dist.cu)
 int dist_keff_hist(xfb_handle h, int nbins, float cmin, float cmax, double *area, double *grad2, bool tracer_state);
@@ -186,6 +197,7 @@ int dist_set_tracer(xfb_handle h, const float *tracer_rows);
 int dist_step(xfb_handle h, int nsteps, float dt);
 int dist_get_field(xfb_handle h, int which, float *out_rows);
 int dist_energy_spectrum(xfb_handle h, int which, int nshells, double *totals, double *e, double *z);
+int dist_spectral_budget(xfb_handle h, int nshells, double *totals, double *budget);
 void dist_release(xfb_handle h);
 
 }  // namespace xfb
